@@ -31,6 +31,8 @@ A "step" is one complete GNK solve of a named workload (`--workload`, default = 
 would not be matched work.  `--ref-budget-s` bounds it: when the budget is exhausted the solve is cut at the current
 outer iteration and the line says so.
 
+`--dump-outputs DIR` writes what the last timed step of the headline workload returned to DIR (see dump_outputs).
+
 Multi-GPU (torchrun, one rank per GPU): the grid rows are partitioned into slabs, scaling is strong.
 """
 import argparse
@@ -80,7 +82,13 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-ttt", action="store_true", help="skip the time-to-tolerance workloads")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the result of the headline workload's last timed step to DIR/*.npy (see dump_outputs)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if a.dump_outputs is not None and a.impl != "ours":
+        ap.error("--dump-outputs writes the result of the GPU path (--impl ours)")
     if a.grid_nodes is not None or a.iters is not None or a.restart is not None or a.ls is not None:
         a.workload = "custom"
     return a
@@ -274,6 +282,26 @@ class ClockSampler(threading.Thread):
 # ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
+DUMP_MAX_X = 1 << 22  # float64 entries of x written by --dump-outputs (32 MiB)
+
+
+def dump_outputs(dump_dir, out, rank):
+    """What the caller of the timed solve receives, so that two builds can be compared output for output:
+      x.npy       the solution (float64); above DUMP_MAX_X entries, the entries at a fixed sample of indices
+                  (numpy default_rng(0), drawn without replacement, in increasing order)
+      counts.npy  [nit, nfev (RegressionResult.nrev), njev, success] as float64
+    The inputs of a workload do not change from run to run (u0 from seed 42), so neither does the sample."""
+    x = np.asarray(out.x, dtype=np.float64)  # every rank takes part in gathering the sharded solution
+    if rank != 0:
+        return
+    if x.size > DUMP_MAX_X:
+        x = x[np.sort(np.random.default_rng(0).choice(x.size, DUMP_MAX_X, replace=False))]
+    os.makedirs(dump_dir, exist_ok=True)
+    np.save(os.path.join(dump_dir, "x.npy"), x)
+    np.save(os.path.join(dump_dir, "counts.npy"),
+            np.array([out.nit, out.nrev, out.njev, float(out.success)], dtype=np.float64))
+
+
 class Harness:
     def __init__(self, a):
         import torch
@@ -307,7 +335,7 @@ class Harness:
         return float(t.item())
 
     # --------------------------------------------------------------------------------------------
-    def measure(self, name, steps, warmup, e2e=True, parity=True, sample_clocks=False):
+    def measure(self, name, steps, warmup, e2e=True, parity=True, sample_clocks=False, dump_dir=None):
         a, g, rt, torch = self.a, self.g, self.rt, self.torch
         spec = workload_spec(a, name)
         G = spec["grid_nodes"]
@@ -354,6 +382,8 @@ class Harness:
         m = dict(value=value, ms_per_step=ms / steps, steps=steps, warmup=warmup, gpu_launches=int(launches),
                  result=dict(nit=int(out.nit), nfev=int(out.nrev), success=bool(out.success)),
                  clocks=sampler.summary() if sampler is not None else None)
+        if dump_dir is not None:
+            dump_outputs(dump_dir, out, self.rank)
         del out
 
         # ---- per-kernel roofline pass (events around every kernel class; not part of the headline timing) ----
@@ -512,7 +542,8 @@ def run_ours(a):
     h = Harness(a)
     rank, world = h.rank, h.world
     name = a.workload
-    head = h.measure(name, a.steps, a.warmup, e2e=not a.no_e2e, parity=not a.no_parity, sample_clocks=True)
+    head = h.measure(name, a.steps, a.warmup, e2e=not a.no_e2e, parity=not a.no_parity, sample_clocks=True,
+                     dump_dir=a.dump_outputs)
 
     extras = {}
     if a.extras == "auto":
@@ -528,9 +559,8 @@ def run_ours(a):
     else:
         want = [w for w in a.extras.split(",") if w]
     for w in want:
-        st, wu = (5, 3) if not w.startswith("bratu_8192") else (3, 3)
         try:
-            e = h.measure(w, st, wu, e2e=not a.no_e2e, parity=not a.no_parity)
+            e = h.measure(w, a.steps, a.warmup, e2e=not a.no_e2e, parity=not a.no_parity)
         except Exception as exc:  # an extra workload must never cost the headline line (raised alike on every rank)
             extras[w] = dict(error=f"{type(exc).__name__}: {exc}")
             continue

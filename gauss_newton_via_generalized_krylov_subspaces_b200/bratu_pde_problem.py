@@ -291,6 +291,11 @@ class StencilJacobian:
         d.apply(self.expu, r, d.ld, 1, self.scale, int(not self.transposed), w, d.ld, d.fields["off"])
 
     def linop(self, sign):
+        # gnk_linop carries no transpose flag and gnk_stencil_normal_diag gives diag(J^T J) only: a transposed operator
+        # would be solved as J.  Callers route J.T through CsrJacobian(rt, J.T.tocsr(), True) instead
+        if self.transposed:
+            raise _lib.GnkError("StencilJacobian.linop: the device CG operator cannot represent J.T; assemble it "
+                                "(CsrJacobian of .tocsr())")
         d = self.pb.dev
         op = _lib.LinOp()
         op.kind = 0

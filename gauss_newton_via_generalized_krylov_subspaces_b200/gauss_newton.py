@@ -41,6 +41,15 @@ def cg_least_squares(A, y, x0=None, cg_rtol=1e-4, preconditioner=True):
     A: scipy sparse matrix / ndarray / device stencil operator, y: ndarray.  Returns (x, cg_iter) where cg_iter
     sums the unpreconditioned and the preconditioned run when ``preconditioner`` is False (reference quirk)."""
     rt = get_runtime()
+    if isinstance(A, StencilJacobian) and A.transposed:
+        # the device stencil operator has no transpose of its own (J is not symmetric: ALPHA d/dx1), and the Jacobi
+        # diagonal of A = J^T needs the row sums of J^2, not the column sums the stencil kernel forms.  The assembled
+        # CSR of J^T is exact on both counts; it exists on one rank only.
+        if rt.world > 1:
+            raise _lib.GnkError(
+                f"cg_least_squares: a transposed Bratu Jacobian (J.T) is not supported with {rt.world} ranks; pass J, "
+                "or solve in a single-rank process")
+        A = CsrJacobian(rt, A.tocsr(), True)
     if isinstance(A, StencilJacobian):
         d = A.pb.dev
         ycol = d.new_col()

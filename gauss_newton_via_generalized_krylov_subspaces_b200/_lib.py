@@ -12,6 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libgnk_b200.so")
 
 GNK_MAX_BASIS = 256
+GNK_TSQR_MAX = 104  # include/gnk_b200.h
 
 
 class Layout(C.Structure):

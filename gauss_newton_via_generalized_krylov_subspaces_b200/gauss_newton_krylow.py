@@ -33,6 +33,8 @@ from .regression_result import RegressionResult
 from .rosenbrock_problem import RosenbrockDeviceProblem
 
 _NB = _lib.GNK_MAX_BASIS
+_TSQR_MAX = _lib.GNK_TSQR_MAX
+_DENSE_QR_MAX = 1 << 22  # doubles of the single-CTA wide-panel QR (csrc/tsqr.cu: run_dense_qr)
 # layout of the per-iteration scalar block (device, one D2H read per Armijo trial)
 _SC_LOSS = 2 * _NB + 8   # 2 doubles: sum(F^2) [, max|F|]
 _SC_CPREV = _SC_LOSS + 2  # sum(c_prev^2)
@@ -181,6 +183,11 @@ def linear_least_squares(A, y):
     n, k = A.shape
     if k + 1 > _NB:
         raise _lib.GnkError(f"linear_least_squares supports at most {_NB - 1} columns")
+    # The host-array entry keeps the single-CTA QR's range for panels wider than 104 columns, as it always had; the
+    # blocked TSQR for larger wide panels serves the device-resident panels of gauss_newton_krylow and gauss_newton.
+    if k + 1 > _TSQR_MAX and n * (k + 1) > _DENSE_QR_MAX:
+        raise _lib.GnkError(f"linear_least_squares with more than {_TSQR_MAX - 1} columns is limited to panels of "
+                            "2^22 doubles")
     lda = round_up(max(n, 1), 16)
     dA = rt.zeros(lda * k)
     for j in range(k):

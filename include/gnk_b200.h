@@ -35,9 +35,10 @@ extern "C" {
 
 #define GNK_B200_ABI_VERSION 1
 #define GNK_MAX_BASIS 256 /* k <= 255 basis columns (+1 rhs column in the least-squares panel) */
-#define GNK_TSQR_MAX 104  /* widest panel of the tiled Householder TSQR; wider panels (the reference's max_iter=200 runs
-                             without restart, bratu_pde_test.py:307-316) take the single-CTA Householder QR, which
-                             needs the whole panel (n_rows * (k+1) <= 2^22 doubles) and a single rank */
+#define GNK_TSQR_MAX 104  /* widest panel of the tiled Householder TSQR; wider panels (runs without a restart) take
+                             the single-CTA Householder QR on one rank while n_rows * (k+1) <= 2^22 doubles (it needs
+                             n_rows >= k+1), and the blocked Householder TSQR spread over the SMs otherwise (several
+                             ranks, or larger panels) */
 
 typedef struct gnk_ctx gnk_ctx;
 
@@ -149,7 +150,11 @@ int gnk_cgs_update(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k
  * d = 0 and d_out[k+2] = -1, and the caller re-issues the call after gnk_tsqr_ls_method(ctx, 1).
  * Panels of 33 <= k+1 <= 56 columns under the same conditions (krylow_restart up to 55; method 0 only) take the same
  * scheme with a wider Gram sweep (5..7 column blocks), a dense Cholesky in one CTA and the refinement form
- * (gram_cgls.cu: gnk_cholqr_wide_try), with the same result block and the same refusal convention. */
+ * (gram_cgls.cu: gnk_cholqr_wide_try), with the same result block and the same refusal convention.
+ * Panels of GNK_TSQR_MAX < k+1 <= GNK_MAX_BASIS columns: one rank and n_rows * (k+1) <= 2^22 doubles take a single-CTA
+ * unblocked Householder QR (n_rows >= k+1 required); several ranks or larger panels take a blocked Householder TSQR
+ * (row-block leaves with compact-WY updates on the FP64 tensor pipe, pairwise tree, all-gather of the ranks' triangles,
+ * reduced in rank order on every rank).  Any lda >= n_rows, 8-byte aligned A and y, ranks with fewer rows than columns. */
 int gnk_tsqr_ls(gnk_ctx* ctx, const double* d_A, int64_t lda, int64_t n_rows, int k,
                 const double* d_y, double sign_a, double* d_out, void* stream);
 

@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(_HERE, "libgnk_b200.so")
 
 GNK_MAX_BASIS = 256
 GNK_TSQR_MAX = 104  # include/gnk_b200.h
+GNK_PATTERN_INVALID = 3  # gnk_csr_pattern: the index pattern is not canonical CSR
 
 
 class Layout(C.Structure):
@@ -68,6 +69,9 @@ SIGNATURES = {
     "gnk_gram_cgls": (_I, [_P, _P, _L, _L, _I, _P, _D, _D, _P, _P]),
     "gnk_spmm_csr": (_I, [_P, _L, _P, _P, _P, _P, _L, _L, _I, _D, _P, _L, _L, _P]),
     "gnk_csr_row_sumsq": (_I, [_P, _L, _P, _P, _P, _P]),
+    "gnk_csr_pattern": (_I, [_P, _L, _L, _L, _P, _P, _I, _P, _P, _P, _P, _P, _P]),
+    "gnk_csr_pattern_equal": (_I, [_P, _L, _L, _P, _P, _I, _P, _P, _P]),
+    "gnk_csr_gather": (_I, [_P, _L, _P, _P, _P, _P]),
     "gnk_axpby": (_I, [_P, _L, _D, _P, _D, _P, _P, _P]),
     "gnk_dot": (_I, [_P, _L, _P, _P, _P, _P]),
     "gnk_cgls": (_I, [_P, C.POINTER(LinOp), _P, _D, _I, _P, _P, C.POINTER(_L), _P]),

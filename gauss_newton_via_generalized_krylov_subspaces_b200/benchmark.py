@@ -33,7 +33,10 @@ def benchmark_method(method, res, x0, jac, error, args=(), kwargs={}):
         loss = res.loss
     else:
         def loss(x):
-            return 0.5 * np.sum(np.asarray(res(x, *args)) ** 2)
+            r = res(x, *args)
+            if hasattr(r, "is_cuda"):  # device callables: a torch tensor, reduced where it lives
+                return 0.5 * float((r.double() ** 2).sum())
+            return 0.5 * np.sum(np.asarray(r) ** 2)
 
     error_list = [error(x0)]
     loss_list = [loss(x0)]

@@ -49,6 +49,9 @@ struct gnk_ctx {
   // gnk_cgls (cgls.cu): the stopping test of CG iteration i is read while iteration i + 1 is already queued; two reads in
   // flight, each with an event on the caller's stream ([0..1]) and one on the copy stream ([2..3])
   cudaEvent_t cg_event[4] = {nullptr, nullptr, nullptr, nullptr};
+  // gnk_csr_pattern (csr.cu): row of every non-zero, sort keys and values, column histogram, cub temp (grown on demand)
+  void* d_pattern = nullptr;
+  size_t pattern_bytes = 0;
 };
 int gnk_ensure_fetch_stream(gnk_ctx* ctx);  // api.cu: creates fetch_stream / fetch_event on first use
 

@@ -7,6 +7,7 @@ import atexit
 import ctypes as C
 import mmap
 import os
+import sys
 import time
 import weakref
 
@@ -529,3 +530,192 @@ class HostCallableProblem:
 
     def jacobian(self, x, aux=None):
         return self.jacobian_host(self.download_global(x))
+
+
+# --------------------------------------------------------------------------------------------------
+# device callables: res / jac take and return CUDA tensors (selected by a CUDA-tensor x0).  The callables are still
+# the user's code, but x, F and J never leave HBM: the residual is copied device to device, the Jacobian's index
+# pattern and its transpose are built on the device (gnk_csr_pattern) and cached while the pattern stays the same.
+# --------------------------------------------------------------------------------------------------
+_INT32_LIMIT = (1 << 31) - 1  # sizes and nnz stay below: int32 indices, and n + 1 row pointers
+
+
+def is_cuda_tensor(x):
+    torch = sys.modules.get("torch")
+    return torch is not None and isinstance(x, torch.Tensor) and x.is_cuda
+
+
+def _require_on_device(rt, t, what):
+    if not isinstance(t, rt.torch.Tensor):
+        raise TypeError(f"{what}: expected a torch.Tensor on {rt.device}, got {type(t).__name__}")
+    if t.device != rt.device:
+        raise ValueError(f"{what}: expected a tensor on {rt.device}, got one on {t.device}")
+
+
+def device_csr(rt, J, shape=None, what="jac"):
+    """A CUDA Jacobian (torch sparse CSR / COO, or a strided (n_res, p) tensor) -> (rowptr, col, val, is_sparse, dense):
+    the canonical CSR of J (COO coalesced, dense without its exact zeros, as scipy.sparse.csr_array(dense)) with int32
+    or int64 indices, float64 values, and the dense tensor itself for a strided input (else None)."""
+    torch = rt.torch
+    _require_on_device(rt, J, what)
+    if J.dim() != 2:
+        raise ValueError(f"{what}: expected a 2-D Jacobian, got shape {tuple(J.shape)}")
+    if shape is not None and tuple(J.shape) != tuple(shape):
+        raise ValueError(f"{what}: expected shape {tuple(shape)} (n_res, p), got {tuple(J.shape)}")
+    n_rows, n_cols = (int(v) for v in J.shape)
+    nnz = J._nnz() if J.layout in (torch.sparse_csr, torch.sparse_coo) else 0
+    if max(n_rows, n_cols, nnz) >= _INT32_LIMIT:
+        raise _lib.GnkError(f"{what}: a {n_rows} x {n_cols} Jacobian with {nnz} stored entries does not fit the int32 "
+                            "indices of the CSR kernels (every dimension and nnz must stay below 2^31 - 1)")
+    dense = None
+    if J.layout == torch.sparse_csr:
+        A = J
+    elif J.layout == torch.sparse_coo:
+        A = J.coalesce().to_sparse_csr()
+    elif J.layout == torch.strided:
+        dense = J
+        A = J.to_sparse_csr()
+    else:
+        raise TypeError(f"{what}: expected a sparse_csr, sparse_coo or strided tensor, got layout {J.layout}")
+    if A._nnz() >= _INT32_LIMIT:
+        raise _lib.GnkError(f"{what}: {A._nnz()} non-zeros do not fit the int32 indices of the CSR kernels")
+    rowptr, col = A.crow_indices().contiguous(), A.col_indices().contiguous()
+    if col.dtype != rowptr.dtype:
+        col = col.to(rowptr.dtype)
+    val = A.values().to(torch.float64).contiguous()
+    return rowptr, col, val, dense is None, dense
+
+
+class CsrPattern:
+    """The index pattern of a CSR matrix on the device, as int32 (rowptr, col), with the sorted pattern of its transpose
+    (rowptr_t, col_t) and perm: transpose position -> non-zero of A (gnk_csr_pattern).  Immutable: a Jacobian built on
+    it keeps it alive, and a changed pattern gets a new object."""
+
+    def __init__(self, rt, n_rows, n_cols, rowptr, col):
+        t = rt.torch
+        self.rt = rt
+        self.n_rows, self.n_cols, self.nnz = int(n_rows), int(n_cols), int(col.numel())
+        i32 = t.int32
+        self.rowptr = t.empty(self.n_rows + 1, dtype=i32, device=rt.device)
+        self.rowptr_t = t.empty(self.n_cols + 1, dtype=i32, device=rt.device)
+        self.col, self.col_t, self.perm = (t.empty(self.nnz, dtype=i32, device=rt.device) for _ in range(3))
+        rc = rt.lib.gnk_csr_pattern(rt.ctx, self.n_rows, self.n_cols, self.nnz, ptr(rowptr), ptr(col),
+                                    rowptr.element_size(), ptr(self.rowptr), ptr(self.col), ptr(self.rowptr_t),
+                                    ptr(self.col_t), ptr(self.perm), rt.stream)
+        if rc == _lib.GNK_PATTERN_INVALID:
+            raise ValueError(rt.lib.gnk_last_error().decode())
+        _lib.check(rc, "gnk_csr_pattern")
+
+    def matches(self, n_rows, n_cols, rowptr, col, flag):
+        """same shape and the same index arrays (one device compare, one int read back)"""
+        if (int(n_rows), int(n_cols), int(col.numel())) != (self.n_rows, self.n_cols, self.nnz):
+            return False
+        rt = self.rt
+        _lib.check(rt.lib.gnk_csr_pattern_equal(rt.ctx, self.n_rows, self.nnz, ptr(rowptr), ptr(col),
+                                                rowptr.element_size(), ptr(self.rowptr), ptr(self.col), ptr(flag),
+                                                rt.stream), "gnk_csr_pattern_equal")
+        return int(rt.read_i32(flag)[0]) == 0
+
+
+class DeviceCsrJacobian:
+    """J on the device as CSR of J and of J^T over a CsrPattern; J^T's values by one gather (gnk_csr_gather).  Same
+    interface as CsrJacobian.  ``user`` is the object the user's jac returned (handed to a step-length plug-in),
+    ``dense`` the strided tensor for a dense Jacobian (gauss_newton's QR branch), else None."""
+
+    transposed = False
+    scale = 1.0
+
+    def __init__(self, rt, pattern, val, is_sparse, user=None, dense=None):
+        self.rt, self.pattern, self.val = rt, pattern, val
+        self.is_sparse, self.user, self.dense = is_sparse, user, dense
+        self.n_res, self.p = pattern.n_rows, pattern.n_cols
+        self.rowptr, self.col, self.rowptr_t, self.col_t = pattern.rowptr, pattern.col, pattern.rowptr_t, pattern.col_t
+        self.val_t = rt.torch.empty_like(val)
+        _lib.check(rt.lib.gnk_csr_gather(rt.ctx, pattern.nnz, ptr(pattern.perm), ptr(val), ptr(self.val_t), rt.stream),
+                   "gnk_csr_gather")
+
+    @classmethod
+    def from_tensor(cls, rt, J, what="A"):
+        rowptr, col, val, is_sparse, dense = device_csr(rt, J, what=what)
+        return cls(rt, CsrPattern(rt, J.shape[0], J.shape[1], rowptr, col), val, is_sparse, J, dense)
+
+    matmat = CsrJacobian.matmat
+    neg_rmatvec = CsrJacobian.neg_rmatvec
+    linop = CsrJacobian.linop
+
+
+class DeviceCallableProblem:
+    """res / jac are Python callables on CUDA tensors: res(x, *args) -> 1-D tensor of n_res values, jac(x, *args) ->
+    torch sparse CSR / COO or strided (n_res, p) tensor.  x is a fresh float64 tensor of length p at every call."""
+
+    distributed = False
+    device_native = True  # x and F stay in HBM
+    user_code = True      # ... but res / jac are the user's: they are evaluated only where the reference evaluates them
+
+    def __init__(self, res, jac, x0, args):
+        self.rt = rt = get_runtime()
+        _require_on_device(rt, x0, "x0")
+        self.res, self.jac, self.args = res, jac, tuple(args)
+        self.p_glob = int(x0.numel())
+        if self.p_glob >= _INT32_LIMIT:
+            raise _lib.GnkError(f"x0 has {self.p_glob} entries; the CSR kernels index with int32")
+        self.sol_fields = flat_layout_fields(self.p_glob)
+        self.sol = make_layout(self.sol_fields)
+        self.n_res = None
+        self.res_fields = None
+        self.pattern = None
+        self.pattern_builds = 0   # gnk_csr_pattern calls: once per distinct sparsity pattern of jac
+        self._flag = rt.torch.zeros(1, dtype=rt.torch.int32, device=rt.device)
+
+    def _ensure_res_layout(self, n_res):
+        if self.n_res is None:
+            if n_res >= _INT32_LIMIT:
+                raise _lib.GnkError(f"res returned {n_res} values; the CSR kernels index with int32")
+            self.n_res = int(n_res)
+            self.res_fields = flat_layout_fields(self.n_res)
+            self.res_lay = make_layout(self.res_fields)
+
+    def new_sol(self):
+        return self.rt.zeros(self.sol_fields["ld"])
+
+    def new_res(self):
+        return self.rt.zeros(self.res_fields["ld"])
+
+    def upload_x(self, x, out):
+        out[:self.p_glob].copy_(x.reshape(-1))
+
+    def download_global(self, t):
+        return self.rt.download(t[:self.p_glob])
+
+    def x_out(self, t):
+        """the iterate as the user sees it: a CUDA tensor of its own"""
+        return t[:self.p_glob].clone()
+
+    def evaluate(self, x):
+        """res at the stored column x -> 1-D CUDA tensor (fixes the residual-space layout at the first call)"""
+        r = self.res(self.x_out(x), *self.args)
+        _require_on_device(self.rt, r, "res")
+        if r.dim() != 1:
+            raise ValueError(f"res: expected a 1-D tensor, got shape {tuple(r.shape)}")
+        if self.n_res is not None and r.shape[0] != self.n_res:
+            raise ValueError(f"res: expected {self.n_res} values (the length of its first result), got {r.shape[0]}")
+        self._ensure_res_layout(r.shape[0])
+        return r
+
+    def residual(self, x, F, loss_slot, aux=None):
+        F[:self.n_res].copy_(self.evaluate(x))
+        self.sumsq(F, loss_slot, self.res_lay)
+
+    def sumsq(self, vec, slot2, lay):
+        rt = self.rt
+        _lib.check(rt.lib.gnk_norm_stats(rt.ctx, C.byref(lay), ptr(vec), ptr(slot2), rt.stream), "gnk_norm_stats")
+
+    def jacobian(self, x, aux=None):
+        J = self.jac(self.x_out(x), *self.args)
+        rowptr, col, val, is_sparse, dense = device_csr(self.rt, J, (self.n_res, self.p_glob))
+        pat = self.pattern
+        if pat is None or not pat.matches(self.n_res, self.p_glob, rowptr, col, self._flag):
+            pat = CsrPattern(self.rt, self.n_res, self.p_glob, rowptr, col)
+            self.pattern = pat
+            self.pattern_builds += 1
+        return DeviceCsrJacobian(self.rt, pat, val, is_sparse, J, dense)

@@ -19,7 +19,8 @@ import numpy as np
 from . import _lib
 from .armijo_goldstein import armijo_device, armijo_goldstein
 from .bratu_pde_problem import BratuDeviceProblem, StencilJacobian
-from .device import CsrJacobian, DeviceVector, get_runtime, make_layout, ptr
+from .device import (CsrJacobian, DeviceCsrJacobian, DeviceVector, _require_on_device, get_runtime, is_cuda_tensor,
+                     make_layout, ptr)
 from .gauss_newton_krylow import _report_rank, require_single_rank_unless_sharded, resolve_problem, tsqr_solve
 from .partition import flat_layout_fields, round_up
 from .regression_result import RegressionResult
@@ -38,9 +39,30 @@ def _cgls(rt, linop, y, rtol, preconditioner, x_out, vlen, x0=None):
 def cg_least_squares(A, y, x0=None, cg_rtol=1e-4, preconditioner=True):
     """Iterative solver for min ||y - A x|| via CG on the normal equations (reference :11-60), on the device.
 
-    A: scipy sparse matrix / ndarray / device stencil operator, y: ndarray.  Returns (x, cg_iter) where cg_iter
+    A: scipy sparse matrix / ndarray / device stencil operator, y: ndarray -- or A: CUDA tensor (torch sparse CSR / COO,
+    or dense), y (and x0): CUDA tensors, and x comes back as a CUDA tensor.  Returns (x, cg_iter) where cg_iter
     sums the unpreconditioned and the preconditioned run when ``preconditioner`` is False (reference quirk)."""
     rt = get_runtime()
+    if is_cuda_tensor(A):
+        require_single_rank_unless_sharded(rt, None, "cg_least_squares")
+        op = DeviceCsrJacobian.from_tensor(rt, A, "cg_least_squares: A")
+        _require_on_device(rt, y, "cg_least_squares: y")
+        y = y.reshape(-1)
+        if y.shape[0] != op.n_res:
+            raise ValueError(f"cg_least_squares: y must have {op.n_res} entries, got {y.shape[0]}")
+        vlen = round_up(max(op.p, op.n_res), 16)
+        dy = rt.zeros(vlen)
+        dy[:op.n_res].copy_(y)
+        x = rt.zeros(vlen)
+        dx0 = None
+        if x0 is not None:
+            _require_on_device(rt, x0, "cg_least_squares: x0")
+            if x0.numel() != op.p:
+                raise ValueError(f"cg_least_squares: x0 must have {op.p} entries, got {x0.numel()}")
+            dx0 = rt.zeros(vlen)
+            dx0[:op.p].copy_(x0.reshape(-1))
+        it = _cgls(rt, op.linop(1.0), dy, cg_rtol, preconditioner, x, vlen, dx0)
+        return x[:op.p].clone(), it
     if isinstance(A, StencilJacobian) and A.transposed:
         # the device stencil operator has no transpose of its own (J is not symmetric: ALPHA d/dx1), and the Jacobi
         # diagonal of A = J^T needs the row sums of J^2, not the column sums the stencil kernel forms.  The assembled
@@ -97,8 +119,9 @@ def gauss_newton(
     """
     rt = get_runtime()
     lib = rt.lib
-    x0_host = np.asarray(x0, dtype=np.float64).reshape(-1)
+    x0_host = x0 if is_cuda_tensor(x0) else np.asarray(x0, dtype=np.float64).reshape(-1)
     prob = resolve_problem(res, jac, x0_host, args)
+    user_dev = getattr(prob, "user_code", False)  # device callables: x, F and J stay in HBM
     is_bratu = isinstance(prob, BratuDeviceProblem)
     require_single_rank_unless_sharded(rt, prob, "gauss_newton")
     # Several ranks (Bratu only: row slabs, as in gauss_newton_krylow): the CG solve exchanges one halo row per operator
@@ -132,6 +155,12 @@ def gauss_newton(
         F, F_trial = prob.new_res(), prob.new_res()
         prob.residual(x, F, scal, aux=aux_cur)
         r_host = None
+    elif user_dev:
+        r0 = prob.evaluate(x)
+        F, F_trial = prob.new_res(), prob.new_res()
+        F[:prob.n_res].copy_(r0)
+        prob.sumsq(F, scal, prob.res_lay)
+        r_host = None
     else:
         r_host = np.asarray(res(x0_host.copy(), *args), dtype=np.float64).reshape(-1)
         prob._ensure_res_layout(r_host.shape[0])
@@ -152,6 +181,9 @@ def gauss_newton(
         if is_bratu:
             jac_ev = prob.jacobian(x, aux=aux_cur)
             sparse_like = True
+        elif user_dev:
+            jac_ev = prob.jacobian(x)
+            sparse_like = jac_ev.is_sparse
         else:
             x_host = prob.download_global(x)
             jac_ev = prob.jacobian_host(x_host)
@@ -165,11 +197,14 @@ def gauss_newton(
             # dense J: min ||-J d - r|| by Householder QR (reference: scipy.linalg.lstsq, full-rank case)
             if p + 1 > _NB:
                 raise _lib.GnkError(f"dense Jacobians are supported up to {_NB - 1} columns")
-            dense = np.asfortranarray(np.asarray(jac_ev.host, dtype=np.float64))
             lda = round_up(max(n_res, 1), 16)
             dA = rt.zeros(lda * p)
-            for j in range(p):
-                rt.upload(np.ascontiguousarray(dense[:, j]), dA[j * lda:j * lda + n_res])
+            if user_dev:
+                dA.view(p, lda)[:, :n_res].copy_(jac_ev.dense.T)
+            else:
+                dense = np.asfortranarray(np.asarray(jac_ev.host, dtype=np.float64))
+                for j in range(p):
+                    rt.upload(np.ascontiguousarray(dense[:, j]), dA[j * lda:j * lda + n_res])
             tsqr_solve(rt, dA, lda, n_res, p, F[res_off:], -1.0, blk, householder=True)
             # scipy.linalg.lstsq (:126) is SVD-based and returns the minimum-norm step for a rank-deficient J; the QR here
             # has no such branch, and an exactly singular R would hand inf/NaN to 100 Armijo trials.  Say so instead.
@@ -197,7 +232,7 @@ def gauss_newton(
             def trial_loss(s):
                 _lib.check(lib.gnk_axpby(rt.ctx, ax_n, 1.0, ptr(x, ax_off), float(s), ptr(d, ax_off),
                                          ptr(x_trial, ax_off), rt.stream), "gnk_axpby")
-                if is_bratu:
+                if is_bratu or user_dev:
                     prob.residual(x_trial, F_trial, scal, aux=aux_trial)
                 else:
                     state["r_host"] = prob.residual_host(prob.download_global(x_trial), F_trial, scal)
@@ -210,16 +245,25 @@ def gauss_newton(
             new_loss = float(state["vals"][0])
             r_host = state.get("r_host")
         else:
-            # user plug-in: called with host objects like the reference (:118-120)
-            if x_host is None:
-                x_host = prob.download_global(x)
-            if r_host is None:
-                r_host = prob.download_global(F)
-            d_host = prob.download_global(d)
-            host_J = jac_ev if is_bratu else jac_ev.host
-            step_length, r_new, nfev_delta = step_length_control(res, x_host, r_host, host_J, args, d_host)
-            r_host = np.asarray(r_new, dtype=np.float64).reshape(-1)
-            prob.upload_x(r_host, F_trial) if is_bratu else rt.upload(r_host, F_trial[:n_res])
+            # user plug-in: called with host objects like the reference (:118-120); with device callables, with the
+            # objects res and jac take and return (CUDA tensors, the user's Jacobian)
+            if user_dev:
+                step_length, r_new, nfev_delta = step_length_control(
+                    res, prob.x_out(x), F[:n_res].clone(), jac_ev.user, args, prob.x_out(d))
+                _require_on_device(rt, r_new, "step_length_control: residual")
+                if r_new.numel() != n_res:
+                    raise ValueError(f"step_length_control: expected a residual of {n_res} values, got {r_new.numel()}")
+                F_trial[:n_res].copy_(r_new.reshape(-1))
+            else:
+                if x_host is None:
+                    x_host = prob.download_global(x)
+                if r_host is None:
+                    r_host = prob.download_global(F)
+                d_host = prob.download_global(d)
+                host_J = jac_ev if is_bratu else jac_ev.host
+                step_length, r_new, nfev_delta = step_length_control(res, x_host, r_host, host_J, args, d_host)
+                r_host = np.asarray(r_new, dtype=np.float64).reshape(-1)
+                prob.upload_x(r_host, F_trial) if is_bratu else rt.upload(r_host, F_trial[:n_res])
             _lib.check(lib.gnk_norm_stats(rt.ctx, C.byref(res_lay), ptr(F_trial), ptr(scal), rt.stream), "gnk_norm_stats")
             reduce(0, 2, 2)
             _lib.check(lib.gnk_dot(rt.ctx, p, ptr(d, off), ptr(d, off), ptr(scal, 5), rt.stream), "gnk_dot")
@@ -243,11 +287,14 @@ def gauss_newton(
         aux_cur, aux_trial = aux_trial, aux_cur
         prev_loss = new_loss
 
-        xv = DeviceVector(prob, x, prob.p_glob)
-        callback(x=xv, nfev=nfev, cg_iter=cg_iter)
-        xref = weakref.ref(xv)
-        del xv
-        DeviceVector.settle(xref)  # a callback that kept x gets its host snapshot before the buffer is reused
+        if user_dev:
+            callback(x=prob.x_out(x), nfev=nfev, cg_iter=cg_iter)
+        else:
+            xv = DeviceVector(prob, x, prob.p_glob)
+            callback(x=xv, nfev=nfev, cg_iter=cg_iter)
+            xref = weakref.ref(xv)
+            del xv
+            DeviceVector.settle(xref)  # a callback that kept x gets its host snapshot before the buffer is reused
 
         if step_length**2 * squared_sum_d <= tol**2 * squared_sum_x_prev:
             success = True
@@ -256,4 +303,5 @@ def gauss_newton(
     if not success:
         print("Warning: The gauss_newton algorithm reached maximal iteration bound before terminating!")
 
-    return RegressionResult("gauss newton", prob.download_global(x), success, nfev, njev, iter)
+    return RegressionResult("gauss newton", prob.x_out(x) if user_dev else prob.download_global(x), success, nfev,
+                            njev, iter)

@@ -25,7 +25,8 @@ import numpy as np
 from . import _lib
 from .armijo_goldstein import armijo_device
 from .bratu_pde_problem import BratuDeviceProblem
-from .device import DeviceVector, HostCallableProblem, get_runtime, make_layout, ptr
+from .device import (DeviceCallableProblem, DeviceVector, HostCallableProblem, get_runtime, is_cuda_tensor,
+                     make_layout, ptr)
 from .krylow import (GeneralizedKrylowSubspace, GeneralizedKrylowSubspaceBreakdown,
                      GeneralizedKrylowSubspaceSpansEntireSpace, MAX_COLUMNS)
 from .partition import flat_layout_fields, round_up, tensor_ls_on_every_rank
@@ -45,6 +46,8 @@ _VERSIONS = ("res_old", "res_new", "jac_old_res_old", "jac_old_res_new")
 
 
 def resolve_problem(res, jac, x0, args, native_rosenbrock=False):
+    if is_cuda_tensor(x0):  # a CUDA-tensor x0: res / jac take and return CUDA tensors
+        return DeviceCallableProblem(res, jac, x0, args)
     if BratuDeviceProblem.match(res, jac) and not args:
         return BratuDeviceProblem(res, jac)
     if native_rosenbrock and RosenbrockDeviceProblem.match(res, jac, args) \
@@ -175,11 +178,24 @@ def cgls_dense(rt, JV, ldjv, n_rows, k, y, sign, rtol, out):
 
 def linear_least_squares(A, y):
     """Least squares solution of ||y - A x|| by Householder TSQR on the device (reference :16-36: economic QR,
-    a print per |r_kk| <= 1e-8, triangular solve).  A: (n, k) ndarray, y: (n,) ndarray -> x: (k,) ndarray."""
+    a print per |r_kk| <= 1e-8, triangular solve).  A: (n, k) ndarray, y: (n,) ndarray -> x: (k,) ndarray; or A: dense
+    (n, k) CUDA tensor, y: CUDA tensor -> x: CUDA tensor."""
     rt = get_runtime()
     require_single_rank_unless_sharded(rt, None, "linear_least_squares")
-    A = np.asarray(A, dtype=np.float64)
-    y = np.asarray(y, dtype=np.float64).reshape(-1)
+    on_device = is_cuda_tensor(A)
+    if on_device:
+        from .device import _require_on_device
+        _require_on_device(rt, A, "linear_least_squares: A")
+        _require_on_device(rt, y, "linear_least_squares: y")
+        if A.dim() != 2 or A.layout != rt.torch.strided:
+            raise ValueError(f"linear_least_squares: A must be a dense 2-D tensor, got shape {tuple(A.shape)} "
+                             f"and layout {A.layout}")
+        y = y.reshape(-1)
+        if y.shape[0] != A.shape[0]:
+            raise ValueError(f"linear_least_squares: y must have {A.shape[0]} entries, got {y.shape[0]}")
+    else:
+        A = np.asarray(A, dtype=np.float64)
+        y = np.asarray(y, dtype=np.float64).reshape(-1)
     n, k = A.shape
     if k + 1 > _NB:
         raise _lib.GnkError(f"linear_least_squares supports at most {_NB - 1} columns")
@@ -190,10 +206,14 @@ def linear_least_squares(A, y):
                             "2^22 doubles")
     lda = round_up(max(n, 1), 16)
     dA = rt.zeros(lda * k)
-    for j in range(k):
-        rt.upload(np.ascontiguousarray(A[:, j]), dA[j * lda:j * lda + n])
     dy = rt.zeros(lda)
-    rt.upload(y, dy[:n])
+    if on_device:
+        dA.view(k, lda)[:, :n].copy_(A.T)
+        dy[:n].copy_(y)
+    else:
+        for j in range(k):
+            rt.upload(np.ascontiguousarray(A[:, j]), dA[j * lda:j * lda + n])
+        rt.upload(y, dy[:n])
     out = rt.zeros(2 * _NB + 8)
     tsqr_solve(rt, dA, lda, n, k, dy, 1.0, out)
     vals = rt.read(out, 2 * k + 4)
@@ -201,7 +221,7 @@ def linear_least_squares(A, y):
         tsqr_solve(rt, dA, lda, n, k, dy, 1.0, out, householder=True)
         vals = rt.read(out, 2 * k + 4)
     _report_rank(vals, k)
-    return vals[:k].copy()
+    return out[:k].clone() if on_device else vals[:k].copy()
 
 
 def gauss_newton_krylow(
@@ -248,7 +268,10 @@ def gauss_newton_krylow(
     # for every other problem a DeviceVector is an ordinary array-like and is read through its host copy
     x0_resident = (isinstance(x0, DeviceVector) and x0._t is not None and BratuDeviceProblem.match(res, jac)
                    and not args and getattr(x0._owner, "pb", None) is res.pb)
-    x0_host = None if x0_resident else np.asarray(x0, dtype=np.float64).reshape(-1)
+    if x0_resident or is_cuda_tensor(x0):
+        x0_host = x0 if not x0_resident else None  # a CUDA tensor stays on the device (DeviceCallableProblem.upload_x)
+    else:
+        x0_host = np.asarray(x0, dtype=np.float64).reshape(-1)
     prob = resolve_problem(res, jac, x0 if x0_resident else x0_host, args, native_rosenbrock=True)
     require_single_rank_unless_sharded(rt, prob, "gauss_newton_krylow")
     if krylow_restart is None:
@@ -283,9 +306,12 @@ def gauss_newton_krylow(
     krylow.dev_combine(c, None, 0.0, x_trial)
     is_bratu = isinstance(prob, BratuDeviceProblem)
     native = is_bratu or getattr(prob, "device_native", False)  # res / jac have device twins: no host evaluation
+    user_code = getattr(prob, "user_code", False)  # device callables: native, but evaluated only where the reference does
     if not native:  # residual-space size of a foreign callable is known after its first evaluation
         r0 = np.asarray(res(prob.download_global(x_trial), *args), dtype=np.float64).reshape(-1)
         prob._ensure_res_layout(r0.shape[0])
+    elif user_code:
+        r0 = prob.evaluate(x_trial)
     F_cur, F_trial = prob.new_res(), prob.new_res()
     res_off = prob.res_fields["off"]
     n_res_own = prob.res_fields["n_own"]
@@ -301,7 +327,10 @@ def gauss_newton_krylow(
     if is_bratu and prob.distributed and not tensor_ls_on_every_rank(prob.sol_fields["m"], rt.world):
         ls_method = 1
 
-    if native:
+    if user_code:
+        F_cur[:n_res_own].copy_(r0)
+        prob.sumsq(F_cur, loss_slot, prob.res_lay)
+    elif native:
         prob.residual(x_trial, F_cur, loss_slot, aux=None)
     else:
         rt.upload(r0, F_cur[:n_res_own])
@@ -378,8 +407,9 @@ def gauss_newton_krylow(
             # working while the host waits for the scalars, judges the trial, runs the callback and enqueues the next
             # iteration's least squares.  A rejected first trial simply does not commit the expansion (it is redone
             # after the accepted trial; w, h, column k and the flag slot are overwritten).  Only with device-native
-            # residual / Jacobian (no host evaluation in between) and when the breakdown flag may be read late.
-            spec_ok = (native and defer_ok and iter + 1 < max_iter and iter % krylow_restart != 0
+            # residual / Jacobian (no host evaluation in between) and when the breakdown flag may be read late.  Never
+            # with the user's device callables: jac would be called at a trial point the reference may reject.
+            spec_ok = (native and not user_code and defer_ok and iter + 1 < max_iter and iter % krylow_restart != 0
                        and version in _VERSIONS and krylow.k < prob.p_glob
                        and os.environ.get("GNK_SPECULATE", "1") != "0")
             state["spec"] = None
@@ -448,11 +478,14 @@ def gauss_newton_krylow(
         # c += s d  (:98): the accepted trial's coordinates are already on the device
         c, c_next = c_next, c
 
-        xv = DeviceVector(prob, x_trial, prob.p_glob)
-        callback(x=xv, nfev=nfev, cg_iter=None)
-        xref = weakref.ref(xv)
-        del xv                      # if the callback kept x, the weak reference is still alive ...
-        DeviceVector.settle(xref)   # ... and x takes its host snapshot before the buffer is reused
+        if user_code:
+            callback(x=prob.x_out(x_trial), nfev=nfev, cg_iter=None)
+        else:
+            xv = DeviceVector(prob, x_trial, prob.p_glob)
+            callback(x=xv, nfev=nfev, cg_iter=None)
+            xref = weakref.ref(xv)
+            del xv                      # if the callback kept x, the weak reference is still alive ...
+            DeviceVector.settle(xref)   # ... and x takes its host snapshot before the buffer is reused
 
         if step_length**2 * squared_sum_d <= tol**2 * squared_sum_x_prev:
             success = True
@@ -511,5 +544,8 @@ def gauss_newton_krylow(
         print("Warning: The gauss_newton_krylow algorithm reached maximal iteration bound before terminating!")
 
     krylow.dev_combine(c, None, 0.0, x_trial)
-    x_final = DeviceVector(prob, x_trial, prob.p_glob) if x_on_device else prob.download_global(x_trial)
+    if user_code:
+        x_final = prob.x_out(x_trial)
+    else:
+        x_final = DeviceVector(prob, x_trial, prob.p_glob) if x_on_device else prob.download_global(x_trial)
     return RegressionResult("gauss newton krylow", x_final, success, nfev, njev, iter)

@@ -181,14 +181,37 @@ int gnk_tsqr_ls_method(gnk_ctx* ctx, int method);
 
 /* ---- generic sparse Jacobians (rosenbrock_problem.py:14-19, foreign callables) ----------------- */
 /* out[:, j] = sign * A * in[:, j] for a CSR matrix with n_rows rows; in columns start at
- * d_in + j*in_ld + in_off, out columns at d_out + j*out_ld + out_off.  The transpose product is the
- * same call on the CSR of A^T (the host uploads both). */
+ * d_in + j*in_ld + in_off, out columns at d_out + j*out_ld + out_off.  Each entry is sign * (the fma chain over the
+ * row in index order, from 0.0), whatever k; the matrix is read once per block of 8 columns.  The transpose
+ * product is the same call on the CSR of A^T (gnk_csr_pattern + gnk_csr_gather, or uploaded by the host). */
 int gnk_spmm_csr(gnk_ctx* ctx, int64_t n_rows, const int32_t* d_rowptr, const int32_t* d_col,
                  const double* d_val, const double* d_in, int64_t in_ld, int64_t in_off, int k,
                  double sign, double* d_out, int64_t out_ld, int64_t out_off, void* stream);
 /* out[i] = sum_j val_ij^2 per CSR row (on the CSR of A^T: diag(A^T A), gauss_newton.py:50-52). */
 int gnk_csr_row_sumsq(gnk_ctx* ctx, int64_t n_rows, const int32_t* d_rowptr, const double* d_val,
                       double* d_out, void* stream);
+
+/* Returned by gnk_csr_pattern for an index pattern that is not canonical CSR; gnk_last_error names the first
+ * defective row and the defect. */
+#define GNK_PATTERN_INVALID 3
+/* Validates a CSR index pattern (n_rows x n_cols, nnz non-zeros; int32 or int64 indices, index_bytes = 4 / 8):
+ * rowptr[0] = 0, non-decreasing, rowptr[n_rows] = nnz, 0 <= col < n_cols, strictly increasing within a row.  Then
+ * writes its int32 copy (rowptr32: n_rows + 1, col32: nnz) and the sorted transpose pattern (rowptr_t: n_cols + 1,
+ * col_t: nnz) with perm[e] = the non-zero of A at transpose position e -- a stable radix sort of the non-zeros by
+ * column, i.e. scipy's sorted csr_array(A.T).  Replaces the host transpose sp.csr_array(A.T) for Jacobians that live
+ * on the device (device.py: DeviceCsrJacobian).  n_rows, n_cols and nnz must be below 2^31 - 1.  Scratch belongs to
+ * the context.  Synchronises the stream. */
+int gnk_csr_pattern(gnk_ctx* ctx, int64_t n_rows, int64_t n_cols, int64_t nnz, const void* d_rowptr,
+                    const void* d_col, int index_bytes, int32_t* d_rowptr32, int32_t* d_col32,
+                    int32_t* d_rowptr_t, int32_t* d_col_t, int32_t* d_perm, void* stream);
+/* *d_differ = 1 if the candidate pattern (int32 / int64) differs from the int32 copy made by gnk_csr_pattern, else 0
+ * (same n_rows and nnz assumed).  Lets a Jacobian with a fixed pattern and new values skip the transpose rebuild. */
+int gnk_csr_pattern_equal(gnk_ctx* ctx, int64_t n_rows, int64_t nnz, const void* d_rowptr, const void* d_col,
+                          int index_bytes, const int32_t* d_rowptr32, const int32_t* d_col32, int32_t* d_differ,
+                          void* stream);
+/* out[e] = in[perm[e]] for n doubles: the values of A^T on the pattern of gnk_csr_pattern (replaces the value half of
+ * sp.csr_array(A.T) per Jacobian). */
+int gnk_csr_gather(gnk_ctx* ctx, int64_t n, const int32_t* d_perm, const double* d_in, double* d_out, void* stream);
 
 /* ---- small vector algebra used by the full-space solver (gauss_newton.py:123-129) -------------- */
 /* out = a*x + b*y over n doubles (x, y, out may alias). */

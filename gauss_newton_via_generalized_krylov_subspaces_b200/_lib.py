@@ -13,6 +13,7 @@ LIB_PATH = os.path.join(_HERE, "libgnk_b200.so")
 
 GNK_MAX_BASIS = 256
 GNK_TSQR_MAX = 104  # include/gnk_b200.h
+GNK_DENSE_QR_MIN, GNK_DENSE_QR_MAX = 256, 4095  # gnk_dense_qr_ls: dense least squares of 256..4095 columns
 GNK_PATTERN_INVALID = 3  # gnk_csr_pattern: the index pattern is not canonical CSR
 
 
@@ -64,6 +65,7 @@ SIGNATURES = {
     "gnk_cgs_dots": (_I, [_P, _LP, _P, _I, _P, _P, _P]),
     "gnk_cgs_update": (_I, [_P, _LP, _P, _I, _P, _P, _P, _P]),
     "gnk_tsqr_ls": (_I, [_P, _P, _L, _L, _I, _P, _D, _P, _P]),
+    "gnk_dense_qr_ls": (_I, [_P, _P, _L, _L, _I, _D, _P, _P]),
     "gnk_stencil_gram_ls": (_I, [_P, _LP, _BP, _P, _P, _L, _I, _I, _P, _D, _P, _L, _D, _P, _P]),
     "gnk_tsqr_ls_method": (_I, [_P, _I]),
     "gnk_gram_cgls": (_I, [_P, _P, _L, _L, _I, _P, _D, _D, _P, _P]),

@@ -63,6 +63,7 @@ int gnk_destroy(gnk_ctx* ctx) {
   if (ctx->d_cholqr) cudaFree(ctx->d_cholqr);
   if (ctx->d_gramw) cudaFree(ctx->d_gramw);
   if (ctx->d_pattern) cudaFree(ctx->d_pattern);
+  if (ctx->d_dqr) cudaFree(ctx->d_dqr);
   if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
   if (ctx->fetch_stream) cudaStreamDestroy(ctx->fetch_stream);
   if (ctx->fetch_event) cudaEventDestroy(ctx->fetch_event);

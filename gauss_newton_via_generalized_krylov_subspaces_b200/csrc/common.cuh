@@ -52,6 +52,9 @@ struct gnk_ctx {
   // gnk_csr_pattern (csr.cu): row of every non-zero, sort keys and values, column histogram, cub temp (grown on demand)
   void* d_pattern = nullptr;
   size_t pattern_bytes = 0;
+  // gnk_dense_qr_ls (dense_qr.cu): panel partials, pivot rows, taus, split partials of V^T C and T^T W (grown on demand)
+  double* d_dqr = nullptr;
+  size_t dqr_bytes = 0;
 };
 int gnk_ensure_fetch_stream(gnk_ctx* ctx);  // api.cu: creates fetch_stream / fetch_event on first use
 

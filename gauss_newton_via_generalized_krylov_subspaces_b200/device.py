@@ -38,7 +38,8 @@ class Runtime:
         self.ctx = ctx
         self.rank, self.world = 0, 1
         self.fused_reductions = False  # gnk_bratu_residual / gnk_cgs_dots / gnk_cgs_update reduce over the ranks themselves
-        self._pinned = torch.empty(4096, dtype=torch.float64, pin_memory=True)
+        # the largest read: the 2p + 4 result block of gnk_dense_qr_ls at p = GNK_DENSE_QR_MAX
+        self._pinned = torch.empty(2 * (_lib.GNK_DENSE_QR_MAX + 1) + 8, dtype=torch.float64, pin_memory=True)
         self._pinned_np = self._pinned.numpy()
         self._pinned_ptr = self._pinned.data_ptr()
         self._pinned2 = torch.empty(1024, dtype=torch.float64, pin_memory=True)
@@ -133,6 +134,8 @@ class Runtime:
         """small device tensor -> numpy: gnk_scalars_fetch + gnk_scalars_wait (one async copy into pinned memory behind
         everything enqueued on the current stream so far, then a wait for that copy)."""
         n = t.numel() if count is None else count
+        if n > self._pinned_np.shape[0]:
+            raise _lib.GnkError(f"scalar read-back of {n} doubles exceeds the {self._pinned_np.shape[0]}-double staging buffer")
         lib, ctx = self.lib, self.ctx
         if lib.gnk_scalars_fetch(ctx, t.data_ptr(), n, self._pinned_ptr, self.stream) or lib.gnk_scalars_wait(ctx):
             _lib.check(-1, "scalar read-back")
@@ -468,6 +471,34 @@ class CsrJacobian:
         return op
 
 
+class DenseJacobian:
+    """A dense Jacobian that gauss_newton solves with gnk_dense_qr_ls (p >= GNK_DENSE_QR_MIN columns): kept as the user
+    returned it -- ``host`` the ndarray / np.matrix, or ``user`` = ``dense`` the strided CUDA tensor -- with no CSR form.
+    The least-squares call gets it as one column-major panel (``fill_panel``)."""
+
+    is_sparse = False
+
+    def __init__(self, rt, host=None, dense=None):
+        self.rt, self.host, self.dense, self.user = rt, host, dense, dense
+        if dense is not None:
+            self.n_res, self.p = (int(v) for v in dense.shape)
+        else:
+            self.n_res, self.p = np.shape(host)
+
+    def fill_panel(self, panel):
+        """panel: (p + 1, lda) view of the column-major least-squares panel; rows :p, entries :n_res get J^T"""
+        n, p = self.n_res, self.p
+        if self.dense is not None:
+            panel[:p, :n].copy_(self.dense.T)  # one device-to-device copy (transpose, and a cast if not float64)
+            return
+        torch = self.rt.torch
+        a = np.asarray(self.host, dtype=np.float64)
+        if a.flags.f_contiguous:  # J^T is C-ordered already: upload it straight into the panel rows
+            panel[:p, :n].copy_(torch.from_numpy(a.T))
+        else:  # one upload of J, transposed on the device
+            panel[:p, :n].copy_(torch.from_numpy(np.ascontiguousarray(a)).to(panel.device).T)
+
+
 class HostCallableProblem:
     """res / jac are arbitrary Python callables returning host objects."""
 
@@ -522,11 +553,18 @@ class HostCallableProblem:
         rt = self.rt
         _lib.check(rt.lib.gnk_norm_stats(rt.ctx, C.byref(lay), ptr(vec), ptr(slot2), rt.stream), "gnk_norm_stats")
 
-    def jacobian_host(self, x_host):
+    def jacobian_host(self, x_host, dense_panel=False):
+        """jac at x_host as a CsrJacobian; with ``dense_panel`` a dense J of p >= GNK_DENSE_QR_MIN columns comes back as a
+        DenseJacobian instead (gauss_newton's blocked QR branch, which needs no CSR form)"""
         import scipy.sparse as sp
 
         J = self.jac(x_host, *self.args)
-        return CsrJacobian(self.rt, J, isinstance(J, (sp.sparray, sp.spmatrix)) or hasattr(J, "_gnk_sparse_like"))
+        sparse = isinstance(J, (sp.sparray, sp.spmatrix)) or hasattr(J, "_gnk_sparse_like")
+        if dense_panel and not sparse and not hasattr(J, "tocsr") and self.p_glob >= _lib.GNK_DENSE_QR_MIN:
+            if np.ndim(J) != 2 or np.shape(J)[1] != self.p_glob:
+                raise ValueError(f"jac: expected a 2-D Jacobian with {self.p_glob} columns, got shape {np.shape(J)}")
+            return DenseJacobian(self.rt, host=J)
+        return CsrJacobian(self.rt, J, sparse)
 
     def jacobian(self, x, aux=None):
         return self.jacobian_host(self.download_global(x))
@@ -710,8 +748,17 @@ class DeviceCallableProblem:
         rt = self.rt
         _lib.check(rt.lib.gnk_norm_stats(rt.ctx, C.byref(lay), ptr(vec), ptr(slot2), rt.stream), "gnk_norm_stats")
 
-    def jacobian(self, x, aux=None):
+    def jacobian(self, x, aux=None, dense_panel=False):
+        """jac at x as a DeviceCsrJacobian; with ``dense_panel`` a strided J of p >= GNK_DENSE_QR_MIN columns comes back
+        as a DenseJacobian instead (gauss_newton's blocked QR branch: no CSR form, no pattern)"""
         J = self.jac(self.x_out(x), *self.args)
+        torch = self.rt.torch
+        if (dense_panel and self.p_glob >= _lib.GNK_DENSE_QR_MIN and isinstance(J, torch.Tensor)
+                and J.layout == torch.strided):
+            _require_on_device(self.rt, J, "jac")
+            if tuple(J.shape) != (self.n_res, self.p_glob):
+                raise ValueError(f"jac: expected shape {(self.n_res, self.p_glob)} (n_res, p), got {tuple(J.shape)}")
+            return DenseJacobian(self.rt, dense=J)
         rowptr, col, val, is_sparse, dense = device_csr(self.rt, J, (self.n_res, self.p_glob))
         pat = self.pattern
         if pat is None or not pat.matches(self.n_res, self.p_glob, rowptr, col, self._flag):

@@ -3,8 +3,10 @@
 Sparse (or matrix-free stencil) Jacobians take the CGLS route of gauss_newton.py:11-60,111-114 -- conjugate
 gradients on the normal equations with the Jacobi preconditioner, built from the same SpMV / SpMV-transpose
 kernels as the Krylov path (``gnk_cgls``); dense Jacobians (the 2x2 / 2x1 problems of
-rosenbrock_3d_test.py and powell_divergence_test.py) take a Householder least-squares solve on the device in
-place of ``scipy.linalg.lstsq`` (:116).  ``step_length_control`` stays a plug-in point: the default
+rosenbrock_3d_test.py and powell_divergence_test.py, up to dense fits of 4095 parameters) take a Householder
+least-squares solve on the device in place of ``scipy.linalg.lstsq`` (:116): ``gnk_tsqr_ls`` up to 255 columns, the
+blocked QR ``gnk_dense_qr_ls`` for 256..4095 columns, which takes J as it comes (one copy into a column-major panel,
+no CSR form) and hands ||J d||^2 = ||R d||^2 to the Armijo rule.  ``step_length_control`` stays a plug-in point: the default
 ``armijo_goldstein`` runs device-native; a user function is called with host objects exactly like the
 reference does (:118-120).
 """
@@ -19,8 +21,8 @@ import numpy as np
 from . import _lib
 from .armijo_goldstein import armijo_device, armijo_goldstein
 from .bratu_pde_problem import BratuDeviceProblem, StencilJacobian
-from .device import (CsrJacobian, DeviceCsrJacobian, DeviceVector, _require_on_device, get_runtime, is_cuda_tensor,
-                     make_layout, ptr)
+from .device import (CsrJacobian, DenseJacobian, DeviceCsrJacobian, DeviceVector, _require_on_device, get_runtime,
+                     is_cuda_tensor, make_layout, ptr)
 from .gauss_newton_krylow import _report_rank, require_single_rank_unless_sharded, resolve_problem, tsqr_solve
 from .partition import flat_layout_fields, round_up
 from .regression_result import RegressionResult
@@ -114,7 +116,8 @@ def gauss_newton(
     Gauss Newton algorithm for minimizing ||res(theta)|| with respect to theta (reference :63-138).
 
     res: residual function res(x, *args); x0: initial guess; jac: jac(x, *args) returning ndarray or sparse
-    (sparse -> CGLS, dense -> direct least squares); step_length_control: plug-in, default Armijo-Goldstein;
+    (sparse -> CGLS, dense -> direct least squares: Householder QR on the device for up to 4095 parameters; a dense J
+    with fewer rows than columns or an exactly singular R factor raises LinAlgError); step_length_control: plug-in, default Armijo-Goldstein;
     callback(x=, nfev=, cg_iter=) once per iteration.
     """
     rt = get_runtime()
@@ -173,7 +176,8 @@ def gauss_newton(
     nfev = 1
     njev = 0
     prev_loss = float(rt.read(scal, 1)[0])
-    blk = rt.zeros(2 * _NB + 8)
+    dense_qr = not is_bratu and p >= _lib.GNK_DENSE_QR_MIN  # a dense J takes gnk_dense_qr_ls (no CSR form)
+    blk = rt.zeros(2 * max(_NB, p + 1) + 8)
     state = {}
 
     for iter in range(1, max_iter):
@@ -182,30 +186,47 @@ def gauss_newton(
             jac_ev = prob.jacobian(x, aux=aux_cur)
             sparse_like = True
         elif user_dev:
-            jac_ev = prob.jacobian(x)
+            jac_ev = prob.jacobian(x, dense_panel=dense_qr)
             sparse_like = jac_ev.is_sparse
         else:
             x_host = prob.download_global(x)
-            jac_ev = prob.jacobian_host(x_host)
+            jac_ev = prob.jacobian_host(x_host, dense_panel=dense_qr)
             sparse_like = jac_ev.is_sparse
         njev += 1
+        panel_qr = dense_qr and not sparse_like
+        if panel_qr and not isinstance(jac_ev, DenseJacobian):  # a dense object with a tocsr method of its own
+            jac_ev = DenseJacobian(rt, host=jac_ev.host)
 
         if sparse_like:
             cg_iter = _cgls(rt, jac_ev.linop(-1.0), F, 1e-4, cg_preconditioner, d, ld if is_bratu else
                             round_up(max(p, n_res), 16))
         else:
             # dense J: min ||-J d - r|| by Householder QR (reference: scipy.linalg.lstsq, full-rank case)
-            if p + 1 > _NB:
-                raise _lib.GnkError(f"dense Jacobians are supported up to {_NB - 1} columns")
+            if p > _lib.GNK_DENSE_QR_MAX:
+                raise _lib.GnkError(f"dense Jacobians are supported up to {_lib.GNK_DENSE_QR_MAX} columns")
             lda = round_up(max(n_res, 1), 16)
-            dA = rt.zeros(lda * p)
-            if user_dev:
-                dA.view(p, lda)[:, :n_res].copy_(jac_ev.dense.T)
+            if panel_qr:
+                if n_res < p:
+                    raise np.linalg.LinAlgError(
+                        f"gauss_newton: the dense Jacobian is rank deficient ({n_res} residuals for {p} parameters); the "
+                        "reference's scipy.linalg.lstsq would return the minimum-norm step here, which the device QR "
+                        "does not implement")
+                # the augmented panel [J | r], column-major; gnk_dense_qr_ls factors it in place
+                dA = rt.empty(lda * (p + 1))
+                panel = dA.view(p + 1, lda)
+                jac_ev.fill_panel(panel)
+                panel[p, :n_res].copy_(F[res_off:res_off + n_res])
+                _lib.check(lib.gnk_dense_qr_ls(rt.ctx, ptr(dA), lda, n_res, p, -1.0, ptr(blk), rt.stream),
+                           "gnk_dense_qr_ls")
             else:
-                dense = np.asfortranarray(np.asarray(jac_ev.host, dtype=np.float64))
-                for j in range(p):
-                    rt.upload(np.ascontiguousarray(dense[:, j]), dA[j * lda:j * lda + n_res])
-            tsqr_solve(rt, dA, lda, n_res, p, F[res_off:], -1.0, blk, householder=True)
+                dA = rt.zeros(lda * p)
+                if user_dev:
+                    dA.view(p, lda)[:, :n_res].copy_(jac_ev.dense.T)
+                else:
+                    dense = np.asfortranarray(np.asarray(jac_ev.host, dtype=np.float64))
+                    for j in range(p):
+                        rt.upload(np.ascontiguousarray(dense[:, j]), dA[j * lda:j * lda + n_res])
+                tsqr_solve(rt, dA, lda, n_res, p, F[res_off:], -1.0, blk, householder=True)
             # scipy.linalg.lstsq (:126) is SVD-based and returns the minimum-norm step for a rank-deficient J; the QR here
             # has no such branch, and an exactly singular R would hand inf/NaN to 100 Armijo trials.  Say so instead.
             ls_vals = rt.read(blk, 2 * p + 4)
@@ -221,11 +242,14 @@ def gauss_newton(
 
         if native_armijo:
             # g = sum((J d)^2), then trials x + s d  (armijo_goldstein.py:49-62)
-            jac_ev.matmat(d, ld, 1, Jd, ldr) if not is_bratu else prob.d.apply(
-                jac_ev.expu, d, ld, 1, -jac_ev.scale, 0, Jd, ldr, res_off)
-            prob.sumsq(Jd, scal[2:4], res_lay) if not is_bratu else _lib.check(
-                lib.gnk_norm_stats(rt.ctx, C.byref(res_lay), ptr(Jd), ptr(scal, 2), rt.stream), "gnk_norm_stats")
-            reduce(2, 2, 2)
+            if panel_qr:  # ||J d||^2 = ||R d||^2 from the least-squares block: no J d product
+                scal[2:3].copy_(blk[p:p + 1])
+            else:
+                jac_ev.matmat(d, ld, 1, Jd, ldr) if not is_bratu else prob.d.apply(
+                    jac_ev.expu, d, ld, 1, -jac_ev.scale, 0, Jd, ldr, res_off)
+                prob.sumsq(Jd, scal[2:4], res_lay) if not is_bratu else _lib.check(
+                    lib.gnk_norm_stats(rt.ctx, C.byref(res_lay), ptr(Jd), ptr(scal, 2), rt.stream), "gnk_norm_stats")
+                reduce(2, 2, 2)
             _lib.check(lib.gnk_dot(rt.ctx, p, ptr(d, off), ptr(d, off), ptr(scal, 5), rt.stream), "gnk_dot")
             reduce(5, 1)
 

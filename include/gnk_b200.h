@@ -158,6 +158,23 @@ int gnk_cgs_update(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k
 int gnk_tsqr_ls(gnk_ctx* ctx, const double* d_A, int64_t lda, int64_t n_rows, int k,
                 const double* d_y, double sign_a, double* d_out, void* stream);
 
+/* Least squares on a dense panel of GNK_DENSE_QR_MIN <= p <= GNK_DENSE_QR_MAX columns: the dense-Jacobian branch of
+ * gauss_newton, scipy.linalg.lstsq(-J, r) (gauss_newton.py:116), for Jacobians wider than gnk_tsqr_ls takes.
+ * d_A holds the augmented n_rows x (p+1) panel [A | y], column-major with stride lda (columns 0..p-1 = A, column p = y);
+ * the call solves min || sign_a*A d - y ||_2 by blocked Householder QR of [sign_a*A | y] (LAPACK dgeqrf form: panels of
+ * 32 columns factored over the SMs, compact-WY trailing updates with mma.m8n8k4.f64 on the FP64 tensor pipe, y updated
+ * with the other trailing columns).  IN PLACE: the panel is overwritten (sign_a*A's R factor in the upper triangle,
+ * the Householder vectors below it, Q^T y in column p); callers pass a scratch copy.  Result block (device, 2p+4
+ * doubles) exactly as gnk_tsqr_ls: d_out[0..p) = d, d_out[p] = ||R d||^2, d_out[p+1] = squared LS residual,
+ * d_out[p+2] = number of |R_jj| <= 1e-8, d_out[p+3] = ||d||^2, d_out[p+4 .. 2p+4) = diag(R).  Needs n_rows >= p,
+ * lda >= n_rows and 8-byte aligned columns.  Every reduction has a fixed order: repeated calls give the same bits and a
+ * power-of-two scaling of A and y changes no rounding.  One rank (the communicator is not used).  Scratch belongs to
+ * the context. */
+#define GNK_DENSE_QR_MIN 256
+#define GNK_DENSE_QR_MAX 4095
+int gnk_dense_qr_ls(gnk_ctx* ctx, double* d_A, int64_t lda, int64_t n_rows, int p, double sign_a, double* d_out,
+                    void* stream);
+
 /* Projected operator AND projected least squares of one GNK outer iteration in one call, for the Bratu stencil
  * (gauss_newton_krylow.py:86 `JV = jac_ev @ krylow.basis` followed by :89 `linear_least_squares(-1 * JV, res_ev)`):
  *   JV[:, j] = sign * (M V[:, j]), j < k   -- written (owned rows, column stride ldjv), bit-identical to gnk_stencil_apply

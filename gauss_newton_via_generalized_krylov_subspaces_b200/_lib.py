@@ -74,6 +74,8 @@ SIGNATURES = {
     "gnk_csr_pattern": (_I, [_P, _L, _L, _L, _P, _P, _I, _P, _P, _P, _P, _P, _P]),
     "gnk_csr_pattern_equal": (_I, [_P, _L, _L, _P, _P, _I, _P, _P, _P]),
     "gnk_csr_gather": (_I, [_P, _L, _P, _P, _P, _P]),
+    "gnk_dense_matmat": (_I, [_P, _L, _L, _P, _L, _L, _P, _L, _L, _I, _D, _P, _L, _L, _P]),
+    "gnk_dense_rmatvec": (_I, [_P, _L, _L, _P, _L, _L, _P, _D, _P, _P]),
     "gnk_axpby": (_I, [_P, _L, _D, _P, _D, _P, _P, _P]),
     "gnk_dot": (_I, [_P, _L, _P, _P, _P, _P]),
     "gnk_cgls": (_I, [_P, C.POINTER(LinOp), _P, _D, _I, _P, _P, C.POINTER(_L), _P]),

@@ -437,6 +437,9 @@ class CsrJacobian:
         self.host = host_J
         self.is_sparse = is_sparse
         A = host_J.tocsr() if hasattr(host_J, "tocsr") else sp.csr_array(np.asarray(host_J, dtype=np.float64))
+        if max(int(A.nnz), *(int(v) for v in A.shape)) >= _INT32_LIMIT:  # the int32 casts below would wrap silently
+            raise _lib.GnkError(f"jac: a {A.shape[0]} x {A.shape[1]} Jacobian with {A.nnz} non-zeros does not fit the "
+                                "int32 indices of the CSR kernels (every dimension and nnz must stay below 2^31 - 1)")
         A = sp.csr_array(A)
         A.sort_indices()
         AT = sp.csr_array(A.T)
@@ -572,8 +575,9 @@ class HostCallableProblem:
 
 # --------------------------------------------------------------------------------------------------
 # device callables: res / jac take and return CUDA tensors (selected by a CUDA-tensor x0).  The callables are still
-# the user's code, but x, F and J never leave HBM: the residual is copied device to device, the Jacobian's index
-# pattern and its transpose are built on the device (gnk_csr_pattern) and cached while the pattern stays the same.
+# the user's code, but x, F and J never leave HBM: the residual is copied device to device; a dense Jacobian is used
+# as it arrives (DenseDeviceJacobian), a sparse one's index pattern and its transpose are built on the device
+# (gnk_csr_pattern) and cached while the pattern stays the same.
 # --------------------------------------------------------------------------------------------------
 _INT32_LIMIT = (1 << 31) - 1  # sizes and nnz stay below: int32 indices, and n + 1 row pointers
 
@@ -591,9 +595,9 @@ def _require_on_device(rt, t, what):
 
 
 def device_csr(rt, J, shape=None, what="jac"):
-    """A CUDA Jacobian (torch sparse CSR / COO, or a strided (n_res, p) tensor) -> (rowptr, col, val, is_sparse, dense):
-    the canonical CSR of J (COO coalesced, dense without its exact zeros, as scipy.sparse.csr_array(dense)) with int32
-    or int64 indices, float64 values, and the dense tensor itself for a strided input (else None)."""
+    """A CUDA matrix (torch sparse CSR / COO, or a strided (n_res, p) tensor) -> (rowptr, col, val, is_sparse): the
+    canonical CSR of J (COO coalesced, dense without its exact zeros, as scipy.sparse.csr_array(dense)) with int32 or
+    int64 indices and float64 values."""
     torch = rt.torch
     _require_on_device(rt, J, what)
     if J.dim() != 2:
@@ -605,13 +609,11 @@ def device_csr(rt, J, shape=None, what="jac"):
     if max(n_rows, n_cols, nnz) >= _INT32_LIMIT:
         raise _lib.GnkError(f"{what}: a {n_rows} x {n_cols} Jacobian with {nnz} stored entries does not fit the int32 "
                             "indices of the CSR kernels (every dimension and nnz must stay below 2^31 - 1)")
-    dense = None
     if J.layout == torch.sparse_csr:
         A = J
     elif J.layout == torch.sparse_coo:
         A = J.coalesce().to_sparse_csr()
     elif J.layout == torch.strided:
-        dense = J
         A = J.to_sparse_csr()
     else:
         raise TypeError(f"{what}: expected a sparse_csr, sparse_coo or strided tensor, got layout {J.layout}")
@@ -621,7 +623,7 @@ def device_csr(rt, J, shape=None, what="jac"):
     if col.dtype != rowptr.dtype:
         col = col.to(rowptr.dtype)
     val = A.values().to(torch.float64).contiguous()
-    return rowptr, col, val, dense is None, dense
+    return rowptr, col, val, J.layout != torch.strided
 
 
 class CsrPattern:
@@ -657,15 +659,14 @@ class CsrPattern:
 
 class DeviceCsrJacobian:
     """J on the device as CSR of J and of J^T over a CsrPattern; J^T's values by one gather (gnk_csr_gather).  Same
-    interface as CsrJacobian.  ``user`` is the object the user's jac returned (handed to a step-length plug-in),
-    ``dense`` the strided tensor for a dense Jacobian (gauss_newton's QR branch), else None."""
+    interface as CsrJacobian.  ``user`` is the object the user's jac returned (handed to a step-length plug-in)."""
 
     transposed = False
     scale = 1.0
 
-    def __init__(self, rt, pattern, val, is_sparse, user=None, dense=None):
+    def __init__(self, rt, pattern, val, is_sparse, user=None):
         self.rt, self.pattern, self.val = rt, pattern, val
-        self.is_sparse, self.user, self.dense = is_sparse, user, dense
+        self.is_sparse, self.user = is_sparse, user
         self.n_res, self.p = pattern.n_rows, pattern.n_cols
         self.rowptr, self.col, self.rowptr_t, self.col_t = pattern.rowptr, pattern.col, pattern.rowptr_t, pattern.col_t
         self.val_t = rt.torch.empty_like(val)
@@ -674,12 +675,49 @@ class DeviceCsrJacobian:
 
     @classmethod
     def from_tensor(cls, rt, J, what="A"):
-        rowptr, col, val, is_sparse, dense = device_csr(rt, J, what=what)
-        return cls(rt, CsrPattern(rt, J.shape[0], J.shape[1], rowptr, col), val, is_sparse, J, dense)
+        rowptr, col, val, is_sparse = device_csr(rt, J, what=what)
+        return cls(rt, CsrPattern(rt, J.shape[0], J.shape[1], rowptr, col), val, is_sparse, J)
 
     matmat = CsrJacobian.matmat
     neg_rmatvec = CsrJacobian.neg_rmatvec
     linop = CsrJacobian.linop
+
+
+class DenseDeviceJacobian:
+    """A strided CUDA Jacobian used as it arrives: J V_k and -J^T r by gnk_dense_matmat / gnk_dense_rmatvec, which give
+    the bits gnk_spmm_csr gives on the CSR of the same matrix -- with no CSR form, no pattern and no copy of J^T, and
+    no int32 limit on the number of entries.  ``user`` is the tensor jac returned (handed to a step-length plug-in),
+    ``dense`` the float64 tensor the kernels read: ``user`` itself, or one contiguous float64 copy when ``user`` is of
+    another dtype or has neither stride equal to 1.  The solvers read ``dense`` until the next jac call returns, so a jac
+    may refill one tensor in place (gauss_newton_krylow forms -J_old^T r of the jac_old_* versions before that call)."""
+
+    is_sparse = False
+
+    def __init__(self, rt, J):
+        torch = rt.torch
+        self.rt, self.user = rt, J
+        self.n_res, self.p = (int(v) for v in J.shape)
+        if J.dtype != torch.float64:
+            J = J.to(torch.float64)  # keeps a dense layout's strides, makes any other layout contiguous
+        if not self._strides(J):
+            J = J.contiguous()
+        self.dense = J
+        self.rs, self.cs = self._strides(J)
+
+    def _strides(self, J):
+        """(row stride, column stride) with the stride of a dimension of size 1 taken as 1, or None if neither is 1"""
+        rs, cs = (1 if n == 1 else int(s) for n, s in zip(J.shape, J.stride()))
+        return (rs, cs) if 1 in (rs, cs) else None
+
+    def matmat(self, V, ldv, k, JV, ldjv):
+        rt = self.rt
+        _lib.check(rt.lib.gnk_dense_matmat(rt.ctx, self.n_res, self.p, ptr(self.dense), self.rs, self.cs, ptr(V), ldv, 0,
+                                           k, 1.0, ptr(JV), ldjv, 0, rt.stream), "gnk_dense_matmat")
+
+    def neg_rmatvec(self, r, w):
+        rt = self.rt
+        _lib.check(rt.lib.gnk_dense_rmatvec(rt.ctx, self.n_res, self.p, ptr(self.dense), self.rs, self.cs, ptr(r), -1.0,
+                                            ptr(w), rt.stream), "gnk_dense_rmatvec")
 
 
 class DeviceCallableProblem:
@@ -749,20 +787,24 @@ class DeviceCallableProblem:
         _lib.check(rt.lib.gnk_norm_stats(rt.ctx, C.byref(lay), ptr(vec), ptr(slot2), rt.stream), "gnk_norm_stats")
 
     def jacobian(self, x, aux=None, dense_panel=False):
-        """jac at x as a DeviceCsrJacobian; with ``dense_panel`` a strided J of p >= GNK_DENSE_QR_MIN columns comes back
-        as a DenseJacobian instead (gauss_newton's blocked QR branch: no CSR form, no pattern)"""
+        """jac at x: a strided J as a DenseDeviceJacobian -- or, with ``dense_panel`` and p >= GNK_DENSE_QR_MIN, as a
+        DenseJacobian (gauss_newton's blocked QR branch) -- and a sparse J as a DeviceCsrJacobian"""
         J = self.jac(self.x_out(x), *self.args)
         torch = self.rt.torch
-        if (dense_panel and self.p_glob >= _lib.GNK_DENSE_QR_MIN and isinstance(J, torch.Tensor)
-                and J.layout == torch.strided):
+        if isinstance(J, torch.Tensor) and J.layout == torch.strided:
             _require_on_device(self.rt, J, "jac")
+            panel = dense_panel and self.p_glob >= _lib.GNK_DENSE_QR_MIN
             if tuple(J.shape) != (self.n_res, self.p_glob):
+                if J.dim() != 2 and not panel:
+                    raise ValueError(f"jac: expected a 2-D Jacobian, got shape {tuple(J.shape)}")
                 raise ValueError(f"jac: expected shape {(self.n_res, self.p_glob)} (n_res, p), got {tuple(J.shape)}")
-            return DenseJacobian(self.rt, dense=J)
-        rowptr, col, val, is_sparse, dense = device_csr(self.rt, J, (self.n_res, self.p_glob))
+            if panel:
+                return DenseJacobian(self.rt, dense=J)
+            return DenseDeviceJacobian(self.rt, J)
+        rowptr, col, val, is_sparse = device_csr(self.rt, J, (self.n_res, self.p_glob))
         pat = self.pattern
         if pat is None or not pat.matches(self.n_res, self.p_glob, rowptr, col, self._flag):
             pat = CsrPattern(self.rt, self.n_res, self.p_glob, rowptr, col)
             self.pattern = pat
             self.pattern_builds += 1
-        return DeviceCsrJacobian(self.rt, pat, val, is_sparse, J, dense)
+        return DeviceCsrJacobian(self.rt, pat, val, is_sparse, J)

@@ -493,6 +493,13 @@ def gauss_newton_krylow(
 
         jac_ev_old = jac_ev
         speculated = state["spec"] is not None and state["spec"] is not False
+        # device callables, jac_old_*: -J_old^T r is formed before jac is called at the new point, so that a jac which
+        # refills the tensor it returned last time cannot change J_old under the expansion (same bits, earlier)
+        w_ready = (user_code and not speculated and version in ("jac_old_res_old", "jac_old_res_new")
+                   and krylow.k < prob.p_glob)
+        if w_ready:
+            krylow.dev_rmatvec(jac_ev_old, F_cur if version == "jac_old_res_old" else F_trial)
+            jac_ev_old = None
         jac_ev = state["spec"] if speculated else prob.jacobian(x_trial, aux=aux[1])  # e^x came out of the trial
         njev += 1
 

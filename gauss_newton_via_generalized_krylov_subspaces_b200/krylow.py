@@ -106,21 +106,26 @@ class GeneralizedKrylowSubspace:
                                                ptr(out), ptr(c_out), cprev2 if cprev2 is not None else ptr(None),
                                                rt.stream), "gnk_combine")
 
+    def dev_rmatvec(self, jac_op, r):
+        """w = -J^T r alone, for a following expansion called with ``jac_op=None``"""
+        with self.rt.mark("spmv_t", 24.0 * self.fields["n_own"]):
+            jac_op.neg_rmatvec(r, self.w)
+
     def dev_expand_enqueue(self, jac_op, r, halo_exchange=None, flag_ptr=None):
         """Enqueue the basis expansion with -J^T r orthogonalised against V_k (krylow.py:55-73) WITHOUT committing it:
         the normalised vector lands in column k of the storage, the breakdown flag of krylow.py:66 in ``flag_ptr`` (a
         device int32; default: this object's own flag), and ``k`` is unchanged until ``commit()``.  Nothing is read
         back, so the caller may enqueue it speculatively (gauss_newton_krylow does, before it knows whether the Armijo
         trial is accepted) -- an expansion that is not committed leaves no trace: w, h, the statistics, column k and the
-        flag are all overwritten by the next one."""
+        flag are all overwritten by the next one.  ``jac_op=None``: w already holds -J^T r (``dev_rmatvec``)."""
         if self.k == self.n_glob:
             raise GeneralizedKrylowSubspaceSpansEntireSpace
         rt, lib = self.rt, self.rt.lib
         if self.k == self.cap:
             self._grow()
         n = self.fields["n_own"]
-        with rt.mark("spmv_t", 24.0 * n):
-            jac_op.neg_rmatvec(r, self.w)
+        if jac_op is not None:
+            self.dev_rmatvec(jac_op, r)
         for ipass in range(self.reorth_passes):
             with rt.mark("cgs_dots", 8.0 * n * (self.k + 1)):
                 _lib.check(lib.gnk_cgs_dots(rt.ctx, C.byref(self.lay), ptr(self.V), self.k, ptr(self.w),

@@ -230,6 +230,23 @@ int gnk_csr_pattern_equal(gnk_ctx* ctx, int64_t n_rows, int64_t nnz, const void*
  * sp.csr_array(A.T) per Jacobian). */
 int gnk_csr_gather(gnk_ctx* ctx, int64_t n, const int32_t* d_perm, const double* d_in, double* d_out, void* stream);
 
+/* ---- dense Jacobians (strided CUDA tensors from device callables, used without a CSR form) ---------- */
+/* J is n_rows x n_cols (both below 2^31 - 1; n_rows * n_cols may exceed 2^31), entry (i, c) at
+ * d_J[i * row_stride + c * col_stride], one of the two strides 1 (row-major or column-major; the other is any
+ * stride >= 0).  Every output is sign * (the fma chain from 0.0 over the entries != 0.0 of the row / column of J in
+ * ascending index order): bit for bit what gnk_spmm_csr gives on the CSR of J / on the sorted CSR of J^T, which drop
+ * exact zeros (+0.0 and -0.0) and keep NaN.  One launch, no synchronisation.
+ * gnk_dense_matmat: out[:, j] = sign * J @ in[:, j] for j < k, with in / out columns as in gnk_spmm_csr (d_in + j*in_ld
+ * + in_off, d_out + j*out_ld + out_off).  A CTA stages tiles of J and of the basis through shared memory and keeps a
+ * register tile of outputs; one pass carries up to 2 / 4 / 16 / 32 basis columns for k <= 2 / 4 / 16 / 32, passes of
+ * 64 columns above (k <= 255: at most 4, adjacent in the grid so that J is read from HBM about once). */
+int gnk_dense_matmat(gnk_ctx* ctx, int64_t n_rows, int64_t n_cols, const double* d_J, int64_t row_stride,
+                     int64_t col_stride, const double* d_in, int64_t in_ld, int64_t in_off, int k, double sign,
+                     double* d_out, int64_t out_ld, int64_t out_off, void* stream);
+/* gnk_dense_rmatvec: out[c] = sign * (J^T r)[c], c < n_cols; one sequential chain of n_rows steps per column. */
+int gnk_dense_rmatvec(gnk_ctx* ctx, int64_t n_rows, int64_t n_cols, const double* d_J, int64_t row_stride,
+                      int64_t col_stride, const double* d_r, double sign, double* d_out, void* stream);
+
 /* ---- small vector algebra used by the full-space solver (gauss_newton.py:123-129) -------------- */
 /* out = a*x + b*y over n doubles (x, y, out may alias). */
 int gnk_axpby(gnk_ctx* ctx, int64_t n, double a, const double* d_x, double b, const double* d_y,

@@ -34,7 +34,7 @@ class LinOp(C.Structure):
     _fields_ = [("kind", C.c_int32), ("pad_", C.c_int32), ("sign", C.c_double), ("lay", Layout), ("prm", Bratu),
                 ("d_expu", C.c_void_p), ("n_res", C.c_int64), ("p", C.c_int64), ("d_rowptr", C.c_void_p),
                 ("d_col", C.c_void_p), ("d_val", C.c_void_p), ("d_rowptr_t", C.c_void_p), ("d_col_t", C.c_void_p),
-                ("d_val_t", C.c_void_p)]
+                ("d_val_t", C.c_void_p), ("d_dense", C.c_void_p), ("row_stride", C.c_int64), ("col_stride", C.c_int64)]
 
 
 _P = C.c_void_p
@@ -76,6 +76,7 @@ SIGNATURES = {
     "gnk_csr_gather": (_I, [_P, _L, _P, _P, _P, _P]),
     "gnk_dense_matmat": (_I, [_P, _L, _L, _P, _L, _L, _P, _L, _L, _I, _D, _P, _L, _L, _P]),
     "gnk_dense_rmatvec": (_I, [_P, _L, _L, _P, _L, _L, _P, _D, _P, _P]),
+    "gnk_dense_col_sumsq": (_I, [_P, _L, _L, _P, _L, _L, _P, _P]),
     "gnk_axpby": (_I, [_P, _L, _D, _P, _D, _P, _P, _P]),
     "gnk_dot": (_I, [_P, _L, _P, _P, _P, _P]),
     "gnk_cgls": (_I, [_P, C.POINTER(LinOp), _P, _D, _I, _P, _P, C.POINTER(_L), _P]),

@@ -5,7 +5,8 @@
 // unpreconditioned CG whose solution is thrown away (gauss_newton.py:45-48) and then ALWAYS runs the
 // preconditioned one (:50-58); the reported iteration count is the sum.
 // A = sign*P for the Bratu stencil (matrix free; A p and A^T t are the same SpMV / SpMV-transpose kernels the
-// Krylov path uses) or a CSR pair for generic Jacobians.  All scalars (rho, p.q, alpha, beta) stay on the
+// Krylov path uses), a CSR pair for generic Jacobians, or a dense matrix read in place (the dense_jac.cu kernels, which
+// give the bits of the CSR pair of the same matrix).  All scalars (rho, p.q, alpha, beta) stay on the
 // device; the host reads one double (||r||^2) per iteration for the stopping test -- one iteration LATE: iteration i + 1
 // is queued before the test of iteration i is looked at, and the two kernels that change the CG state (direction, step)
 // repeat the test on the device and do nothing once it has fired, so the device never waits for the host and the result
@@ -111,6 +112,13 @@ struct Cg {
       return gnk_stencil_apply(ctx, &op->lay, &op->prm, op->d_expu, in, op->lay.ld, 1, op->sign, transpose, out,
                                op->lay.ld, op->lay.off, st);
     }
+    if (op->kind == 2) {
+      if (!transpose)
+        return gnk_dense_matmat(ctx, op->n_res, op->p, op->d_dense, op->row_stride, op->col_stride, in, 0, 0, 1,
+                                op->sign, out, 0, 0, st);
+      return gnk_dense_rmatvec(ctx, op->n_res, op->p, op->d_dense, op->row_stride, op->col_stride, in, op->sign, out,
+                               st);
+    }
     if (!transpose)
       return gnk_spmm_csr(ctx, op->n_res, op->d_rowptr, op->d_col, op->d_val, in, 0, 0, 1, op->sign, out, 0, 0, st);
     return gnk_spmm_csr(ctx, op->p, op->d_rowptr_t, op->d_col_t, op->d_val_t, in, 0, 0, 1, op->sign, out, 0, 0, st);
@@ -150,7 +158,8 @@ extern "C" int gnk_cgls_x0(gnk_ctx* ctx, const gnk_linop* op, const double* d_y,
                            int preconditioner, double* d_x, double* d_work, int64_t* iters, void* stream) {
   GNK_REQUIRE(ctx && op && d_y && d_x && d_work && iters, "gnk_cgls: null argument");
   GNK_REQUIRE(d_x0 != d_x, "gnk_cgls: x0 and x must not alias (x0 is read again by the second run)");
-  GNK_REQUIRE(op->kind == 0 || op->kind == 1, "gnk_cgls: unknown operator kind");
+  GNK_REQUIRE(op->kind == 0 || op->kind == 1 || op->kind == 2, "gnk_cgls: unknown operator kind");
+  GNK_REQUIRE(op->kind != 2 || ctx->nranks == 1, "gnk_cgls: a dense operator runs on one rank");
   Cg cg;
   cg.ctx = ctx;
   cg.op = op;
@@ -208,7 +217,12 @@ extern "C" int gnk_cgls_x0(gnk_ctx* ctx, const gnk_linop* op, const double* d_y,
         if (op->sign * op->sign != 1.0)
           if (int rc = gnk_axpby(ctx, n, op->sign * op->sign, dinv + o, 0.0, nullptr, dinv + o, st)) return rc;
       } else {
-        if (int rc = gnk_csr_row_sumsq(ctx, op->p, op->d_rowptr_t, op->d_val_t, dinv, st)) return rc;
+        if (op->kind == 1) {
+          if (int rc = gnk_csr_row_sumsq(ctx, op->p, op->d_rowptr_t, op->d_val_t, dinv, st)) return rc;
+        } else {
+          if (int rc = gnk_dense_col_sumsq(ctx, op->n_res, op->p, op->d_dense, op->row_stride, op->col_stride, dinv, st))
+            return rc;
+        }
         if (op->sign * op->sign != 1.0)
           if (int rc = gnk_axpby(ctx, n, op->sign * op->sign, dinv, 0.0, nullptr, dinv, st)) return rc;
       }

@@ -3,10 +3,13 @@
 //   gnk_dense_matmat   out[:, j] = sign * J @ in[:, j], j < k      (J @ V_k, gauss_newton_krylow.py:86; J d of the
 //                                                                  Armijo rule, gauss_newton.py)
 //   gnk_dense_rmatvec  out = sign * J^T @ r                        (-J^T r, krylow.py:62)
+//   gnk_dense_col_sumsq out[c] = sum_i J[i, c]^2                    (diag(A^T A), the Jacobi preconditioner of
+//                                                                  cg_least_squares, gauss_newton.py:50-52)
 // Bits: every output is sign * acc, acc an fma chain from 0.0 over the NON-ZERO entries of its row of J (matmat) or
 // column of J (rmatvec) in ascending index order -- exactly what gnk_spmm_csr computes on the CSR of J resp. on the
 // sorted CSR of J^T, because CSR drops exact zeros (+0.0 and -0.0) and keeps NaN.  So an entry a takes part iff
-// a != 0.0.  No FP64 tensor-core MMA: its partial sums round differently.
+// a != 0.0.  gnk_dense_col_sumsq is the fma(a, a, acc) chain of gnk_csr_row_sumsq on the sorted CSR of J^T (skipping
+// +-0.0 cannot change that sum; NaN is kept).  No FP64 tensor-core MMA: its partial sums round differently.
 #include "common.cuh"
 
 namespace {
@@ -120,21 +123,114 @@ cudaError_t launch_matmat(bool row_major, int64_t n_rows, int64_t n_cols, const 
   return cudaGetLastError();
 }
 
-// ---- J^T @ r -----------------------------------------------------------------------------------------------------
+// ---- J @ v, one column (k = 1: the A p of every CG iteration, the J d of the Armijo rule) -----------------------
+// The smallest dense_matmat_kernel configuration carries two basis columns, one stage of look-ahead and 256 rows per
+// CTA; with few rows (8192 x 8192) that leaves most SMs idle: 0.07 of the HBM bound on a B200, against 0.33 here.  On
+// tall matrices both reach 0.50 (DESIGN.md section 6).  Here a CTA owns BM rows, one chain per row run by threads 0..BM-1, and all 256 threads
+// keep MV_STAGES - 1 tiles of BM rows x BK = MV_TILE / BM columns (and the matching entries of v) in flight with
+// cp.async, coalesced along rows for row-major J and along columns for column-major J.  Each thread issues its loads
+// at the same place of every tile, so its addresses advance by a constant.  Few rows (fewer CTAs than the SMs can
+// hold) take BM = 32: more CTAs, and 512-byte row segments.
+constexpr int MV_THREADS = 256, MV_TILE = 2048, MV_STAGES = 4;
+
+constexpr size_t matvec_smem(int bm) { return sizeof(double) * MV_STAGES * (MV_TILE / bm) * (bm + 2); }
+
+template <int BM, bool ROW_MAJOR>
+__global__ void __launch_bounds__(MV_THREADS) dense_matvec_kernel(int64_t n_rows, int64_t n_cols,
+                                                                   const double* __restrict__ J, int64_t rs,
+                                                                   int64_t cs, const double* __restrict__ v,
+                                                                   double sign, double* __restrict__ out) {
+  constexpr int BK = MV_TILE / BM, PER = MV_TILE / MV_THREADS;
+  static_assert(MV_THREADS % BM == 0 && MV_THREADS % BK == 0, "tile mapping");
+  extern __shared__ double mv_smem[];
+  auto Js = reinterpret_cast<double(*)[BK][BM + 1]>(mv_smem);              // [MV_STAGES][BK][BM + 1], J transposed
+  auto Xs = reinterpret_cast<double(*)[BK]>(mv_smem + MV_STAGES * BK * (BM + 1));  // [MV_STAGES][BK]
+  const int tid = threadIdx.x;
+  const int64_t row0 = (int64_t)blockIdx.x * BM;
+  const int64_t tiles = (n_cols + BK - 1) / BK;
+  // load m of this thread in every tile: row i0 + m * DI, column c0 + m * DC of the tile
+  const int i0 = ROW_MAJOR ? tid / BK : tid % BM, c0 = ROW_MAJOR ? tid % BK : tid / BM;
+  constexpr int DI = ROW_MAJOR ? MV_THREADS / BK : 0, DC = ROW_MAJOR ? 0 : MV_THREADS / BM;
+
+  auto load = [&](int64_t t) {
+    if (t >= tiles) return;
+    const int buf = (int)(t % MV_STAGES);
+    const int64_t cb = t * BK;
+#pragma unroll
+    for (int m = 0; m < PER; ++m) {
+      const int i = i0 + m * DI, c = c0 + m * DC;
+      const int64_t rr = row0 + i, cc = cb + c;
+      const bool ok = rr < n_rows && cc < n_cols;
+      cp_async8(&Js[buf][c][i], ok ? J + rr * rs + cc * cs : J, ok);
+    }
+    if (tid < BK) {
+      const bool ok = cb + tid < n_cols;
+      cp_async8(&Xs[buf][tid], ok ? v + cb + tid : v, ok);
+    }
+  };
+
+#pragma unroll
+  for (int s = 0; s < MV_STAGES - 1; ++s) {
+    load(s);
+    cp_async_commit();
+  }
+  double acc = 0.0;
+  for (int64_t t = 0; t < tiles; ++t) {
+    cp_async_wait<MV_STAGES - 2>();
+    __syncthreads();  // tile t has landed, and the chains of tile t - 1 are done with their buffer
+    load(t + MV_STAGES - 1);
+    cp_async_commit();
+    if (tid < BM) {
+      const int buf = (int)(t % MV_STAGES);
+#pragma unroll
+      for (int c = 0; c < BK; ++c) {
+        const double a = Js[buf][c][tid];
+        if (a != 0.0) acc = fma(a, Xs[buf][c], acc);
+      }
+    }
+  }
+  if (tid < BM && row0 + tid < n_rows) out[row0 + tid] = sign * acc;
+}
+
+template <int BM>
+int launch_matvec(gnk_ctx* ctx, bool row_major, int64_t n_rows, int64_t n_cols, const double* J, int64_t rs,
+                  int64_t cs, const double* v, double sign, double* out, cudaStream_t st) {
+  auto kern = row_major ? dense_matvec_kernel<BM, true> : dense_matvec_kernel<BM, false>;
+  static bool attr_set[2][64] = {};  // per layout and device
+  bool& set = attr_set[row_major ? 1 : 0][ctx->device & 63];
+  if (!set) {
+    GNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)matvec_smem(BM)));
+    set = true;
+  }
+  const int64_t blocks = ceil_div(n_rows, BM);
+  if (blocks > INT32_MAX) return gnk_fail("kernel launch", cudaErrorInvalidConfiguration, __FILE__, __LINE__);
+  kern<<<(unsigned)blocks, MV_THREADS, matvec_smem(BM), st>>>(n_rows, n_cols, J, rs, cs, v, sign, out);
+  GNK_LAUNCH_CHECK(ctx);
+  return 0;
+}
+
+int launch_matvec_sized(gnk_ctx* ctx, bool row_major, int64_t n_rows, int64_t n_cols, const double* J, int64_t rs,
+                        int64_t cs, const double* v, double sign, double* out, cudaStream_t st) {
+  if (ceil_div(n_rows, 256) >= 3 * (int64_t)ctx->sm_count)
+    return launch_matvec<256>(ctx, row_major, n_rows, n_cols, J, rs, cs, v, sign, out, st);
+  return launch_matvec<32>(ctx, row_major, n_rows, n_cols, J, rs, cs, v, sign, out, st);
+}
+
+// ---- J^T @ r and the squared column norms --------------------------------------------------------------------------
 // The bit contract fixes one sequential chain of n_rows steps per column of J, so the parallelism is n_cols threads.
 // A CTA owns RV_CW = 16 columns: all 256 threads keep RV_STAGES - 1 tiles of RV_R rows x 16 columns (and the matching
 // entries of r) in flight with cp.async -- 128-byte row segments for row-major J, 512-byte column segments for
 // column-major J -- while 16 threads run the chains out of shared memory.  The time is about n_rows dependent FMA
-// latencies unless n_cols is large enough for the loads to saturate HBM.
+// latencies unless n_cols is large enough for the loads to saturate HBM.  SQUARE: the chain is fma(a, a, acc) and r is
+// neither read nor loaded (gnk_dense_col_sumsq).
 constexpr int RV_THREADS = 256, RV_CW = 16, RV_R = 64, RV_STAGES = 5;
 
-template <bool ROW_MAJOR>
-__global__ void __launch_bounds__(RV_THREADS) dense_rmatvec_kernel(int64_t n_rows, int64_t n_cols,
-                                                                    const double* __restrict__ J, int64_t rs,
-                                                                    int64_t cs, const double* __restrict__ r,
-                                                                    double sign, double* __restrict__ out) {
+template <bool ROW_MAJOR, bool SQUARE>
+__device__ __forceinline__ void column_chains(int64_t n_rows, int64_t n_cols, const double* __restrict__ J, int64_t rs,
+                                              int64_t cs, const double* __restrict__ r, double sign,
+                                              double* __restrict__ out) {
   __shared__ double Js[RV_STAGES][RV_R][RV_CW + 1];
-  __shared__ double Rs[RV_STAGES][RV_R];
+  __shared__ double Rs[SQUARE ? 1 : RV_STAGES][RV_R];
   const int tid = threadIdx.x;
   const int64_t c0 = (int64_t)blockIdx.x * RV_CW;
   const int64_t tiles = (n_rows + RV_R - 1) / RV_R;
@@ -149,7 +245,7 @@ __global__ void __launch_bounds__(RV_THREADS) dense_rmatvec_kernel(int64_t n_row
       const bool ok = rr < n_rows && cc < n_cols;
       cp_async8(&Js[buf][i][c], ok ? J + rr * rs + cc * cs : J, ok);
     }
-    if (tid < RV_R) {
+    if (!SQUARE && tid < RV_R) {
       const bool ok = row0 + tid < n_rows;
       cp_async8(&Rs[buf][tid], ok ? r + row0 + tid : r, ok);
     }
@@ -171,11 +267,26 @@ __global__ void __launch_bounds__(RV_THREADS) dense_rmatvec_kernel(int64_t n_row
 #pragma unroll 8
       for (int i = 0; i < RV_R; ++i) {
         const double a = Js[buf][i][tid];
-        if (a != 0.0) acc = fma(a, Rs[buf][i], acc);
+        if (a != 0.0) acc = fma(a, SQUARE ? a : Rs[buf][i], acc);
       }
     }
   }
-  if (tid < RV_CW && c0 + tid < n_cols) out[c0 + tid] = sign * acc;
+  if (tid < RV_CW && c0 + tid < n_cols) out[c0 + tid] = SQUARE ? acc : sign * acc;
+}
+
+template <bool ROW_MAJOR>
+__global__ void __launch_bounds__(RV_THREADS) dense_rmatvec_kernel(int64_t n_rows, int64_t n_cols,
+                                                                    const double* __restrict__ J, int64_t rs,
+                                                                    int64_t cs, const double* __restrict__ r,
+                                                                    double sign, double* __restrict__ out) {
+  column_chains<ROW_MAJOR, false>(n_rows, n_cols, J, rs, cs, r, sign, out);
+}
+
+template <bool ROW_MAJOR>
+__global__ void __launch_bounds__(RV_THREADS) dense_col_sumsq_kernel(int64_t n_rows, int64_t n_cols,
+                                                                      const double* __restrict__ J, int64_t rs,
+                                                                      int64_t cs, double* __restrict__ out) {
+  column_chains<ROW_MAJOR, true>(n_rows, n_cols, J, rs, cs, nullptr, 1.0, out);
 }
 
 bool dense_layout_ok(int64_t n_rows, int64_t n_cols, int64_t rs, int64_t cs) {
@@ -200,8 +311,12 @@ int gnk_dense_matmat(gnk_ctx* ctx, int64_t n_rows, int64_t n_cols, const double*
   if (n_rows == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   const bool rm = row_major(n_cols, row_stride, col_stride);
+  if (k == 1)
+    return launch_matvec_sized(ctx, rm, n_rows, n_cols, d_J, row_stride, col_stride, d_in + in_off, sign,
+                               d_out + out_off, st);
   cudaError_t e;
-  // basis columns one pass carries: 2 / 4 / 16 / 32 while k fits, then passes of 64 columns (k <= 255: at most 4)
+  // basis columns one pass carries: 1 (dense_matvec_kernel) / 2 / 4 / 16 / 32 while k fits, then passes of 64 columns
+  // (k <= 255: at most 4)
   if (k <= 2)
     e = launch_matmat<1, 2, 1, 8>(rm, n_rows, n_cols, d_J, row_stride, col_stride, d_in, in_ld, in_off, k, sign, d_out,
                                   out_ld, out_off, st);
@@ -237,6 +352,22 @@ int gnk_dense_rmatvec(gnk_ctx* ctx, int64_t n_rows, int64_t n_cols, const double
   else
     dense_rmatvec_kernel<false><<<grid, RV_THREADS, 0, st>>>(n_rows, n_cols, d_J, row_stride, col_stride, d_r, sign,
                                                              d_out);
+  GNK_LAUNCH_CHECK(ctx);
+  return 0;
+}
+
+int gnk_dense_col_sumsq(gnk_ctx* ctx, int64_t n_rows, int64_t n_cols, const double* d_J, int64_t row_stride,
+                        int64_t col_stride, double* d_out, void* stream) {
+  GNK_REQUIRE(ctx && d_J && d_out, "gnk_dense_col_sumsq: null argument");
+  GNK_REQUIRE(dense_layout_ok(n_rows, n_cols, row_stride, col_stride),
+              "gnk_dense_col_sumsq: bad sizes or strides (n_rows, n_cols < 2^31 - 1; one stride must be 1)");
+  if (n_cols == 0) return 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  const unsigned grid = (unsigned)ceil_div(n_cols, RV_CW);
+  if (row_major(n_cols, row_stride, col_stride))
+    dense_col_sumsq_kernel<true><<<grid, RV_THREADS, 0, st>>>(n_rows, n_cols, d_J, row_stride, col_stride, d_out);
+  else
+    dense_col_sumsq_kernel<false><<<grid, RV_THREADS, 0, st>>>(n_rows, n_cols, d_J, row_stride, col_stride, d_out);
   GNK_LAUNCH_CHECK(ctx);
   return 0;
 }

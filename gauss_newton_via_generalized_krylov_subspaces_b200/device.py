@@ -719,6 +719,15 @@ class DenseDeviceJacobian:
         _lib.check(rt.lib.gnk_dense_rmatvec(rt.ctx, self.n_res, self.p, ptr(self.dense), self.rs, self.cs, ptr(r), -1.0,
                                             ptr(w), rt.stream), "gnk_dense_rmatvec")
 
+    def linop(self, sign):
+        """the kind-2 gnk_linop of sign * J for gnk_cgls: the matrix read in place, no CSR pair"""
+        op = _lib.LinOp()
+        op.kind = 2
+        op.sign = sign
+        op.n_res, op.p = self.n_res, self.p
+        op.d_dense, op.row_stride, op.col_stride = ptr(self.dense), self.rs, self.cs
+        return op
+
 
 class DeviceCallableProblem:
     """res / jac are Python callables on CUDA tensors: res(x, *args) -> 1-D tensor of n_res values, jac(x, *args) ->

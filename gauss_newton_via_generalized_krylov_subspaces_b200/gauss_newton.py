@@ -21,8 +21,8 @@ import numpy as np
 from . import _lib
 from .armijo_goldstein import armijo_device, armijo_goldstein
 from .bratu_pde_problem import BratuDeviceProblem, StencilJacobian
-from .device import (CsrJacobian, DenseJacobian, DeviceCsrJacobian, DeviceVector, _require_on_device, get_runtime,
-                     is_cuda_tensor, make_layout, ptr)
+from .device import (_INT32_LIMIT, CsrJacobian, DenseDeviceJacobian, DenseJacobian, DeviceCsrJacobian, DeviceVector,
+                     _require_on_device, get_runtime, is_cuda_tensor, make_layout, ptr)
 from .gauss_newton_krylow import _report_rank, require_single_rank_unless_sharded, resolve_problem, tsqr_solve
 from .partition import flat_layout_fields, round_up
 from .regression_result import RegressionResult
@@ -38,16 +38,31 @@ def _cgls(rt, linop, y, rtol, preconditioner, x_out, vlen, x0=None):
     return int(iters.value)
 
 
+def _device_operator(rt, A, what="cg_least_squares: A"):
+    """a CUDA A -> DenseDeviceJacobian (strided) or DeviceCsrJacobian (sparse CSR / COO)"""
+    if A.layout != rt.torch.strided:
+        return DeviceCsrJacobian.from_tensor(rt, A, what)
+    _require_on_device(rt, A, what)
+    if A.dim() != 2:
+        raise ValueError(f"{what}: expected a 2-D Jacobian, got shape {tuple(A.shape)}")
+    if max(A.shape) >= _INT32_LIMIT:
+        raise _lib.GnkError(f"{what}: a {A.shape[0]} x {A.shape[1]} matrix does not fit the dense kernels (n_res and p "
+                            "must stay below 2^31 - 1; their product may be larger)")
+    return DenseDeviceJacobian(rt, A)
+
+
 def cg_least_squares(A, y, x0=None, cg_rtol=1e-4, preconditioner=True):
     """Iterative solver for min ||y - A x|| via CG on the normal equations (reference :11-60), on the device.
 
     A: scipy sparse matrix / ndarray / device stencil operator, y: ndarray -- or A: CUDA tensor (torch sparse CSR / COO,
-    or dense), y (and x0): CUDA tensors, and x comes back as a CUDA tensor.  Returns (x, cg_iter) where cg_iter
+    or dense), y (and x0): CUDA tensors, and x comes back as a CUDA tensor.  A dense CUDA A is read in place (one
+    contiguous float64 copy if it is of another dtype or has no unit stride), with no CSR form and no limit on its number
+    of entries; the result is the one its CSR form gives, bit for bit.  Returns (x, cg_iter) where cg_iter
     sums the unpreconditioned and the preconditioned run when ``preconditioner`` is False (reference quirk)."""
     rt = get_runtime()
     if is_cuda_tensor(A):
         require_single_rank_unless_sharded(rt, None, "cg_least_squares")
-        op = DeviceCsrJacobian.from_tensor(rt, A, "cg_least_squares: A")
+        op = _device_operator(rt, A)
         _require_on_device(rt, y, "cg_least_squares: y")
         y = y.reshape(-1)
         if y.shape[0] != op.n_res:

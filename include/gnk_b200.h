@@ -239,13 +239,18 @@ int gnk_csr_gather(gnk_ctx* ctx, int64_t n, const int32_t* d_perm, const double*
  * gnk_dense_matmat: out[:, j] = sign * J @ in[:, j] for j < k, with in / out columns as in gnk_spmm_csr (d_in + j*in_ld
  * + in_off, d_out + j*out_ld + out_off).  A CTA stages tiles of J and of the basis through shared memory and keeps a
  * register tile of outputs; one pass carries up to 2 / 4 / 16 / 32 basis columns for k <= 2 / 4 / 16 / 32, passes of
- * 64 columns above (k <= 255: at most 4, adjacent in the grid so that J is read from HBM about once). */
+ * 64 columns above (k <= 255: at most 4, adjacent in the grid so that J is read from HBM about once).  k = 1 takes a
+ * kernel of its own: one chain per row, fed by a four-stage cp.async ring. */
 int gnk_dense_matmat(gnk_ctx* ctx, int64_t n_rows, int64_t n_cols, const double* d_J, int64_t row_stride,
                      int64_t col_stride, const double* d_in, int64_t in_ld, int64_t in_off, int k, double sign,
                      double* d_out, int64_t out_ld, int64_t out_off, void* stream);
 /* gnk_dense_rmatvec: out[c] = sign * (J^T r)[c], c < n_cols; one sequential chain of n_rows steps per column. */
 int gnk_dense_rmatvec(gnk_ctx* ctx, int64_t n_rows, int64_t n_cols, const double* d_J, int64_t row_stride,
                       int64_t col_stride, const double* d_r, double sign, double* d_out, void* stream);
+/* gnk_dense_col_sumsq: out[c] = sum_i J[i, c]^2, c < n_cols: the Jacobi diagonal diag(J^T J), bit for bit
+ * gnk_csr_row_sumsq on the sorted CSR of J^T (one fma(a, a, acc) chain per column from 0.0, rows ascending). */
+int gnk_dense_col_sumsq(gnk_ctx* ctx, int64_t n_rows, int64_t n_cols, const double* d_J, int64_t row_stride,
+                        int64_t col_stride, double* d_out, void* stream);
 
 /* ---- small vector algebra used by the full-space solver (gauss_newton.py:123-129) -------------- */
 /* out = a*x + b*y over n doubles (x, y, out may alias). */
@@ -255,25 +260,33 @@ int gnk_dot(gnk_ctx* ctx, int64_t n, const double* d_x, const double* d_y, doubl
 
 /* ---- CGLS (gauss_newton.py:11-60 on top of scipy.sparse.linalg.cg) ------------------------------ */
 typedef struct {
-  int32_t kind;      /* 0 = Bratu stencil (A = sign*P), 1 = CSR pair                                */
+  int32_t kind;      /* 0 = Bratu stencil (A = sign*P), 1 = CSR pair, 2 = dense                     */
   int32_t pad_;
   double sign;       /* A = sign * Op                                                               */
   /* kind 0 */
   gnk_layout lay;
   gnk_bratu prm;
   const double* d_expu;
-  /* kind 1: A (n_res x p) as CSR and A^T as CSR */
+  /* kind 1: A (n_res x p) as CSR and A^T as CSR; kind 2 uses n_res and p as well */
   int64_t n_res, p;
   const int32_t *d_rowptr, *d_col;
   const double* d_val;
   const int32_t *d_rowptr_t, *d_col_t;
   const double* d_val_t;
+  /* kind 2: A dense, read in place, A[i, j] at d_dense[i * row_stride + j * col_stride] with one stride 1 (the
+   * layouts of gnk_dense_matmat).  Read only when kind == 2, so a caller that builds the struct without these fields
+   * for kind 0 or 1 stays valid. */
+  const double* d_dense;
+  int64_t row_stride, col_stride;
 } gnk_linop;
 /* Solves A^T A x = A^T y by Jacobi-preconditioned CG exactly as the reference does, including its
  * quirk (preconditioner == 0 first runs an unpreconditioned CG whose result is discarded and whose
  * iterations are added to *iters).  d_y: residual vector (stencil: stored column, halo >= 1 valid;
- * CSR: n_res doubles).  d_x: result (stencil: stored column; CSR: p doubles).  d_work: at least
- * 7 stored columns (stencil) / 7 * roundup16(max(p, n_res)) doubles (CSR).  Synchronises the stream. */
+ * CSR, dense: n_res doubles).  d_x: result (stencil: stored column; CSR, dense: p doubles).  d_work: at least
+ * 7 stored columns (stencil) / 7 * roundup16(max(p, n_res)) doubles (CSR, dense).  A dense operator takes
+ * gnk_dense_matmat (k = 1) for A p, gnk_dense_rmatvec for A^T t and gnk_dense_col_sumsq for the Jacobi diagonal: the
+ * bits of the CSR pair of the same matrix, without its copy and with no limit on n_res * p; one rank only.
+ * Synchronises the stream. */
 int gnk_cgls(gnk_ctx* ctx, const gnk_linop* op, const double* d_y, double rtol, int preconditioner,
              double* d_x, double* d_work, int64_t* iters, void* stream);
 /* The same with the initial guess that cg_least_squares forwards to scipy's cg (gauss_newton.py:14,46,56: `x0=x0`):

@@ -63,6 +63,7 @@ SIGNATURES = {
     "gnk_normalize": (_I, [_P, _LP, _P, _P, _D, _P, _P, _P]),
     "gnk_normalize_halo": (_I, [_P, _LP, _P, _P, _D, _P, _P, _P]),
     "gnk_cgs_dots": (_I, [_P, _LP, _P, _I, _P, _P, _P]),
+    "gnk_bratu_trial_project": (_I, [_P, _LP, _BP, _P, _I, _P, _P, _D, _P, _P, _P, _P, _P, _P, _P]),
     "gnk_cgs_update": (_I, [_P, _LP, _P, _I, _P, _P, _P, _P]),
     "gnk_tsqr_ls": (_I, [_P, _P, _L, _L, _I, _P, _D, _P, _P]),
     "gnk_dense_qr_ls": (_I, [_P, _P, _L, _L, _I, _D, _P, _P]),

@@ -180,6 +180,109 @@ __global__ void __launch_bounds__(TPBX) apply_kernel(gnk_layout lay, gnk_bratu p
   }
 }
 
+// The speculative trial of a res_old outer iteration in one pass over V_k (gauss_newton_krylow.py:91 + krylow.py:62,64):
+//   x = V_k (c + s d)                 over the whole stored column            == combine_kernel
+//   w = -J(x)^T F = M(x)^T F          owned points; M(x) = L + alpha D + lam diag(e^x)  == apply_kernel, transpose 1
+//   h = V_k^T w                                                               == dots_kernel
+// F is the residual at the CURRENT point (depth-1 halo rows valid), and x enters w only through the diagonal e^{x_i} at
+// the same point, so every owned point is self-contained: no neighbouring x, no halo of x.  Every value has the bits
+// of the kernels it replaces: x is the same fma chain over the columns; e^x the residual kernel's exp; w apply_refbits
+// with the same operands; h walks the points exactly as dots_kernel does (same grid, same points per thread in the
+// same order, same fma form, same warp -> CTA -> last-CTA tree) -- holding all k <= 8 NB columns of a point at once
+// instead of sweeping 8-column blocks leaves each column's accumulation sequence unchanged.  V is read from HBM once
+// (the k double2 of a point stay in registers between the x and h phases), F with default caching: its +-m rows are
+// L2 hits.  NB = 4 needs 254 registers; ptxas spills 24 bytes there, only inside exp's out-of-range branch.
+template <int NB>
+__global__ void __launch_bounds__(DOTS_TPB) trial_project_kernel(
+    gnk_layout lay, gnk_bratu prm, const double* __restrict__ V, int k, const double* __restrict__ c,
+    const double* __restrict__ d, double s, double* __restrict__ x, double* __restrict__ c_out,
+    double* __restrict__ cprev2, const double* __restrict__ F, double* __restrict__ w,
+    double* __restrict__ partials, unsigned int* ticket, double* __restrict__ h, gnk_p2p_dev pd) {
+  constexpr int NJ = 8 * NB;
+  constexpr int NFULL = 8 * (NB - 1);  // columns every launch of this instance has (k > 8 (NB - 1))
+  __shared__ double coef[GNK_MAX_BASIS];
+  __shared__ double wpart[DOTS_TPB / 32][GNK_MAX_BASIS];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  pdl_begin();
+  combine_coefficients(k, c, d, s, coef, c_out, cprev2);
+  const int m = lay.m;
+  const int64_t ld = lay.ld;
+  const double d0 = __dadd_rn(4.0 * prm.c_lap, -prm.c_adv);  // as apply_kernel forms the transposed operator
+  const double cu = __dadd_rn(-prm.c_lap, prm.c_adv);        // weight of row i-1 (c_sup)
+  const double cl = -prm.c_lap;                              // row i+1 and the j neighbours
+  const double* Vo = V + lay.off;
+  const double* Fo = F + lay.off;
+  const int64_t nv = lay.n_own >> 1;
+  const int64_t gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  double acc[NJ];
+#pragma unroll
+  for (int u = 0; u < NJ; ++u) acc[u] = 0.0;
+#pragma unroll 1
+  for (int64_t i = gt; i < nv; i += stride) {
+    // a column step the compiler cannot hoist: otherwise it keeps k 64-bit column offsets live across the loop
+    int64_t step = ld;
+    asm volatile("" : "+l"(step));
+    double2 v[NJ];
+    const double* pv = Vo + 2 * i;
+#pragma unroll
+    for (int u = 0; u < NJ; ++u) {
+      if (u < NFULL || u < k) v[u] = __ldcs(reinterpret_cast<const double2*>(pv));
+      pv += step;
+    }
+    double2 xv = make_double2(0.0, 0.0);
+#pragma unroll
+    for (int u = 0; u < NJ; ++u) {
+      if (u < NFULL || u < k) {
+        xv.x = fma(v[u].x, coef[u], xv.x);
+        xv.y = fma(v[u].y, coef[u], xv.y);
+      }
+    }
+    *reinterpret_cast<double2*>(x + lay.off + 2 * i) = xv;
+    const int64_t p = 2 * i;
+    const int j0 = (int)((unsigned)p % (unsigned)m);  // the entry takes slabs of < 2^31 owned unknowns
+    const double2 mid = *reinterpret_cast<const double2*>(Fo + p);
+    const double2 up = *reinterpret_cast<const double2*>(Fo + p - m);
+    const double2 dn = *reinterpret_cast<const double2*>(Fo + p + m);
+    const double lf = j0 > 0 ? Fo[p - 1] : 0.0;
+    const double rt = (j0 + 2) < m ? Fo[p + 2] : 0.0;
+    double dga = d0, dgb = d0;
+    if (prm.lam != 0.0) {
+      dga = __dadd_rn(d0, __dmul_rn(prm.lam, exp(xv.x)));
+      dgb = __dadd_rn(d0, __dmul_rn(prm.lam, exp(xv.y)));
+    }
+    double2 wv;
+    wv.x = apply_refbits(cu, cl, dga, cl, up.x, lf, mid.x, mid.y, dn.x);
+    wv.y = apply_refbits(cu, cl, dgb, cl, up.y, mid.x, mid.y, rt, dn.y);
+    *reinterpret_cast<double2*>(w + lay.off + p) = wv;
+#pragma unroll
+    for (int u = 0; u < NJ; ++u) {
+      if (u < NFULL || u < k) acc[u] = fma(v[u].y, wv.y, fma(v[u].x, wv.x, acc[u]));
+    }
+  }
+  // x on the rest of the stored column, [0, off) and [off + n_own, ld): combine_kernel covers the whole column, and the
+  // residual at depth 1 reads x on the halo rows
+  const int64_t nlo = lay.off >> 1, nrest = nlo + ((ld - lay.off - lay.n_own) >> 1);
+  for (int64_t q = gt; q < nrest; q += stride) {
+    const int64_t e = q < nlo ? 2 * q : lay.off + lay.n_own + 2 * (q - nlo);
+    double2 xv = make_double2(0.0, 0.0);
+    for (int u = 0; u < k; ++u) {
+      const double2 vv = __ldcs(reinterpret_cast<const double2*>(V + (int64_t)u * ld + e));
+      xv.x = fma(vv.x, coef[u], xv.x);
+      xv.y = fma(vv.y, coef[u], xv.y);
+    }
+    *reinterpret_cast<double2*>(x + e) = xv;
+  }
+#pragma unroll
+  for (int u = 0; u < NJ; ++u) {
+    if (u < k) {
+      const double r = warp_sum(acc[u]);
+      if (lane == 0) wpart[wid][u] = r;
+    }
+  }
+  dots_finish(wpart, k, partials, ticket, h, pd);
+}
+
 // diag(J^T J): squared column norms of P
 template <bool VEC>
 __global__ void __launch_bounds__(TPBX) normal_diag_kernel(gnk_layout lay, gnk_bratu prm,
@@ -297,6 +400,30 @@ int gnk_stencil_apply(gnk_ctx* ctx, const gnk_layout* lay, const gnk_bratu* prm,
   else
     GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), apply_kernel<false>, grid, dim3(TPBX), 0, (cudaStream_t)stream, *lay, *prm, e, d_in, in_ld, sign,
                         transpose, tr, d_out, out_ld, out_off));
+  GNK_LAUNCH_CHECK(ctx);
+  return 0;
+}
+
+int gnk_bratu_trial_project(gnk_ctx* ctx, const gnk_layout* lay, const gnk_bratu* prm, const double* d_V, int k,
+                            const double* d_c, const double* d_d, double s, double* d_x, double* d_c_out,
+                            double* d_cprev2, const double* d_F, double* d_w, double* d_h, void* stream) {
+  GNK_REQUIRE(ctx && prm && d_V && d_c && d_x && d_F && d_w && d_h, "gnk_bratu_trial_project: null argument");
+  GNK_REQUIRE(check_layout(lay) == 0, "gnk_bratu_trial_project: inconsistent stencil layout");
+  GNK_REQUIRE(k >= 1, "gnk_bratu_trial_project: k out of range");
+  GNK_REQUIRE(d_c_out != d_c, "gnk_bratu_trial_project: c_out must not alias c (rejected trials re-read c)");
+  // double2 points never straddle a grid row and stay 16-byte aligned; k columns of a point fit the registers
+  if ((lay->m & 1) || (lay->off & 1) || (lay->ld & 1) || k > 32 || lay->n_own >= (int64_t(1) << 31)) return 1;
+  const int grid = dots_grid(ctx, lay->n_own);  // gnk_cgs_dots' grid: it fixes the summation order of h
+  auto kern = trial_project_kernel<4>;
+  if (k <= 8)
+    kern = trial_project_kernel<1>;
+  else if (k <= 16)
+    kern = trial_project_kernel<2>;
+  else if (k <= 24)
+    kern = trial_project_kernel<3>;
+  GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), kern, dim3(grid), dim3(DOTS_TPB), 0, (cudaStream_t)stream, *lay, *prm,
+                      d_V, k, d_c, d_d, s, d_x, d_c_out, d_cprev2, d_F, d_w, ctx->d_partials + PART_DOTS,
+                      ctx->d_tickets + TK_DOTS, d_h, p2p_next(ctx)));
   GNK_LAUNCH_CHECK(ctx);
   return 0;
 }

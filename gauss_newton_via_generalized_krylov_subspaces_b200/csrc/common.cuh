@@ -291,6 +291,73 @@ __device__ __forceinline__ double apply_refbits(double cu, double cl, double dg,
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
 // ------------------------------------------------------------------------------------------------
+// Pieces shared by combine_kernel + dots_kernel (vector_ops.cu) and trial_project_kernel (bratu_stencil.cu), which
+// forms the same x, h bit for bit in one pass over the basis: whatever fixes those bits lives here once.
+// ------------------------------------------------------------------------------------------------
+// coef[j] = c[j] + s d[j] (d may be NULL: coef = c) into shared memory, as one fused multiply-add (the contraction nvcc
+// chose for the plain expression, written out so that it cannot change).  CTA 0 also writes c_out[j] = coef[j] (j < k)
+// and c_out[k] = 0 -- the accepted trial's x_coordinate with the entry of the next basis column already appended
+// (gauss_newton_krylow.py:98,124) -- and cprev2 = sum_j c[j]^2 for the stop test (:96-97).  Ends with a barrier.
+__device__ __forceinline__ void combine_coefficients(int k, const double* __restrict__ c, const double* __restrict__ d,
+                                                     double s, double* coef, double* __restrict__ c_out,
+                                                     double* __restrict__ cprev2) {
+  for (int j = threadIdx.x; j < k; j += blockDim.x) coef[j] = d ? __fma_rn(s, d[j], c[j]) : c[j];
+  __syncthreads();
+  if (blockIdx.x == 0) {
+    if (c_out) {
+      for (int j = threadIdx.x; j <= k && j < GNK_MAX_BASIS; j += blockDim.x) c_out[j] = (j < k) ? coef[j] : 0.0;
+    }
+    if (cprev2 && threadIdx.x < 32) {
+      double a = 0.0;
+      for (int j = threadIdx.x; j < k; j += 32) a = fma(c[j], c[j], a);
+      a = warp_sum(a);
+      if (threadIdx.x == 0) cprev2[0] = a;
+    }
+  }
+}
+
+// h = V_k^T w: 256-thread CTAs, >= 4 double2 per thread before another CTA is added; 4 CTAs per SM are resident, more
+// only lengthen the last CTA's reduction over the per-CTA partials.  The grid fixes the summation order of h.
+constexpr int DOTS_TPB = 256;
+inline int dots_grid(const gnk_ctx* ctx, int64_t n_own) {
+  int64_t g = ceil_div(n_own / 8, DOTS_TPB);
+  const int64_t cap = (int64_t)ctx->sm_count * 4;
+  if (g > cap) g = cap;
+  if (g < 1) g = 1;
+  return (int)g;
+}
+
+// The reduction tail of h: wpart[w][j] holds warp w's sum of column j (written by lane 0 of every warp).  Sums the
+// warps in a fixed order into this CTA's partial, then the CTA that arrives last sums the partials (one warp per column,
+// lanes strided over the CTAs) into h[0..k) and, with the peer mailboxes, over the ranks.
+template <int NW>
+__device__ __forceinline__ void dots_finish(const double (&wpart)[NW][GNK_MAX_BASIS], int k,
+                                            double* __restrict__ partials, unsigned int* ticket,
+                                            double* __restrict__ h, const gnk_p2p_dev& pd) {
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  __syncthreads();
+  for (int j = threadIdx.x; j < k; j += blockDim.x) {
+    double r = wpart[0][j];
+#pragma unroll
+    for (int q = 1; q < NW; ++q) r += wpart[q][j];  // fixed warp order: deterministic
+    partials[(int64_t)blockIdx.x * GNK_MAX_BASIS + j] = r;
+  }
+  if (grid_arrive_last(ticket)) {
+    const int nw = blockDim.x >> 5;
+    for (int j = wid; j < k; j += nw) {
+      double a = 0.0;
+      for (int b = lane; b < (int)gridDim.x; b += 32) a += __ldcg(partials + (int64_t)b * GNK_MAX_BASIS + j);
+      a = warp_sum(a);
+      if (lane == 0) h[j] = a;
+    }
+    if (pd.peers) {  // sum over the ranks, in this CTA, over the peers' mailboxes
+      __syncthreads();
+      p2p_tail_allreduce(pd, h, k, 0);
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // Programmatic dependent launch between the ~11 kernels of an outer iteration.  A kernel launched with gnk_launch may
 // be scheduled as soon as every CTA of its predecessor has passed pdl_begin(): its CTAs become resident while the
 // predecessor drains and start the instant it has completed, which hides the launch latency and the block-scheduling

@@ -21,10 +21,8 @@ __device__ __forceinline__ double2 ld2_stream(const double* p) {
 __device__ __forceinline__ void st2(double* p, double2 v) { *reinterpret_cast<double2*>(p) = v; }
 
 // ---------------------------------------------------------------------------------------------
-// c_out (optional): CTA 0 also writes the coordinates of the point it forms, c_out[j] = c[j] + s d[j] (j < k) and
-// c_out[k] = 0 -- the accepted trial's x_coordinate with the entry of the next basis column already appended
-// (gauss_newton_krylow.py:98,124) -- and cprev2 = sum_j c[j]^2 for the stop test (:96-97).  Saves three tiny launches
-// per outer iteration.
+// c_out / cprev2 (optional): the coordinate bookkeeping of combine_coefficients (common.cuh).  Saves three tiny
+// launches per outer iteration.
 __global__ void __launch_bounds__(TPB) combine_kernel(const double* __restrict__ V, int64_t ld, int64_t len,
                                                        int k, const double* __restrict__ c,
                                                        const double* __restrict__ d, double s,
@@ -32,19 +30,7 @@ __global__ void __launch_bounds__(TPB) combine_kernel(const double* __restrict__
                                                        double* __restrict__ cprev2) {
   __shared__ double coef[GNK_MAX_BASIS];
   pdl_begin();
-  for (int j = threadIdx.x; j < k; j += blockDim.x) coef[j] = d ? (c[j] + s * d[j]) : c[j];
-  __syncthreads();
-  if (blockIdx.x == 0) {
-    if (c_out) {
-      for (int j = threadIdx.x; j <= k && j < GNK_MAX_BASIS; j += blockDim.x) c_out[j] = (j < k) ? coef[j] : 0.0;
-    }
-    if (cprev2 && threadIdx.x < 32) {
-      double a = 0.0;
-      for (int j = threadIdx.x; j < k; j += 32) a = fma(c[j], c[j], a);
-      a = warp_sum(a);
-      if (threadIdx.x == 0) cprev2[0] = a;
-    }
-  }
+  combine_coefficients(k, c, d, s, coef, c_out, cprev2);
   const int64_t nv = len >> 1;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += stride) {
@@ -271,26 +257,7 @@ __global__ void __launch_bounds__(TPB, 4) dots_kernel(const double* __restrict__
       }
     }
   }
-  __syncthreads();
-  for (int j = threadIdx.x; j < k; j += TPB) {
-    double r = wpart[0][j];
-#pragma unroll
-    for (int q = 1; q < TPB / 32; ++q) r += wpart[q][j];  // fixed warp order: deterministic
-    partials[(int64_t)blockIdx.x * GNK_MAX_BASIS + j] = r;
-  }
-  if (grid_arrive_last(ticket)) {
-    const int nw = blockDim.x >> 5;
-    for (int j = wid; j < k; j += nw) {
-      double a = 0.0;
-      for (int b = lane; b < (int)gridDim.x; b += 32) a += __ldcg(partials + (int64_t)b * GNK_MAX_BASIS + j);
-      a = warp_sum(a);
-      if (lane == 0) h[j] = a;
-    }
-    if (pd.peers) {  // sum over the ranks, in this CTA, over the peers' mailboxes
-      __syncthreads();
-      p2p_tail_allreduce(pd, h, k, 0);
-    }
-  }
+  dots_finish(wpart, k, partials, ticket, h, pd);
 }
 
 // w[i] -= sum_j V[j*ld+i] h[j]; stats of the new w
@@ -481,9 +448,8 @@ int gnk_cgs_dots(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, 
   GNK_REQUIRE(ctx && lay && d_V && d_w && d_h, "gnk_cgs_dots: null argument");
   GNK_REQUIRE(k >= 1 && k <= GNK_MAX_BASIS, "gnk_cgs_dots: k out of range");
   GNK_REQUIRE((lay->off & 1) == 0 && (lay->ld & 1) == 0, "gnk_cgs_dots: off/ld must be even");
-  // >= 4 double2 per thread before another CTA is added; 4 CTAs per SM are resident (launch bounds), more only lengthen
-  // the last CTA's reduction over the per-CTA partials
-  int grid = stream_grid(ctx, lay->n_own / 8, 4);
+  static_assert(TPB == DOTS_TPB, "dots_kernel runs dots_finish's block size");
+  const int grid = dots_grid(ctx, lay->n_own);
   GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), dots_kernel, dim3(grid), dim3(TPB), 0, (cudaStream_t)stream, d_V + lay->off, lay->ld, lay->n_own, k,
                       d_w + lay->off, ctx->d_partials + PART_DOTS, ctx->d_tickets + TK_DOTS, d_h, p2p_next(ctx)));
   GNK_LAUNCH_CHECK(ctx);

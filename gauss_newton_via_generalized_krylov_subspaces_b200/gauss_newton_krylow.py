@@ -29,7 +29,7 @@ from .device import (DeviceCallableProblem, DeviceVector, HostCallableProblem, g
                      make_layout, ptr)
 from .krylow import (GeneralizedKrylowSubspace, GeneralizedKrylowSubspaceBreakdown,
                      GeneralizedKrylowSubspaceSpansEntireSpace, MAX_COLUMNS)
-from .partition import flat_layout_fields, round_up, tensor_ls_on_every_rank
+from .partition import flat_layout_fields, round_up, tensor_ls_on_every_rank, trial_project_fused
 from .regression_result import RegressionResult
 from .rosenbrock_problem import RosenbrockDeviceProblem
 
@@ -326,6 +326,7 @@ def gauss_newton_krylow(
     ls_method = 0
     if is_bratu and prob.distributed and not tensor_ls_on_every_rank(prob.sol_fields["m"], rt.world):
         ls_method = 1
+    fuse_trial = is_bratu and version == "res_old" and trial_project_fused(prob.sol_fields["m"], rt.world)
 
     if user_code:
         F_cur[:n_res_own].copy_(r0)
@@ -425,13 +426,21 @@ def gauss_newton_krylow(
 
             # Armijo-Goldstein in coordinate space  (:91-93)
             def trial_loss(s):
-                krylow.dev_combine(c, blk, s, x_trial, c_out=c_next, cprev2=ptr(blk, _SC_CPREV))
+                speculate = spec_ok and state["spec"] is None
+                # res_old expands with -J(x_trial)^T F_cur: the speculative trial point, that vector and its inner
+                # products with V_k come out of one pass over the basis instead of three
+                h_ready = (speculate and fuse_trial
+                           and krylow.dev_trial_project(prob.d.prm, c, blk, s, x_trial, c_next, ptr(blk, _SC_CPREV),
+                                                        F_cur))
+                if not h_ready:
+                    krylow.dev_combine(c, blk, s, x_trial, c_out=c_next, cprev2=ptr(blk, _SC_CPREV))
                 with rt.mark("residual", 32.0 * n_res_own):
                     prob.residual(x_trial, F_trial, loss_slot, aux=aux[1])
-                if spec_ok and state["spec"] is None:
+                if speculate:
                     pending_read = rt.read_begin(blk, _BLK)   # the scalars of this trial are complete here ...
                     jac_new = prob.jacobian(x_trial, aux=aux[1])
-                    krylow.dev_expand_enqueue(*expansion_operands(jac_new), hx, ptr(blk, other_slot()))
+                    krylow.dev_expand_enqueue(*expansion_operands(jac_new), hx, ptr(blk, other_slot()),
+                                              h_ready=h_ready)
                     state["spec"] = jac_new
                     state["vals"] = rt.read_end(pending_read)   # ... and are read while the expansion runs
                 else:

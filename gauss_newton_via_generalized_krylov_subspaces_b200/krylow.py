@@ -106,32 +106,52 @@ class GeneralizedKrylowSubspace:
                                                ptr(out), ptr(c_out), cprev2 if cprev2 is not None else ptr(None),
                                                rt.stream), "gnk_combine")
 
+    def dev_trial_project(self, prm, c, d, s, out, c_out, cprev2, F):
+        """``dev_combine(c, d, s, out, c_out, cprev2)``, ``w = -J(out)^T F`` and the first ``h = V_k^T w`` of the
+        expansion in one pass over V_k (gnk_bratu_trial_project, Bratu stencil, bit-identical to the separate kernels).
+        F: the residual at the current point with valid depth-1 halo rows.  Returns False, having launched nothing,
+        when the library does not take the inputs; the caller then runs the separate kernels."""
+        rt = self.rt
+        with rt.mark("trial_project", 8.0 * self.fields["n_own"] * (self.k + 3)) as mk:
+            rc = rt.lib.gnk_bratu_trial_project(rt.ctx, C.byref(self.lay), C.byref(prm), ptr(self.V), self.k, ptr(c),
+                                                ptr(d), float(s), ptr(out), ptr(c_out), cprev2, ptr(F), ptr(self.w),
+                                                ptr(self.h), rt.stream)
+            mk.cancel = rc != 0
+        if rc == 1:
+            return False
+        _lib.check(rc, "gnk_bratu_trial_project")
+        if not rt.fused_reductions:
+            rt.allreduce(self.h, self.k, 0)
+        return True
+
     def dev_rmatvec(self, jac_op, r):
         """w = -J^T r alone, for a following expansion called with ``jac_op=None``"""
         with self.rt.mark("spmv_t", 24.0 * self.fields["n_own"]):
             jac_op.neg_rmatvec(r, self.w)
 
-    def dev_expand_enqueue(self, jac_op, r, halo_exchange=None, flag_ptr=None):
+    def dev_expand_enqueue(self, jac_op, r, halo_exchange=None, flag_ptr=None, h_ready=False):
         """Enqueue the basis expansion with -J^T r orthogonalised against V_k (krylow.py:55-73) WITHOUT committing it:
         the normalised vector lands in column k of the storage, the breakdown flag of krylow.py:66 in ``flag_ptr`` (a
         device int32; default: this object's own flag), and ``k`` is unchanged until ``commit()``.  Nothing is read
         back, so the caller may enqueue it speculatively (gauss_newton_krylow does, before it knows whether the Armijo
         trial is accepted) -- an expansion that is not committed leaves no trace: w, h, the statistics, column k and the
-        flag are all overwritten by the next one.  ``jac_op=None``: w already holds -J^T r (``dev_rmatvec``)."""
+        flag are all overwritten by the next one.  ``jac_op=None``: w already holds -J^T r (``dev_rmatvec``).
+        ``h_ready``: w and the first pass's h = V_k^T w are already formed (``dev_trial_project`` of this call's trial)."""
         if self.k == self.n_glob:
             raise GeneralizedKrylowSubspaceSpansEntireSpace
         rt, lib = self.rt, self.rt.lib
         if self.k == self.cap:
             self._grow()
         n = self.fields["n_own"]
-        if jac_op is not None:
+        if jac_op is not None and not h_ready:
             self.dev_rmatvec(jac_op, r)
         for ipass in range(self.reorth_passes):
-            with rt.mark("cgs_dots", 8.0 * n * (self.k + 1)):
-                _lib.check(lib.gnk_cgs_dots(rt.ctx, C.byref(self.lay), ptr(self.V), self.k, ptr(self.w),
-                                            ptr(self.h), rt.stream), "gnk_cgs_dots")
-            if not rt.fused_reductions:  # else summed over the ranks inside the kernel (peer mailboxes)
-                rt.allreduce(self.h, self.k, 0)
+            if ipass > 0 or not h_ready:
+                with rt.mark("cgs_dots", 8.0 * n * (self.k + 1)):
+                    _lib.check(lib.gnk_cgs_dots(rt.ctx, C.byref(self.lay), ptr(self.V), self.k, ptr(self.w),
+                                                ptr(self.h), rt.stream), "gnk_cgs_dots")
+                if not rt.fused_reductions:  # else summed over the ranks inside the kernel (peer mailboxes)
+                    rt.allreduce(self.h, self.k, 0)
             with rt.mark("cgs_update", 8.0 * n * (self.k + 2)):
                 _lib.check(lib.gnk_cgs_update(rt.ctx, C.byref(self.lay), ptr(self.V), self.k, ptr(self.h),
                                               ptr(self.w), ptr(self.stats), rt.stream), "gnk_cgs_update")

@@ -34,6 +34,16 @@ def tensor_ls_on_every_rank(m: int, world: int) -> bool:
     return all(cn >= LS_TENSOR_MIN_ROWS and cn % 2 == 0 for cn in all_counts(m, world))
 
 
+def trial_project_fused(m: int, world: int) -> bool:
+    """True if gauss_newton_krylow forms its speculative Armijo trial and the first Gram-Schmidt inner products in one
+    pass over the basis (gnk_bratu_trial_project): an even row length and slabs of >= 16384 owned unknowns -- the grids
+    the pass is built for; smaller ones, where launches rather than the basis traffic dominate, and the numpy mock of the
+    C ABI keep the separate kernels.  One rank only: the fused pass takes the Gram-Schmidt dots' place in the sequence
+    of collectives, and several ranks keep today's sequence until that has run on more than one GPU.  Decided from m
+    and world alone, so every rank decides alike."""
+    return world == 1 and m % 2 == 0 and all(cn >= LS_TENSOR_MIN_ROWS for cn in all_counts(m, world))
+
+
 def round_up(x: int, q: int) -> int:
     return (x + q - 1) // q * q
 

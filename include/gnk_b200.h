@@ -132,6 +132,19 @@ int gnk_cgs_dots(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, 
 int gnk_cgs_update(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, const double* d_h,
                    double* d_w, double* d_stats, void* stream);
 
+/* The speculative first Armijo trial of a res_old outer iteration and the Gram-Schmidt inner products of the basis
+ * expansion behind it, in ONE pass over V_k (krylow.py:41-42,62,64, armijo_goldstein.py:56), for the Bratu stencil:
+ *   d_x      = V_k (c + s d) over the whole stored column, d_c_out / d_cprev2    == gnk_combine_step
+ *   d_w      = -J(x)^T F over owned entries (halo rows untouched)                == gnk_stencil_apply(e^x, F, 1, +1, 1)
+ *   d_h[0..k) = V_k^T w, reduced over the ranks like gnk_cgs_dots                  == gnk_cgs_dots
+ * where e^x is formed from x in registers (gnk_bratu_residual's exp) and d_F is a stored column whose depth-1 halo rows
+ * are valid (the residual at the current point).  Bit-identical to the four calls it replaces.  Returns 1 -- nothing
+ * launched -- for inputs it does not take (odd m, off or ld; k > 32; 2^31 or more owned unknowns): the caller then
+ * issues those calls. */
+int gnk_bratu_trial_project(gnk_ctx* ctx, const gnk_layout* lay, const gnk_bratu* prm, const double* d_V, int k,
+                            const double* d_c, const double* d_d, double s, double* d_x, double* d_c_out,
+                            double* d_cprev2, const double* d_F, double* d_w, double* d_h, void* stream);
+
 /* ---- projected least squares (gauss_newton_krylow.py:16-36, :89) ------------------------------- */
 /* Householder TSQR of the n_rows x (k+1) panel [sign_a*A | y] (A column-major, stride lda) and
  * solution of min || sign_a*A d - y ||_2.  Results (device): d_out[0..k) = d, d_out[k] = ||R d||^2

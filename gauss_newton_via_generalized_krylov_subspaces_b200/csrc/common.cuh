@@ -55,6 +55,11 @@ struct gnk_ctx {
   // gnk_dense_qr_ls (dense_qr.cu): panel partials, pivot rows, taus, split partials of V^T C and T^T W (grown on demand)
   double* d_dqr = nullptr;
   size_t dqr_bytes = 0;
+  // gnk_basis_ls_wide on several ranks (dense_qr.cu): padded slab, triangles, gathered triangles, stacked panel
+  double* d_wls = nullptr;
+  size_t wls_bytes = 0;
+  // gnk_cgs_dots for k >= GNK_MAX_BASIS (vector_ops.cu): per-CTA partials of h, dots grid x GNK_MAX_BASIS_WIDE doubles
+  double* d_wdots = nullptr;
 };
 int gnk_ensure_fetch_stream(gnk_ctx* ctx);  // api.cu: creates fetch_stream / fetch_event on first use
 
@@ -179,8 +184,9 @@ __host__ __device__ inline size_t p2p_halo_off(int nranks, int parity, int side)
   return P2P_FLAG_BYTES + sizeof(double) * (size_t)(2 * nranks * P2P_GMAX) +
          sizeof(double) * (size_t)((parity * 2 + side) * P2P_HMAX);
 }
-// flag-in-data lines of the in-kernel all-reduces (p2p_tail_allreduce): 16 bytes per double, after the halo slots
-constexpr int P2P_LLMAX = 1024;
+// flag-in-data lines of the in-kernel all-reduces (p2p_tail_allreduce, p2p_tail_allreduce_wide): 16 bytes per double,
+// after the halo slots; one line per entry of the widest h (k <= GNK_MAX_BASIS_WIDE - 1)
+constexpr int P2P_LLMAX = GNK_MAX_BASIS_WIDE;
 __host__ __device__ inline size_t p2p_ll_off(int nranks, int parity, int r) {
   return p2p_halo_off(nranks, 2, 0) + 16 * (size_t)((parity * nranks + r) * P2P_LLMAX);
 }
@@ -274,6 +280,24 @@ __device__ __forceinline__ void p2p_tail_allreduce(const gnk_p2p_dev& pd, double
     a = is_max ? fmax(a, b) : a + b;
   }
   vals[t] = a;
+}
+// The same reduction for count > blockDim.x (the h of a basis with k >= GNK_MAX_BASIS columns, count < P2P_LLMAX): every
+// thread first publishes all its entries, then reduces them; entry t gets exactly the rank-ordered arithmetic of
+// p2p_tail_allreduce (op 0, sum).
+__device__ __forceinline__ void p2p_tail_allreduce_wide(const gnk_p2p_dev& pd, double* vals, int count) {
+  const int parity = (int)(pd.seq & 1ull);
+  const unsigned tag = (unsigned)(pd.seq % 0xFFFFFFFFull) + 1u;
+  for (int t = threadIdx.x; t < count; t += blockDim.x) {
+    const double v = vals[t];
+    for (int r = 0; r < pd.nranks; ++r)
+      st_ll(static_cast<char*>(pd.peers[r]) + p2p_ll_off(pd.nranks, parity, pd.rank) + 16 * (size_t)t, v, tag);
+  }
+  const char* mine = static_cast<const char*>(pd.peers[pd.rank]);
+  for (int t = threadIdx.x; t < count; t += blockDim.x) {
+    double a = ld_ll(mine + p2p_ll_off(pd.nranks, parity, 0) + 16 * (size_t)t, tag);
+    for (int r = 1; r < pd.nranks; ++r) a += ld_ll(mine + p2p_ll_off(pd.nranks, parity, r) + 16 * (size_t)t, tag);
+    vals[t] = a;
+  }
 }
 
 // One row of sign * (M v) or sign * (M^T v), M = L + alpha D + lam diag(e^u), in the order scipy uses for

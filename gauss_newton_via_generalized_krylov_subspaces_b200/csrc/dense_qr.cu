@@ -399,15 +399,8 @@ int panel_grid_max(gnk_ctx* ctx) {
   return occ * ctx->sm_count;
 }
 
-}  // namespace
-
-extern "C" int gnk_dense_qr_ls(gnk_ctx* ctx, double* d_A, int64_t lda, int64_t n_rows, int p, double sign_a,
-                               double* d_out, void* stream) {
-  GNK_REQUIRE(ctx && d_A && d_out, "gnk_dense_qr_ls: null argument");
-  GNK_REQUIRE(p >= GNK_DENSE_QR_MIN && p <= GNK_DENSE_QR_MAX, "gnk_dense_qr_ls: p out of range");
-  GNK_REQUIRE(n_rows >= p && lda >= n_rows, "gnk_dense_qr_ls: bad panel (needs n_rows >= p and lda >= n_rows)");
-  GNK_REQUIRE(((uintptr_t)d_A & 7) == 0, "gnk_dense_qr_ls: the panel must be 8-byte aligned");
-  cudaStream_t st = (cudaStream_t)stream;
+// Blocked Householder factorisation of [sign_a * A | y] in place (everything of gnk_dense_qr_ls but the solve).
+int dqr_factor(gnk_ctx* ctx, double* d_A, int64_t lda, int64_t n_rows, int p, double sign_a, cudaStream_t st) {
   const int c = p + 1;
   const int gmax = panel_grid_max(ctx);
   if (gmax <= 0) return -1;
@@ -466,7 +459,118 @@ extern "C" int gnk_dense_qr_ls(gnk_ctx* ctx, double* d_A, int64_t lda, int64_t n
     dqr_update_kernel<<<dim3((unsigned)ceil_div(m, TM), ntile), UT, 0, st>>>(d_A, lda, n_rows, c, j0, nbp, w2, ldw);
     GNK_LAUNCH_CHECK(ctx);
   }
+  return 0;
+}
+
+// ---- gnk_basis_ls_wide on several ranks -------------------------------------------------------------------------
+// src: n x (p+1) panel (stride ld, n rows valid), dst: the same with rows_to >= n rows (stride ldd), zero-padded
+__global__ void wls_pad_kernel(const double* __restrict__ src, int64_t ld, int64_t n, int p, double* __restrict__ dst,
+                               int64_t ldd, int64_t rows_to) {
+  const int64_t total = rows_to * (int64_t)(p + 1);
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t j = e / rows_to, i = e - j * rows_to;
+    dst[j * ldd + i] = i < n ? src[j * ld + i] : 0.0;
+  }
+}
+
+// T ((p+1) x (p+1), column-major, stride p+1) = [[R, z], [0, rho]] of a factored panel: R the upper triangle of
+// columns 0..p-1, z = (Q^T y)[0..p); T[p][p] (rho) is written by wls_rho_kernel
+__global__ void wls_pack_kernel(const double* __restrict__ P, int64_t lda, int p, double* __restrict__ T) {
+  const int64_t c = p + 1, total = c * c;
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t j = e / c, i = e - j * c;
+    if (i == p && j == p) continue;
+    T[e] = (i <= j && i < p) ? P[j * lda + i] : 0.0;
+  }
+}
+
+// rho = sqrt(sum_{i >= p} (Q^T y)_i^2) in one CTA, fixed order
+__global__ void __launch_bounds__(ST) wls_rho_kernel(const double* __restrict__ P, int64_t lda, int64_t n, int p,
+                                                     double* __restrict__ T) {
+  __shared__ double sh[ST / 32];
+  const double* qy = P + (int64_t)p * lda;
+  double s = 0.0;
+  for (int64_t i = p + threadIdx.x; i < n; i += ST) s = fma(qy[i], qy[i], s);
+  s = solve_block_sum(s, sh);
+  if (threadIdx.x == 0) T[(int64_t)p * (p + 1) + p] = sqrt(s);
+}
+
+// stack (column-major, stride lds): rank r's triangle in rows r (p+1) .. (r+1) (p+1) - 1
+__global__ void wls_stack_kernel(const double* __restrict__ G, int nranks, int p, double* __restrict__ S,
+                                 int64_t lds) {
+  const int64_t c = p + 1, tri = c * c, total = tri * nranks;
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = e / tri, q = e - r * tri, j = q / c, i = q - j * c;
+    S[j * lds + r * c + i] = G[e];
+  }
+}
+
+int ensure_wls(gnk_ctx* ctx, size_t bytes, cudaStream_t st) {
+  if (bytes <= ctx->wls_bytes) return 0;
+  GNK_CUDA(cudaStreamSynchronize(st));
+  if (ctx->d_wls) GNK_CUDA(cudaFree(ctx->d_wls));
+  ctx->d_wls = nullptr;
+  ctx->wls_bytes = 0;
+  GNK_CUDA(cudaMalloc(&ctx->d_wls, bytes));
+  ctx->wls_bytes = bytes;
+  return 0;
+}
+
+}  // namespace
+
+int gnk_comm_allgather_doubles(gnk_ctx* ctx, const double* d_send, double* d_recv, int64_t count, void* stream);
+
+extern "C" int gnk_dense_qr_ls(gnk_ctx* ctx, double* d_A, int64_t lda, int64_t n_rows, int p, double sign_a,
+                               double* d_out, void* stream) {
+  GNK_REQUIRE(ctx && d_A && d_out, "gnk_dense_qr_ls: null argument");
+  GNK_REQUIRE(p >= GNK_DENSE_QR_MIN && p <= GNK_DENSE_QR_MAX, "gnk_dense_qr_ls: p out of range");
+  GNK_REQUIRE(n_rows >= p && lda >= n_rows, "gnk_dense_qr_ls: bad panel (needs n_rows >= p and lda >= n_rows)");
+  GNK_REQUIRE(((uintptr_t)d_A & 7) == 0, "gnk_dense_qr_ls: the panel must be 8-byte aligned");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (int rc = dqr_factor(ctx, d_A, lda, n_rows, p, sign_a, st)) return rc;
   dqr_solve_kernel<<<1, ST, 0, st>>>(d_A, lda, n_rows, p, d_out);
+  GNK_LAUNCH_CHECK(ctx);
+  return 0;
+}
+
+extern "C" int gnk_basis_ls_wide(gnk_ctx* ctx, double* d_P, int64_t ldp, int64_t n_rows, int k, double sign_a,
+                                 double* d_out, void* stream) {
+  GNK_REQUIRE(ctx && d_P && d_out, "gnk_basis_ls_wide: null argument");
+  GNK_REQUIRE(k >= GNK_DENSE_QR_MIN && k < GNK_MAX_BASIS_WIDE, "gnk_basis_ls_wide: k out of range (256..4095)");
+  GNK_REQUIRE(n_rows >= 0 && ldp >= n_rows, "gnk_basis_ls_wide: bad panel (needs ldp >= n_rows)");
+  GNK_REQUIRE(((uintptr_t)d_P & 7) == 0, "gnk_basis_ls_wide: the panel must be 8-byte aligned");
+  if (ctx->nranks == 1) {
+    GNK_REQUIRE(n_rows >= (int64_t)k + 1,
+                "gnk_basis_ls_wide: fewer residuals than basis columns + 1 (the projected problem is underdetermined)");
+    return gnk_dense_qr_ls(ctx, d_P, ldp, n_rows, k, sign_a, d_out, stream);
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  const int64_t c = (int64_t)k + 1, tri = c * c, N = ctx->nranks;
+  const int64_t ldpad = (c + 1) & ~(int64_t)1, lds = (N * c + 1) & ~(int64_t)1;
+  const bool pad = n_rows < c;
+  // scratch: [padded slab | own triangle | gathered triangles | stacked panel]
+  const int64_t off_tri = pad ? ldpad * c : 0, off_all = off_tri + tri, off_stack = off_all + N * tri;
+  if (int rc = ensure_wls(ctx, sizeof(double) * (size_t)(off_stack + lds * c), st)) return rc;
+  double* base = ctx->d_wls;
+  double* slab = d_P;
+  int64_t ld = ldp, rows = n_rows;
+  if (pad) {
+    wls_pad_kernel<<<ctx->sm_count, 256, 0, st>>>(d_P, ldp, n_rows, k, base, ldpad, c);
+    GNK_LAUNCH_CHECK(ctx);
+    slab = base;
+    ld = ldpad;
+    rows = c;
+  }
+  if (int rc = dqr_factor(ctx, slab, ld, rows, k, sign_a, st)) return rc;
+  wls_pack_kernel<<<ctx->sm_count, 256, 0, st>>>(slab, ld, k, base + off_tri);
+  GNK_LAUNCH_CHECK(ctx);
+  wls_rho_kernel<<<1, ST, 0, st>>>(slab, ld, rows, k, base + off_tri);
+  GNK_LAUNCH_CHECK(ctx);
+  if (int rc = gnk_comm_allgather_doubles(ctx, base + off_tri, base + off_all, tri, st)) return rc;
+  wls_stack_kernel<<<4 * ctx->sm_count, 256, 0, st>>>(base + off_all, (int)N, k, base + off_stack, lds);
+  GNK_LAUNCH_CHECK(ctx);
+  if (int rc = dqr_factor(ctx, base + off_stack, lds, N * c, k, 1.0, st)) return rc;
+  dqr_solve_kernel<<<1, ST, 0, st>>>(base + off_stack, lds, N * c, k, d_out);
   GNK_LAUNCH_CHECK(ctx);
   return 0;
 }

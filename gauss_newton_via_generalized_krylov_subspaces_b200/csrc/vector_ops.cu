@@ -5,6 +5,7 @@
 //   cgs_dots    h = V_k^T w                       krylow.py:64 (inner product half)
 //   cgs_update  w -= V_k h  (+ stats of new w)    krylow.py:64 (update half) + :66,:71
 //   axpby, dot                                    gauss_newton.py:123-129
+// combine, cgs_dots and cgs_update have wide twins for bases of 256..4095 columns (*_wide_kernel).
 // Every thread moves 128-bit (double2) words, columns are walked with independent loads in flight,
 // grids are sized in multiples of the SM count, cross-CTA reductions use a fixed-order
 // "last CTA finishes" tree so results are run-to-run deterministic.
@@ -336,6 +337,187 @@ __global__ void __launch_bounds__(TPB) update_kernel(const double* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------------
+// Bases of GNK_MAX_BASIS <= k < GNK_MAX_BASIS_WIDE columns (runs without a restart).  Same per-element arithmetic as the
+// kernels above, with the k coefficients in 8k bytes of dynamic shared memory (at most 32 KB: 7 CTAs of 256 threads
+// per SM) and the per-warp sums of the dots staged in chunks of WCH columns.  Still one pass over V_k per launch.
+constexpr int WCH = 256;  // columns per chunk of the per-warp sums of dots_wide_kernel (a multiple of JB)
+
+// combine_coefficients (common.cuh) for any k: c_out receives k + 1 doubles
+__device__ __forceinline__ void combine_coefficients_wide(int k, const double* __restrict__ c,
+                                                          const double* __restrict__ d, double s, double* coef,
+                                                          double* __restrict__ c_out, double* __restrict__ cprev2) {
+  for (int j = threadIdx.x; j < k; j += blockDim.x) coef[j] = d ? __fma_rn(s, d[j], c[j]) : c[j];
+  __syncthreads();
+  if (blockIdx.x == 0) {
+    if (c_out) {
+      for (int j = threadIdx.x; j <= k; j += blockDim.x) c_out[j] = (j < k) ? coef[j] : 0.0;
+    }
+    if (cprev2 && threadIdx.x < 32) {
+      double a = 0.0;
+      for (int j = threadIdx.x; j < k; j += 32) a = fma(c[j], c[j], a);
+      a = warp_sum(a);
+      if (threadIdx.x == 0) cprev2[0] = a;
+    }
+  }
+}
+
+// sum_j V[j*ld + 2i .. 2i+1] coef[j], eight 128-bit loads in flight
+__device__ __forceinline__ double2 combine_row(const double* __restrict__ p, int64_t ld, int k,
+                                               const double* __restrict__ coef) {
+  double2 acc = make_double2(0.0, 0.0);
+  int j = 0;
+  for (; j + 8 <= k; j += 8) {
+    double2 v[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) v[u] = ld2_stream(p + (int64_t)(j + u) * ld);
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+      acc.x = fma(v[u].x, coef[j + u], acc.x);
+      acc.y = fma(v[u].y, coef[j + u], acc.y);
+    }
+  }
+  for (; j < k; ++j) {
+    double2 v = ld2_stream(p + (int64_t)j * ld);
+    acc.x = fma(v.x, coef[j], acc.x);
+    acc.y = fma(v.y, coef[j], acc.y);
+  }
+  return acc;
+}
+
+__global__ void __launch_bounds__(TPB) combine_wide_kernel(const double* __restrict__ V, int64_t ld, int64_t len,
+                                                            int k, const double* __restrict__ c,
+                                                            const double* __restrict__ d, double s,
+                                                            double* __restrict__ x, double* __restrict__ c_out,
+                                                            double* __restrict__ cprev2) {
+  extern __shared__ double coef[];
+  pdl_begin();
+  combine_coefficients_wide(k, c, d, s, coef, c_out, cprev2);
+  const int64_t nv = len >> 1;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < nv; i += stride)
+    st2(x + 2 * i, combine_row(V + 2 * i, ld, k, coef));
+}
+
+// h = V_k^T w.  partials: column-major per CTA (partials[j * gridDim.x + b]), so that the last CTA reads them coalesced
+// while summing in dots_finish's order (lanes strided over the CTAs, then the warp tree): per entry the bits of
+// dots_kernel at the same n.
+__global__ void __launch_bounds__(TPB, 4) dots_wide_kernel(const double* __restrict__ V, int64_t ld, int64_t n, int k,
+                                                         const double* __restrict__ w, double* __restrict__ partials,
+                                                         unsigned int* ticket, double* __restrict__ h,
+                                                         gnk_p2p_dev pd) {
+  __shared__ double wpart[TPB / 32][WCH];
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  const int G = gridDim.x;
+  pdl_begin();
+  for (int c0 = 0; c0 < k; c0 += WCH) {
+    const int kc = min(WCH, k - c0);
+    for (int jb = 0; jb < kc; jb += JB) {
+      double acc[JB];
+#pragma unroll
+      for (int u = 0; u < JB; ++u) acc[u] = 0.0;
+      const int nj = min(JB, kc - jb);
+      const double* Vb = V + (int64_t)(c0 + jb) * ld;
+      switch (nj) {
+        case 8: dots_pass<8>(Vb, ld, n, w, acc); break;
+        case 7: dots_pass<7>(Vb, ld, n, w, acc); break;
+        case 6: dots_pass<6>(Vb, ld, n, w, acc); break;
+        case 5: dots_pass<5>(Vb, ld, n, w, acc); break;
+        case 4: dots_pass<4>(Vb, ld, n, w, acc); break;
+        case 3: dots_pass<3>(Vb, ld, n, w, acc); break;
+        case 2: dots_pass<2>(Vb, ld, n, w, acc); break;
+        default: dots_pass<1>(Vb, ld, n, w, acc); break;
+      }
+#pragma unroll
+      for (int u = 0; u < JB; ++u) {
+        if (u < nj) {
+          const double r = warp_sum(acc[u]);
+          if (lane == 0) wpart[wid][jb + u] = r;
+        }
+      }
+    }
+    __syncthreads();
+    for (int j = threadIdx.x; j < kc; j += blockDim.x) {
+      double r = wpart[0][j];
+#pragma unroll
+      for (int q = 1; q < TPB / 32; ++q) r += wpart[q][j];
+      partials[(int64_t)(c0 + j) * G + blockIdx.x] = r;
+    }
+    __syncthreads();  // wpart is refilled by the next chunk
+  }
+  if (grid_arrive_last(ticket)) {
+    for (int j = wid; j < k; j += TPB / 32) {
+      const double* pj = partials + (int64_t)j * G;
+      double a = 0.0;
+      for (int b = lane; b < G; b += 32) a += __ldcg(pj + b);
+      a = warp_sum(a);
+      if (lane == 0) h[j] = a;
+    }
+    if (pd.peers) {  // sum over the ranks, in this CTA, over the peers' mailboxes
+      __syncthreads();
+      p2p_tail_allreduce_wide(pd, h, k);
+    }
+  }
+}
+
+// w[i] -= sum_j V[j*ld+i] h[j]; stats of the new w (update_kernel for any k)
+__global__ void __launch_bounds__(TPB) update_wide_kernel(const double* __restrict__ V, int64_t ld, int64_t n, int k,
+                                                           const double* __restrict__ h, double* __restrict__ w,
+                                                           double* __restrict__ partials, unsigned int* ticket,
+                                                           double* __restrict__ stats, gnk_p2p_dev pd) {
+  extern __shared__ double coef[];
+  __shared__ double sh[32];
+  pdl_begin();
+  for (int j = threadIdx.x; j < k; j += blockDim.x) coef[j] = h[j];
+  __syncthreads();
+  const int64_t nv = n >> 1;
+  const int64_t gt = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  double ss = 0.0, mx = 0.0;
+  for (int64_t i = gt; i < nv; i += stride) {
+    const double2 acc = combine_row(V + 2 * i, ld, k, coef);
+    double2 wv = ld2(w + 2 * i);
+    wv.x -= acc.x;
+    wv.y -= acc.y;
+    st2(w + 2 * i, wv);
+    ss = fma(wv.x, wv.x, ss);
+    ss = fma(wv.y, wv.y, ss);
+    mx = fmax(mx, fmax(fabs(wv.x), fabs(wv.y)));
+  }
+  if ((n & 1) && gt == 0) {
+    double acc = 0.0;
+    for (int j = 0; j < k; ++j) acc = fma(V[(int64_t)j * ld + n - 1], coef[j], acc);
+    double wv = w[n - 1] - acc;
+    w[n - 1] = wv;
+    ss = fma(wv, wv, ss);
+    mx = fmax(mx, fabs(wv));
+  }
+  if (stats == nullptr) return;
+  ss = block_sum(ss, sh);
+  mx = block_max(mx, sh);
+  if (threadIdx.x == 0) {
+    partials[2 * blockIdx.x] = ss;
+    partials[2 * blockIdx.x + 1] = mx;
+  }
+  if (grid_arrive_last(ticket)) {
+    double a = 0.0, b = 0.0;
+    for (int i = threadIdx.x; i < (int)gridDim.x; i += blockDim.x) {
+      a += __ldcg(partials + 2 * i);
+      b = fmax(b, __ldcg(partials + 2 * i + 1));
+    }
+    a = block_sum(a, sh);
+    b = block_max(b, sh);
+    if (threadIdx.x == 0) {
+      stats[0] = a;
+      stats[1] = b;
+    }
+    if (pd.peers) {
+      __syncthreads();
+      p2p_tail_allreduce(pd, stats, 2, 2);
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(TPB) axpby_kernel(int64_t n, double a, const double* x, double b,
                                                      const double* y, double* out) {
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
@@ -379,10 +561,16 @@ extern "C" {
 int gnk_combine_step(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, const double* d_c,
                      const double* d_d, double s, double* d_x, double* d_c_out, double* d_cprev2, void* stream) {
   GNK_REQUIRE(ctx && lay && d_V && d_c && d_x, "gnk_combine: null argument");
-  GNK_REQUIRE(k >= 1 && k <= GNK_MAX_BASIS, "gnk_combine: k out of range");
+  GNK_REQUIRE(k >= 1 && k < GNK_MAX_BASIS_WIDE, "gnk_combine: k out of range");
   GNK_REQUIRE((lay->ld & 1) == 0, "gnk_combine: ld must be even");
   GNK_REQUIRE(d_c_out != d_c, "gnk_combine_step: c_out must not alias c (rejected trials re-read c)");
   int grid = stream_grid(ctx, lay->ld / 2, 8);
+  if (k >= GNK_MAX_BASIS) {
+    GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), combine_wide_kernel, dim3(grid), dim3(TPB), sizeof(double) * k,
+                        (cudaStream_t)stream, d_V, lay->ld, lay->ld, k, d_c, d_d, s, d_x, d_c_out, d_cprev2));
+    GNK_LAUNCH_CHECK(ctx);
+    return 0;
+  }
   GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), combine_kernel, dim3(grid), dim3(TPB), 0, (cudaStream_t)stream, d_V, lay->ld, lay->ld, k, d_c, d_d, s,
                       d_x, d_c_out, d_cprev2));
   GNK_LAUNCH_CHECK(ctx);
@@ -446,10 +634,20 @@ int gnk_normalize_halo(gnk_ctx* ctx, const gnk_layout* lay, const double* d_x, c
 int gnk_cgs_dots(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, const double* d_w, double* d_h,
                  void* stream) {
   GNK_REQUIRE(ctx && lay && d_V && d_w && d_h, "gnk_cgs_dots: null argument");
-  GNK_REQUIRE(k >= 1 && k <= GNK_MAX_BASIS, "gnk_cgs_dots: k out of range");
+  GNK_REQUIRE(k >= 1 && k < GNK_MAX_BASIS_WIDE, "gnk_cgs_dots: k out of range");
   GNK_REQUIRE((lay->off & 1) == 0 && (lay->ld & 1) == 0, "gnk_cgs_dots: off/ld must be even");
   static_assert(TPB == DOTS_TPB, "dots_kernel runs dots_finish's block size");
   const int grid = dots_grid(ctx, lay->n_own);
+  if (k >= GNK_MAX_BASIS) {
+    static_assert(P2P_LLMAX >= GNK_MAX_BASIS_WIDE - 1, "the mailbox lines must hold the widest h");
+    if (!ctx->d_wdots)  // dots_grid is at most 4 CTAs per SM
+      GNK_CUDA(cudaMalloc(&ctx->d_wdots, sizeof(double) * 4 * (size_t)ctx->sm_count * GNK_MAX_BASIS_WIDE));
+    GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), dots_wide_kernel, dim3(grid), dim3(TPB), 0, (cudaStream_t)stream,
+                        d_V + lay->off, lay->ld, lay->n_own, k, d_w + lay->off, ctx->d_wdots,
+                        ctx->d_tickets + TK_DOTS, d_h, p2p_next(ctx)));
+    GNK_LAUNCH_CHECK(ctx);
+    return 0;
+  }
   GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), dots_kernel, dim3(grid), dim3(TPB), 0, (cudaStream_t)stream, d_V + lay->off, lay->ld, lay->n_own, k,
                       d_w + lay->off, ctx->d_partials + PART_DOTS, ctx->d_tickets + TK_DOTS, d_h, p2p_next(ctx)));
   GNK_LAUNCH_CHECK(ctx);
@@ -459,9 +657,17 @@ int gnk_cgs_dots(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, 
 int gnk_cgs_update(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, const double* d_h, double* d_w,
                    double* d_stats, void* stream) {
   GNK_REQUIRE(ctx && lay && d_V && d_w && d_h, "gnk_cgs_update: null argument");
-  GNK_REQUIRE(k >= 1 && k <= GNK_MAX_BASIS, "gnk_cgs_update: k out of range");
+  GNK_REQUIRE(k >= 1 && k < GNK_MAX_BASIS_WIDE, "gnk_cgs_update: k out of range");
   GNK_REQUIRE((lay->off & 1) == 0 && (lay->ld & 1) == 0, "gnk_cgs_update: off/ld must be even");
   int grid = stream_grid(ctx, lay->n_own / 2, 8);
+  if (k >= GNK_MAX_BASIS) {
+    GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), update_wide_kernel, dim3(grid), dim3(TPB), sizeof(double) * k,
+                        (cudaStream_t)stream, d_V + lay->off, lay->ld, lay->n_own, k, d_h, d_w + lay->off,
+                        ctx->d_partials + PART_UPDATE, ctx->d_tickets + TK_UPDATE, d_stats,
+                        d_stats ? p2p_next(ctx) : gnk_p2p_dev{nullptr, 0, 1, 0ull}));
+    GNK_LAUNCH_CHECK(ctx);
+    return 0;
+  }
   GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), update_kernel, dim3(grid), dim3(TPB), 0, (cudaStream_t)stream, d_V + lay->off, lay->ld, lay->n_own, k,
                       d_h, d_w + lay->off, ctx->d_partials + PART_UPDATE, ctx->d_tickets + TK_UPDATE, d_stats,
                       d_stats ? p2p_next(ctx) : gnk_p2p_dev{nullptr, 0, 1, 0ull}));

@@ -38,11 +38,12 @@ class Runtime:
         self.ctx = ctx
         self.rank, self.world = 0, 1
         self.fused_reductions = False  # gnk_bratu_residual / gnk_cgs_dots / gnk_cgs_update reduce over the ranks themselves
-        # the largest read: the 2p + 4 result block of gnk_dense_qr_ls at p = GNK_DENSE_QR_MAX
-        self._pinned = torch.empty(2 * (_lib.GNK_DENSE_QR_MAX + 1) + 8, dtype=torch.float64, pin_memory=True)
+        # the largest reads: the 2p + 4 result block of gnk_dense_qr_ls at p = GNK_DENSE_QR_MAX, and the scalar block of
+        # gauss_newton_krylow with a basis of GNK_MAX_BASIS_WIDE - 1 columns (2 * GNK_MAX_BASIS_WIDE + 14 doubles)
+        self._pinned = torch.empty(2 * _lib.GNK_MAX_BASIS_WIDE + 16, dtype=torch.float64, pin_memory=True)
         self._pinned_np = self._pinned.numpy()
         self._pinned_ptr = self._pinned.data_ptr()
-        self._pinned2 = torch.empty(1024, dtype=torch.float64, pin_memory=True)
+        self._pinned2 = torch.empty(2 * _lib.GNK_MAX_BASIS_WIDE + 16, dtype=torch.float64, pin_memory=True)
         self._pinned2_np = self._pinned2.numpy()
         self._pinned2_ptr = self._pinned2.data_ptr()
         self._pinned_i = torch.empty(16, dtype=torch.int32, pin_memory=True)
@@ -183,8 +184,12 @@ class Runtime:
         return int(self.lib.gnk_launch_count(self.ctx))
 
     def allreduce(self, t, count, op=0):
+        """rank-ordered sum / max of t[:count] over the ranks, in collectives of at most 256 doubles (element-wise:
+        the chunking changes no bit)"""
         if self.world > 1:
-            _lib.check(self.lib.gnk_comm_allreduce(self.ctx, ptr(t), int(count), int(op), self.stream), "allreduce")
+            for off in range(0, int(count), 256):
+                _lib.check(self.lib.gnk_comm_allreduce(self.ctx, ptr(t, off), min(256, int(count) - off), int(op),
+                                                       self.stream), "allreduce")
 
 
 class _Mark:

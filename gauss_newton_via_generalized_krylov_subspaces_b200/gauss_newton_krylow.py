@@ -28,7 +28,7 @@ from .bratu_pde_problem import BratuDeviceProblem
 from .device import (DeviceCallableProblem, DeviceVector, HostCallableProblem, get_runtime, is_cuda_tensor,
                      make_layout, ptr)
 from .krylow import (GeneralizedKrylowSubspace, GeneralizedKrylowSubspaceBreakdown,
-                     GeneralizedKrylowSubspaceSpansEntireSpace, MAX_COLUMNS)
+                     GeneralizedKrylowSubspaceSpansEntireSpace, resolve_max_columns)
 from .partition import flat_layout_fields, round_up, tensor_ls_on_every_rank, trial_project_fused
 from .regression_result import RegressionResult
 from .rosenbrock_problem import RosenbrockDeviceProblem
@@ -36,12 +36,20 @@ from .rosenbrock_problem import RosenbrockDeviceProblem
 _NB = _lib.GNK_MAX_BASIS
 _TSQR_MAX = _lib.GNK_TSQR_MAX
 _DENSE_QR_MAX = 1 << 22  # doubles of the single-CTA wide-panel QR (csrc/tsqr.cu: run_dense_qr)
-# layout of the per-iteration scalar block (device, one D2H read per Armijo trial)
-_SC_LOSS = 2 * _NB + 8   # 2 doubles: sum(F^2) [, max|F|]
-_SC_CPREV = _SC_LOSS + 2  # sum(c_prev^2)
-_SC_FLAG = _SC_CPREV + 2   # int32 in a double slot: the deferred Krylov breakdown flag (krylow.dev_update)
-_SC_FLAG2 = _SC_CPREV + 3  # second slot: an expansion writes its flag to the slot that is NOT pending, committing it flips
-_BLK = _SC_CPREV + 6
+
+
+def scalar_layout(max_columns):
+    """Offsets of the per-iteration scalar block (device, one D2H read per Armijo trial) for a basis of at most
+    ``max_columns`` columns: [d(k) | g | resid2 | ndef | dnorm2 | diagR(k) ... | loss(2) | cprev2 | flag | flag2 ..].
+    Bases of up to 255 columns all get the layout of 255.  -> (loss, cprev, flag, flag2, total)"""
+    nb = max(_NB, max_columns + 1)
+    loss = 2 * nb + 8   # 2 doubles: sum(F^2) [, max|F|]
+    cprev = loss + 2    # sum(c_prev^2)
+    flag = cprev + 2    # int32 in a double slot: the deferred Krylov breakdown flag (krylow.dev_update)
+    flag2 = cprev + 3   # second slot: an expansion writes its flag to the slot that is NOT pending, committing it flips
+    return loss, cprev, flag, flag2, cprev + 6
+
+
 _VERSIONS = ("res_old", "res_new", "jac_old_res_old", "jac_old_res_new")
 
 
@@ -120,11 +128,12 @@ def cgls_dense(rt, JV, ldjv, n_rows, k, y, sign, rtol, out):
     Returns the number of CG iterations."""
     lib = rt.lib
     lay = make_layout(dict(flat_layout_fields(n_rows), ld=ldjv))
-    h = rt.zeros(_NB)
-    pdev = rt.zeros(_NB)
+    nb = max(_NB, k + 4)
+    h = rt.zeros(nb)
+    pdev = rt.zeros(nb)
     t = rt.empty(ldjv)
     stats = rt.zeros(2 * k)
-    stage = rt.pinned(_NB)
+    stage = rt.pinned(nb)
     stage_np = stage.numpy()
 
     def at_times(vec):  # A^T vec = sign * JV^T vec
@@ -238,6 +247,7 @@ def gauss_newton_krylow(
     x_on_device: bool = False,
     ls_solver: str = "qr",
     cg_rtol: float = 1e-4,
+    max_basis_columns: Optional[int] = None,
 ) -> RegressionResult:
     """
     Parameters
@@ -256,11 +266,16 @@ def gauss_newton_krylow(
         of the projected problem with tolerance ``cg_rtol`` (BASELINE config 5).
     x_on_device: leave the solution in HBM (RegressionResult.x is then a lazy DeviceVector).  x0 may likewise be a
         DeviceVector made by ``BratuPdeProblem.dev.resident(u0)``.
+    max_basis_columns: the widest Krylov basis the solve may build: None = 255, or an int in 1..4095.  A run without a
+        restart adds one column per iteration and raises GnkError when it would pass this width.  Bounds the device
+        memory of the basis: V_k and J V_k take 16 * n * max_basis_columns bytes.  Bases of 256 columns or more solve
+        the projected least squares by blocked Householder QR (gnk_basis_ls_wide).
 
     Returns
     -------
     RegressionResult
     """
+    max_basis_columns = resolve_max_columns(max_basis_columns, "max_basis_columns")
     rt = get_runtime()
     lib = rt.lib
     success = False
@@ -277,16 +292,18 @@ def gauss_newton_krylow(
     if krylow_restart is None:
         krylow_restart = max_iter
 
-    krylow = GeneralizedKrylowSubspace(prob, capacity=min(max_iter, krylow_restart) + 1, reorth_passes=reorth_passes)
+    krylow = GeneralizedKrylowSubspace(prob, capacity=min(max_iter, krylow_restart) + 1, reorth_passes=reorth_passes,
+                                       max_columns=max_basis_columns)
     krylow._setup(prob.p_glob, prob.sol_fields, prob.sol, prob, krylow.capacity)
     ld = krylow.ld
     sol_lay = prob.sol
 
-    blk = rt.zeros(_BLK)            # [d(k) | g | resid2 | ndef | dnorm2 | diagR(k) ... | loss(2) | cprev2]
-    loss_slot = blk[_SC_LOSS:_SC_LOSS + 2]
+    sc_loss, sc_cprev, sc_flag, sc_flag2, blk_len = scalar_layout(max_basis_columns)
+    blk = rt.zeros(blk_len)
+    loss_slot = blk[sc_loss:sc_loss + 2]
     # coordinates: the current point's c and the trial's c + s d, which gnk_combine_step leaves on the device (with the
     # next column's zero entry appended, :124); accepting a trial swaps the two -- no k-sized kernel is launched
-    cbuf = [rt.zeros(_NB), rt.zeros(_NB)]
+    cbuf = [rt.zeros(max(_NB, max_basis_columns + 1)) for _ in range(2)]
     c, c_next = cbuf
     one = rt.pinned(1)
 
@@ -347,10 +364,10 @@ def gauss_newton_krylow(
     jv_cap = 0
     # pending: the last basis expansion left its breakdown flag unread (see below); fslot: the slot that holds it.  A new
     # expansion always writes the OTHER slot, so neither a device copy nor a race with the read-back is needed.
-    state = {"pending": False, "fslot": _SC_FLAG}
+    state = {"pending": False, "fslot": sc_flag}
 
     def other_slot():
-        return _SC_FLAG2 if state["fslot"] == _SC_FLAG else _SC_FLAG
+        return sc_flag2 if state["fslot"] == sc_flag else sc_flag
 
     defer_ok = ls_solver == "qr" and os.environ.get("GNK_DEFER_BREAKDOWN", "1") != "0"
 
@@ -363,13 +380,15 @@ def gauss_newton_krylow(
             k = krylow.k
             state["rank_reported"] = False
             if k > jv_cap:
-                jv_cap = min(MAX_COLUMNS, max(krylow.cap, k))
-                JV = rt.empty(jv_cap * ldjv)
+                jv_cap = min(max_basis_columns, max(krylow.cap, k))
+                # from 256 columns on, the residual becomes column k of the panel [J V_k | r] that gnk_basis_ls_wide
+                # factors in place
+                JV = rt.empty((jv_cap + (jv_cap >= _NB)) * ldjv)
             # projected operator and projected least squares  (:86-89)
             ls_done = False
             # Bratu + QR: one TMA-staged kernel applies the stencil, stores J V_k and forms the Gram matrix of the
             # panel in the same sweep (gnk_stencil_gram_ls); it answers 1 when the panel does not qualify
-            if (is_bratu and ls_solver == "qr" and ls_method == 0 and not jac_ev.transposed
+            if (is_bratu and ls_solver == "qr" and ls_method == 0 and k < _NB and not jac_ev.transposed
                     and jac_ev.scale == 1.0):
                 # algorithmic bytes (SURVEY 8d): the SpMM's 16nk + 8n plus the least-squares panel once, 8n(k+1)
                 with rt.mark("spmm+ls", 8.0 * n_res_own * (3 * k + 2)) as mk:
@@ -386,6 +405,11 @@ def gauss_newton_krylow(
                     jac_ev.matmat(krylow.V, ld, k, JV, ldjv)
             if ls_done:
                 pass
+            elif ls_solver == "qr" and k >= _NB:
+                JV[k * ldjv:k * ldjv + n_res_own].copy_(F_cur[res_off:res_off + n_res_own])
+                with rt.mark("ls_wide", 8.0 * n_res_own * (k + 1)):
+                    _lib.check(lib.gnk_basis_ls_wide(rt.ctx, ptr(JV), ldjv, n_res_own, k, -1.0, ptr(blk), rt.stream),
+                               "gnk_basis_ls_wide")
             elif ls_solver == "qr":
                 with rt.mark("tsqr", 8.0 * n_res_own * (k + 1)):
                     tsqr_solve(rt, JV, ldjv, n_res_own, k, F_cur[res_off:], -1.0, blk, method=ls_method)
@@ -430,14 +454,14 @@ def gauss_newton_krylow(
                 # res_old expands with -J(x_trial)^T F_cur: the speculative trial point, that vector and its inner
                 # products with V_k come out of one pass over the basis instead of three
                 h_ready = (speculate and fuse_trial
-                           and krylow.dev_trial_project(prob.d.prm, c, blk, s, x_trial, c_next, ptr(blk, _SC_CPREV),
+                           and krylow.dev_trial_project(prob.d.prm, c, blk, s, x_trial, c_next, ptr(blk, sc_cprev),
                                                         F_cur))
                 if not h_ready:
-                    krylow.dev_combine(c, blk, s, x_trial, c_out=c_next, cprev2=ptr(blk, _SC_CPREV))
+                    krylow.dev_combine(c, blk, s, x_trial, c_out=c_next, cprev2=ptr(blk, sc_cprev))
                 with rt.mark("residual", 32.0 * n_res_own):
                     prob.residual(x_trial, F_trial, loss_slot, aux=aux[1])
                 if speculate:
-                    pending_read = rt.read_begin(blk, _BLK)   # the scalars of this trial are complete here ...
+                    pending_read = rt.read_begin(blk, blk_len)   # the scalars of this trial are complete here ...
                     jac_new = prob.jacobian(x_trial, aux=aux[1])
                     krylow.dev_expand_enqueue(*expansion_operands(jac_new), hx, ptr(blk, other_slot()),
                                               h_ready=h_ready)
@@ -446,7 +470,7 @@ def gauss_newton_krylow(
                 else:
                     if state["spec"] is not None:
                         state["spec"] = False  # a later trial: the speculation belonged to a rejected one
-                    state["vals"] = rt.read(blk, _BLK)
+                    state["vals"] = rt.read(blk, blk_len)
                 if state["pending"] and state["vals"][state["fslot"]:state["fslot"] + 1].view(np.int32)[0] != 0:
                     raise _DeferredBreakdown()
                 if ls_solver == "qr" and ls_refused(state["vals"], k):
@@ -456,7 +480,7 @@ def gauss_newton_krylow(
                     # judged: an exactly singular R must surface as LinAlgError, not as 100 rejected NaN trials
                     state["rank_reported"] = True
                     _report_rank(state["vals"], k)
-                return float(state["vals"][_SC_LOSS])
+                return float(state["vals"][sc_loss])
 
             def line_search():
                 return armijo_device(trial_loss, prev_loss, lambda: float(state["vals"][k]),
@@ -482,7 +506,7 @@ def gauss_newton_krylow(
         nfev += nfev_delta
         vals = state["vals"]
         squared_sum_d = float(vals[k + 3])
-        squared_sum_x_prev = float(vals[_SC_CPREV])
+        squared_sum_x_prev = float(vals[sc_cprev])
 
         # c += s d  (:98): the accepted trial's coordinates are already on the device
         c, c_next = c_next, c
@@ -548,7 +572,7 @@ def gauss_newton_krylow(
 
         # the trial becomes the current point
         F_cur, F_trial = F_trial, F_cur
-        prev_loss = float(vals[_SC_LOSS])
+        prev_loss = float(vals[sc_loss])
         if use_aux:
             aux[0], aux[1], aux[2] = aux[1], aux[2], aux[0]
         del jac_ev_old

@@ -18,6 +18,17 @@ from .device import CsrJacobian, HostCallableProblem, get_runtime, make_layout, 
 from .partition import flat_layout_fields
 
 MAX_COLUMNS = _lib.GNK_MAX_BASIS - 1  # the TSQR panel carries one extra right-hand-side column
+MAX_COLUMNS_WIDE = _lib.GNK_MAX_BASIS_WIDE - 1  # widest basis a caller may opt into (max_columns)
+
+
+def resolve_max_columns(max_columns, who="max_columns"):
+    """None -> MAX_COLUMNS (the default cap); an int in 1 .. MAX_COLUMNS_WIDE -> itself; anything else: ValueError"""
+    if max_columns is None:
+        return MAX_COLUMNS
+    if isinstance(max_columns, bool) or not isinstance(max_columns, (int, np.integer)) \
+            or not 1 <= int(max_columns) <= MAX_COLUMNS_WIDE:
+        raise ValueError(f"{who} must be None or an int in 1..{MAX_COLUMNS_WIDE}, got {max_columns!r}")
+    return int(max_columns)
 
 
 class GeneralizedKrylowSubspaceBreakdown(Exception):
@@ -43,11 +54,15 @@ class GeneralizedKrylowSubspace:
     Attributes
     ----------
     basis: The basis of the generalized Krylov subspace as an (n, k) host ndarray (downloaded on access).
+
+    max_columns: the widest basis this object may allocate (None: 255).  Up to 4095 columns may be asked for; V_k then
+    takes up to 8 * n * max_columns bytes of device memory.  Growing past it raises GnkError.
     """
 
-    def __init__(self, problem=None, capacity=None, reorth_passes=1):
+    def __init__(self, problem=None, capacity=None, reorth_passes=1, max_columns=None):
         self.problem = problem
         self.capacity = capacity
+        self.max_columns = resolve_max_columns(max_columns)
         self.reorth_passes = int(reorth_passes)
         self.k = 0
         self.V = None
@@ -61,21 +76,21 @@ class GeneralizedKrylowSubspace:
         self.fields, self.lay, self.owner = fields, lay, owner
         self.ld = fields["ld"]
         cap = min(self.n_glob, capacity if capacity is not None else 32)
-        self.cap = max(1, min(cap, MAX_COLUMNS))
+        self.cap = max(1, min(cap, self.max_columns))
         # no zero-fill of the basis storage (4 GB at 4096^2, k <= 30: 0.7 ms per solve): every column is written in full
         # -- owned rows and halo rows -- by the normalisation kernel before anything reads it, and columns >= k are
         # never part of any arithmetic (the fused least-squares kernel gives its padding lanes weight 0 on finite data)
         self.V = rt.empty(self.cap * self.ld)
         self.w = rt.zeros(self.ld)          # its halo rows stay zero: they become the new column's Dirichlet rows
-        self.h = rt.zeros(_lib.GNK_MAX_BASIS)
+        self.h = rt.zeros(max(_lib.GNK_MAX_BASIS, self.max_columns))
         self.stats = rt.zeros(2)
         self.flag = rt.zeros(1, dtype=rt.torch.int32)
         self._ready = True
 
     def _grow(self):
-        if self.cap >= MAX_COLUMNS:
-            raise _lib.GnkError(f"Krylov basis wider than {MAX_COLUMNS} columns is not supported; pass krylow_restart")
-        new_cap = min(MAX_COLUMNS, max(self.cap * 2, 2), self.n_glob)
+        if self.cap >= self.max_columns:
+            raise _lib.GnkError(f"Krylov basis wider than {self.max_columns} columns is not supported; pass krylow_restart")
+        new_cap = min(self.max_columns, max(self.cap * 2, 2), self.n_glob)
         V = self.rt.empty(new_cap * self.ld)
         V[:self.k * self.ld].copy_(self.V[:self.k * self.ld])
         self.V, self.cap = V, new_cap
@@ -216,7 +231,7 @@ class GeneralizedKrylowSubspace:
 
     def x(self, x_coordinate):
         rt = self.rt
-        c = rt.zeros(_lib.GNK_MAX_BASIS)
+        c = rt.zeros(max(_lib.GNK_MAX_BASIS, self.k))
         rt.upload(np.asarray(x_coordinate, dtype=np.float64), c[:self.k])
         out = rt.zeros(self.ld)
         self.dev_combine(c, None, 0.0, out)

@@ -35,6 +35,8 @@ extern "C" {
 
 #define GNK_B200_ABI_VERSION 1
 #define GNK_MAX_BASIS 256 /* k <= 255 basis columns (+1 rhs column in the least-squares panel) */
+#define GNK_MAX_BASIS_WIDE 4096 /* k <= 4095: the streaming entries (combine, dots, update) and gnk_basis_ls_wide for
+                                   bases grown without a restart; k <= 255 runs the kernels of GNK_MAX_BASIS */
 #define GNK_TSQR_MAX 104  /* widest panel of the tiled Householder TSQR; wider panels (runs without a restart) take
                              the single-CTA Householder QR on one rank while n_rows * (k+1) <= 2^22 doubles (it needs
                              n_rows >= k+1), and the blocked Householder TSQR spread over the SMs otherwise (several
@@ -100,13 +102,17 @@ int gnk_stencil_normal_diag(gnk_ctx* ctx, const gnk_layout* lay, const gnk_bratu
 
 /* ---- Krylov basis (krylow.py:30-73) ----------------------------------------------------------- */
 /* x = V_k (c + s d) over the whole stored column (krylow.py:41-42, armijo_goldstein.py:56).
- * d_d may be NULL (x = V_k c).  c, d are device vectors of length k. */
+ * d_d may be NULL (x = V_k c).  c, d are device vectors of length k.
+ * The four streaming entries below (gnk_combine, gnk_combine_step, gnk_cgs_dots, gnk_cgs_update) take
+ * 1 <= k < GNK_MAX_BASIS_WIDE.  For k <= 255 they launch the kernels they always did (same bits, one launch each).  For
+ * k >= 256 they launch wide kernels: still one pass over V_k per launch, the coefficients staged in 8k bytes of shared
+ * memory per CTA, and fixed-order "last CTA finishes" reductions (run-to-run and rank-to-rank deterministic). */
 int gnk_combine(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, const double* d_c,
                 const double* d_d, double s, double* d_x, void* stream);
 /* gnk_combine that also leaves the coordinate bookkeeping of the outer iteration on the device (gauss_newton_krylow.py
  * :96-98,124), so that no k-sized kernel has to be launched for it: d_c_out[j] = c[j] + s d[j] for j < k and
- * d_c_out[k] = 0 (the trial's x_coordinate with the entry of the next basis column appended; GNK_MAX_BASIS doubles,
- * must not alias d_c; may be NULL), *d_cprev2 = sum_j c[j]^2 (may be NULL). */
+ * d_c_out[k] = 0 (the trial's x_coordinate with the entry of the next basis column appended; GNK_MAX_BASIS doubles
+ * for k <= 255, k + 1 doubles above; must not alias d_c; may be NULL), *d_cprev2 = sum_j c[j]^2 (may be NULL). */
 int gnk_combine_step(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, const double* d_c,
                      const double* d_d, double s, double* d_x, double* d_c_out, double* d_cprev2, void* stream);
 /* d_stats[0] = sum of squares, d_stats[1] = max |.| over the owned part of a stored column
@@ -124,7 +130,8 @@ int gnk_normalize(gnk_ctx* ctx, const gnk_layout* lay, const double* d_x, const 
  * rank's halo rows.  Single rank / no mailboxes: gnk_normalize (+ gnk_comm_halo_exchange). */
 int gnk_normalize_halo(gnk_ctx* ctx, const gnk_layout* lay, const double* d_x, const double* d_stats, double atol,
                        double* d_out, int32_t* d_flag, void* stream);
-/* h = V_k^T w over owned entries (first half of krylow.py:64). */
+/* h = V_k^T w over owned entries (first half of krylow.py:64).  With the peer mailboxes attached h is summed over the
+ * ranks inside the kernel for every k (gnk_comm_fused_reductions); otherwise the caller all-reduces d_h[0..k). */
 int gnk_cgs_dots(gnk_ctx* ctx, const gnk_layout* lay, const double* d_V, int k, const double* d_w,
                  double* d_h, void* stream);
 /* w -= V_k h over owned entries (second half of krylow.py:64); d_stats as gnk_norm_stats of the
@@ -187,6 +194,20 @@ int gnk_tsqr_ls(gnk_ctx* ctx, const double* d_A, int64_t lda, int64_t n_rows, in
 #define GNK_DENSE_QR_MAX 4095
 int gnk_dense_qr_ls(gnk_ctx* ctx, double* d_A, int64_t lda, int64_t n_rows, int p, double sign_a, double* d_out,
                     void* stream);
+
+/* Projected least squares of a GNK outer iteration whose basis has 256 <= k <= 4095 columns (runs without a restart,
+ * gauss_newton_krylow.py:89): min || sign_a*JV d - r ||_2 on the row-sharded panel d_P = [JV | r] of n_rows x (k+1)
+ * (column-major, stride ldp; columns 0..k-1 = JV, column k = r), IN PLACE (the panel is overwritten).  Result block
+ * (device, 2k+4 doubles) exactly as gnk_tsqr_ls.
+ *   One rank: gnk_dense_qr_ls on the panel; needs n_rows >= k+1 (fewer residuals than basis columns is refused, as the
+ *   reference's economic QR + solve_triangular fails there).
+ *   Several ranks: every rank factors its slab with the same blocked Householder kernels (a slab of fewer than k+1 rows
+ *   goes through a zero-padded scratch panel of k+1 rows), packs its (k+1) x (k+1) triangle [[R, Q^T r], [0, rho]]
+ *   (rho = norm of the slab's residual part of Q^T r), all-gathers the triangles (NCCL above the mailbox size) and
+ *   factors the stack in rank order: every rank computes the same bits.  Scratch belongs to the context.
+ * Every reduction has a fixed order: repeated calls give the same bits, a power-of-two scaling changes no rounding. */
+int gnk_basis_ls_wide(gnk_ctx* ctx, double* d_P, int64_t ldp, int64_t n_rows, int k, double sign_a, double* d_out,
+                      void* stream);
 
 /* Projected operator AND projected least squares of one GNK outer iteration in one call, for the Bratu stencil
  * (gauss_newton_krylow.py:86 `JV = jac_ev @ krylow.basis` followed by :89 `linear_least_squares(-1 * JV, res_ev)`):

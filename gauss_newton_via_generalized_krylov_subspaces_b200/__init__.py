@@ -23,7 +23,7 @@ from .krylow import (GeneralizedKrylowSubspace, GeneralizedKrylowSubspaceBreakdo
 from .bratu_pde_problem import BratuPdeProblem, default_u  # noqa: E402
 from .gauss_newton_krylow import gauss_newton_krylow, linear_least_squares  # noqa: E402
 from .gauss_newton import cg_least_squares, gauss_newton  # noqa: E402
-from .device import DeviceVector, get_runtime  # noqa: E402
+from .device import DeviceLinearOperator, DeviceVector, autograd_jacobian, get_runtime  # noqa: E402
 
 
 def install_flat_names(overwrite=True):
@@ -36,4 +36,4 @@ def install_flat_names(overwrite=True):
 __all__ = ["RegressionResult", "StepLengthConvergenceError", "armijo_goldstein", "GeneralizedKrylowSubspace",
            "GeneralizedKrylowSubspaceBreakdown", "GeneralizedKrylowSubspaceSpansEntireSpace", "BratuPdeProblem",
            "default_u", "gauss_newton_krylow", "linear_least_squares", "cg_least_squares", "gauss_newton",
-           "DeviceVector", "get_runtime", "install_flat_names"]
+           "DeviceLinearOperator", "DeviceVector", "autograd_jacobian", "get_runtime", "install_flat_names"]

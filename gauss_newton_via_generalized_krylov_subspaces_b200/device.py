@@ -167,8 +167,8 @@ class Runtime:
         out.copy_(src, non_blocking=True)
 
     def download(self, t):
-        """device tensor -> new host ndarray (through a pinned staging buffer it owns)."""
-        h = self.pinned(t.numel(), t.dtype)
+        """device tensor -> new host ndarray of the same shape (through a pinned staging buffer it owns)."""
+        h = self.pinned(t.numel(), t.dtype).view(t.shape)
         h.copy_(t, non_blocking=True)
         self.sync()
         return h.numpy()
@@ -507,6 +507,75 @@ class DenseJacobian:
             panel[:p, :n].copy_(torch.from_numpy(np.ascontiguousarray(a)).to(panel.device).T)
 
 
+class HostBasisMirror:
+    """An F-ordered host copy of the leading columns of a Krylov basis that lives in HBM, for operators that run on the
+    host.  ``view`` downloads only the columns appended since the last call (8 p bytes per new column, not 8 p k per
+    product); the basis calls ``truncate`` when it restarts (``dev_start``) or retracts a column, since the device
+    column at that index is then rewritten.  Columns below ``valid`` hold the device columns bit for bit."""
+
+    def __init__(self, rt, p):
+        self.rt, self.p = rt, int(p)
+        self.a = np.empty((self.p, 0), order="F")
+        self.valid = 0
+
+    def truncate(self, k):
+        self.valid = min(self.valid, int(k))
+
+    def view(self, V, ldv, k):
+        """read-only (p, k) view of V_k (V: the stored columns, ``ldv`` doubles apart)"""
+        if k > self.a.shape[1]:
+            a = np.empty((self.p, max(k, 2 * self.a.shape[1])), order="F")
+            a[:, :self.valid] = self.a[:, :self.valid]
+            self.a = a
+        if k > self.valid:
+            cols = V[self.valid * ldv:k * ldv].view(k - self.valid, ldv)[:, :self.p]
+            self.a.T[self.valid:k] = self.rt.download(cols)
+            self.valid = k
+        v = self.a[:, :k]
+        v.flags.writeable = False  # an operator that wrote here would desynchronise the mirror from the device basis
+        return v
+
+
+class HostOperatorJacobian:
+    """A scipy.sparse.linalg.LinearOperator Jacobian, applied on the host with the reference's own expressions:
+    ``J @ V_k`` on a host mirror of the basis, uploaded into the J V_k panel, and ``-J.T @ r`` on the downloaded
+    residual.  ``mirror`` is the HostBasisMirror of the basis the products run over (None: stand-alone ``update``,
+    which forms only -J^T r)."""
+
+    transposed = False
+    scale = 1.0
+    is_sparse = False
+    matrix_free = True
+
+    def __init__(self, rt, op, mirror=None):
+        self.rt, self.user, self.mirror = rt, op, mirror
+        self.n_res, self.p = (int(v) for v in op.shape)
+
+    def matmat(self, V, ldv, k, JV, ldjv):
+        J, rt = self.user, self.rt
+        with rt.mark("op_matmat", 0.0):  # the host's share, mirror download and upload included
+            JVk = np.asarray(J @ self.mirror.view(V, ldv, k), dtype=np.float64)
+            if JVk.shape != (self.n_res, k):
+                raise ValueError(f"jac: the LinearOperator's J @ V_k has shape {JVk.shape}, expected {(self.n_res, k)}")
+            rt.upload(JVk.T, JV[:k * ldjv].view(k, ldjv)[:, :self.n_res])
+
+    def neg_rmatvec(self, r, w):
+        J, rt = self.user, self.rt
+        with rt.mark("op_rmatvec", 0.0):
+            r = rt.download(r[:self.n_res])
+            w_host = np.asarray(-J.T @ r, dtype=np.float64)
+            if w_host.shape != (self.p,):
+                raise ValueError(f"jac: the LinearOperator's -J.T @ r has shape {w_host.shape}, expected {(self.p,)}")
+            rt.upload(w_host, w[:self.p])
+
+
+def _host_operator(rt, J, shape, mirror=None):
+    """a scipy LinearOperator of shape ``shape`` (n_res, p) -> HostOperatorJacobian; any other shape: ValueError"""
+    if tuple(J.shape) != tuple(shape):
+        raise ValueError(f"jac: expected a LinearOperator of shape {tuple(shape)} (n_res, p), got {tuple(J.shape)}")
+    return HostOperatorJacobian(rt, J, mirror)
+
+
 class HostCallableProblem:
     """res / jac are arbitrary Python callables returning host objects."""
 
@@ -521,6 +590,7 @@ class HostCallableProblem:
         self.n_res = None
         self.res_fields = None
         self.last_res_host = None
+        self.basis_mirror = None  # HostBasisMirror, made when jac first returns a LinearOperator
 
     # residual-space layout is known after the first residual evaluation
     def _ensure_res_layout(self, n_res):
@@ -563,10 +633,16 @@ class HostCallableProblem:
 
     def jacobian_host(self, x_host, dense_panel=False):
         """jac at x_host as a CsrJacobian; with ``dense_panel`` a dense J of p >= GNK_DENSE_QR_MIN columns comes back as a
-        DenseJacobian instead (gauss_newton's blocked QR branch, which needs no CSR form)"""
+        DenseJacobian instead (gauss_newton's blocked QR branch, which needs no CSR form); a scipy LinearOperator comes
+        back as a HostOperatorJacobian over this problem's basis mirror"""
         import scipy.sparse as sp
+        from scipy.sparse.linalg import LinearOperator
 
         J = self.jac(x_host, *self.args)
+        if isinstance(J, LinearOperator):
+            if self.basis_mirror is None:
+                self.basis_mirror = HostBasisMirror(self.rt, self.p_glob)
+            return _host_operator(self.rt, J, (self.n_res, self.p_glob), self.basis_mirror)
         sparse = isinstance(J, (sp.sparray, sp.spmatrix)) or hasattr(J, "_gnk_sparse_like")
         if dense_panel and not sparse and not hasattr(J, "tocsr") and self.p_glob >= _lib.GNK_DENSE_QR_MIN:
             if np.ndim(J) != 2 or np.shape(J)[1] != self.p_glob:
@@ -734,9 +810,132 @@ class DenseDeviceJacobian:
         return op
 
 
+class DeviceLinearOperator:
+    """A matrix-free Jacobian on CUDA tensors, for ``jac`` of a problem whose ``x0`` is a CUDA tensor -- named after
+    scipy.sparse.linalg.LinearOperator.
+
+    shape: (n_res, p).
+    matvec(v): (p,) -> (n_res,), the product J v.
+    rmatvec(u): (n_res,) -> (p,), the product J^T u.  Required: every basis expansion needs -J^T r.
+    matmat(V): (p, k) -> (n_res, k), the product J V.  Default: ``matvec`` over the columns of V, stacked.
+
+    Inputs and outputs are CUDA tensors on one device.  An output of another floating-point dtype is converted to
+    float64; an output that is not a strided tensor on the input's device, or has the wrong shape, raises TypeError /
+    ValueError naming the expected and actual values.  gauss_newton_krylow calls ``matmat`` once per outer iteration
+    with a (p, k) view of its Krylov basis (no copy: do not write into it) and ``rmatvec`` once per basis expansion, and
+    uses the operator only until the next ``jac`` call returns.  gauss_newton and cg_least_squares do not take
+    operators: they need J itself."""
+
+    def __init__(self, shape, matvec=None, rmatvec=None, matmat=None):
+        if len(shape) != 2 or any(isinstance(v, bool) or not isinstance(v, (int, np.integer)) or v < 0 for v in shape):
+            raise ValueError(f"DeviceLinearOperator: shape must be (n_res, p) of two ints >= 0, got {shape!r}")
+        if rmatvec is None:
+            raise TypeError("DeviceLinearOperator: rmatvec is required (gauss_newton_krylow expands its basis with -J^T r)")
+        if matvec is None and matmat is None:
+            raise TypeError("DeviceLinearOperator: give matvec, matmat or both")
+        self.shape = (int(shape[0]), int(shape[1]))
+        self._matvec, self._rmatvec, self._matmat = matvec, rmatvec, matmat
+
+    def _io(self, t, what, shape, like=None):
+        """checks a tensor against ``shape`` (and ``like``'s device) -> the tensor as float64"""
+        import torch
+        dev = like.device if like is not None else None
+        if not isinstance(t, torch.Tensor) or t.layout != torch.strided:
+            got = type(t).__name__ if not isinstance(t, torch.Tensor) else f"a tensor of layout {t.layout}"
+            raise TypeError(f"{what}: expected a strided torch.Tensor{f' on {dev}' if dev else ''}, got {got}")
+        if dev is not None and t.device != dev:
+            raise ValueError(f"{what}: expected a tensor on {dev}, got one on {t.device}")
+        if tuple(t.shape) != shape:
+            raise ValueError(f"{what}: expected shape {shape}, got {tuple(t.shape)}")
+        if not t.is_floating_point():
+            raise TypeError(f"{what}: expected a floating-point tensor, got dtype {t.dtype}")
+        return t if t.dtype == torch.float64 else t.to(torch.float64)
+
+    def matvec(self, v):
+        n_res, p = self.shape
+        v = self._io(v, "DeviceLinearOperator.matvec: v", (p,))
+        if self._matvec is None:
+            return self.matmat(v[:, None])[:, 0]
+        return self._io(self._matvec(v), "DeviceLinearOperator.matvec", (n_res,), v)
+
+    def rmatvec(self, u):
+        n_res, p = self.shape
+        u = self._io(u, "DeviceLinearOperator.rmatvec: u", (n_res,))
+        return self._io(self._rmatvec(u), "DeviceLinearOperator.rmatvec", (p,), u)
+
+    def matmat(self, V):
+        import torch
+        n_res, p = self.shape
+        k = V.shape[1] if isinstance(V, torch.Tensor) and V.dim() == 2 else -1
+        V = self._io(V, "DeviceLinearOperator.matmat: V", (p, k))
+        if self._matmat is None:
+            if k == 0:
+                return V.new_zeros((n_res, 0))
+            return torch.stack([self.matvec(V[:, j]) for j in range(k)], dim=1)
+        return self._io(self._matmat(V), "DeviceLinearOperator.matmat", (n_res, k), V)
+
+
+def autograd_jacobian(res):
+    """-> jac(x, *args) returning a DeviceLinearOperator of res's Jacobian at x, built with torch.func: J v by ``jvp``,
+    J V by ``vmap`` of that ``jvp`` over the columns (one batched forward-mode pass), and J^T u by the ``vjp`` taken
+    once per operator.  Gives gauss_newton_krylow without a Jacobian: only res, on CUDA tensors, must be differentiable
+    by torch.
+
+    Each jac call evaluates res once more (the vjp's forward pass) and keeps that pass's saved tensors until the
+    operator is dropped, at the next jac call.  If res cannot run under ``vmap`` (data-dependent control flow, in-place
+    writes into a tensor that is not batched, ``.item()``), build the operator yourself with ``matvec`` alone, for
+    example ``DeviceLinearOperator(shape, matvec=lambda v: torch.func.jvp(f, (x,), (v,))[1], rmatvec=...)``: J V is
+    then formed one column at a time."""
+    from torch.func import jvp, vjp, vmap
+
+    def jac(x, *args):
+        def f(y):
+            return res(y, *args)
+
+        fx, pullback = vjp(f, x)
+
+        def matvec(v):
+            return jvp(f, (x,), (v,))[1]
+
+        return DeviceLinearOperator((int(fx.shape[0]), int(x.shape[0])), matvec=matvec,
+                                    rmatvec=lambda u: pullback(u)[0],
+                                    matmat=vmap(matvec, in_dims=1, out_dims=1))
+
+    return jac
+
+
+class DeviceOperatorJacobian:
+    """A DeviceLinearOperator behind the Jacobian interface of the solvers: J V_k by one ``matmat`` call on a view of the
+    basis (no copy), copied into the J V_k panel with one device-to-device copy, and -J^T r by one ``rmatvec`` call.
+    ``user`` is the operator."""
+
+    transposed = False
+    scale = 1.0
+    is_sparse = False
+    matrix_free = True
+
+    def __init__(self, rt, op):
+        self.rt, self.user = rt, op
+        self.n_res, self.p = op.shape
+
+    def matmat(self, V, ldv, k, JV, ldjv):
+        rt = self.rt
+        with rt.mark("op_matmat", 0.0):
+            JVk = self.user.matmat(V[:k * ldv].view(k, ldv)[:, :self.p].T)
+        with rt.mark("panel_copy", 16.0 * self.n_res * k):
+            JV[:k * ldjv].view(k, ldjv)[:, :self.n_res].copy_(JVk.T)
+
+    def neg_rmatvec(self, r, w):
+        rt = self.rt
+        with rt.mark("op_rmatvec", 0.0):
+            u = self.user.rmatvec(r[:self.n_res])
+        rt.torch.neg(u, out=w[:self.p])
+
+
 class DeviceCallableProblem:
     """res / jac are Python callables on CUDA tensors: res(x, *args) -> 1-D tensor of n_res values, jac(x, *args) ->
-    torch sparse CSR / COO or strided (n_res, p) tensor.  x is a fresh float64 tensor of length p at every call."""
+    torch sparse CSR / COO or strided (n_res, p) tensor, or a DeviceLinearOperator (gauss_newton_krylow only).  x is a
+    fresh float64 tensor of length p at every call."""
 
     distributed = False
     device_native = True  # x and F stay in HBM
@@ -802,9 +1001,15 @@ class DeviceCallableProblem:
 
     def jacobian(self, x, aux=None, dense_panel=False):
         """jac at x: a strided J as a DenseDeviceJacobian -- or, with ``dense_panel`` and p >= GNK_DENSE_QR_MIN, as a
-        DenseJacobian (gauss_newton's blocked QR branch) -- and a sparse J as a DeviceCsrJacobian"""
+        DenseJacobian (gauss_newton's blocked QR branch) -- a sparse J as a DeviceCsrJacobian, and a DeviceLinearOperator
+        as a DeviceOperatorJacobian"""
         J = self.jac(self.x_out(x), *self.args)
         torch = self.rt.torch
+        if isinstance(J, DeviceLinearOperator):
+            if J.shape != (self.n_res, self.p_glob):
+                raise ValueError(f"jac: expected a DeviceLinearOperator of shape {(self.n_res, self.p_glob)} (n_res, p), "
+                                 f"got {J.shape}")
+            return DeviceOperatorJacobian(self.rt, J)
         if isinstance(J, torch.Tensor) and J.layout == torch.strided:
             _require_on_device(self.rt, J, "jac")
             panel = dense_panel and self.p_glob >= _lib.GNK_DENSE_QR_MIN

@@ -21,8 +21,8 @@ import numpy as np
 from . import _lib
 from .armijo_goldstein import armijo_device, armijo_goldstein
 from .bratu_pde_problem import BratuDeviceProblem, StencilJacobian
-from .device import (_INT32_LIMIT, CsrJacobian, DenseDeviceJacobian, DenseJacobian, DeviceCsrJacobian, DeviceVector,
-                     _require_on_device, get_runtime, is_cuda_tensor, make_layout, ptr)
+from .device import (_INT32_LIMIT, CsrJacobian, DenseDeviceJacobian, DenseJacobian, DeviceCsrJacobian,
+                     DeviceLinearOperator, DeviceVector, _require_on_device, get_runtime, is_cuda_tensor, make_layout, ptr)
 from .gauss_newton_krylow import _report_rank, require_single_rank_unless_sharded, resolve_problem, tsqr_solve
 from .partition import flat_layout_fields, round_up
 from .regression_result import RegressionResult
@@ -51,6 +51,13 @@ def _device_operator(rt, A, what="cg_least_squares: A"):
     return DenseDeviceJacobian(rt, A)
 
 
+def _refuse_operator(who, J):
+    """matrix-free operators serve gauss_newton_krylow only: these solvers need J's entries (the reference fails here
+    too, in scipy.linalg.lstsq(-1 * J, r) and in the A.T @ A of its Jacobi preconditioner)"""
+    raise TypeError(f"{who}: got a {type(J).__name__}, a matrix-free operator; {who} needs the Jacobian's entries "
+                    "(a dense array or a sparse matrix).  Matrix-free Jacobians are taken by gauss_newton_krylow.")
+
+
 def cg_least_squares(A, y, x0=None, cg_rtol=1e-4, preconditioner=True):
     """Iterative solver for min ||y - A x|| via CG on the normal equations (reference :11-60), on the device.
 
@@ -59,6 +66,9 @@ def cg_least_squares(A, y, x0=None, cg_rtol=1e-4, preconditioner=True):
     contiguous float64 copy if it is of another dtype or has no unit stride), with no CSR form and no limit on its number
     of entries; the result is the one its CSR form gives, bit for bit.  Returns (x, cg_iter) where cg_iter
     sums the unpreconditioned and the preconditioned run when ``preconditioner`` is False (reference quirk)."""
+    from scipy.sparse.linalg import LinearOperator
+    if isinstance(A, (LinearOperator, DeviceLinearOperator)):
+        _refuse_operator("cg_least_squares", A)
     rt = get_runtime()
     if is_cuda_tensor(A):
         require_single_rank_unless_sharded(rt, None, "cg_least_squares")
@@ -208,6 +218,8 @@ def gauss_newton(
             jac_ev = prob.jacobian_host(x_host, dense_panel=dense_qr)
             sparse_like = jac_ev.is_sparse
         njev += 1
+        if getattr(jac_ev, "matrix_free", False):
+            _refuse_operator("gauss_newton", jac_ev.user)
         panel_qr = dense_qr and not sparse_like
         if panel_qr and not isinstance(jac_ev, DenseJacobian):  # a dense object with a tocsr method of its own
             jac_ev = DenseJacobian(rt, host=jac_ev.host)

@@ -14,7 +14,7 @@ import math
 import numpy as np
 
 from . import _lib
-from .device import CsrJacobian, HostCallableProblem, get_runtime, make_layout, ptr
+from .device import CsrJacobian, HostCallableProblem, _host_operator, get_runtime, make_layout, ptr
 from .partition import flat_layout_fields
 
 MAX_COLUMNS = _lib.GNK_MAX_BASIS - 1  # the TSQR panel carries one extra right-hand-side column
@@ -110,7 +110,15 @@ class GeneralizedKrylowSubspace:
         if ss[1] <= 1e-8:
             raise ValueError("x0 is not allowed to be 0 in the gauss_newton_krylow algorithm")
         self.k = 1
+        self._truncate_mirror(0)  # column 0 is new
         return math.sqrt(ss[0])
+
+    def _truncate_mirror(self, k):
+        """the host copy of V_k that a host LinearOperator Jacobian reads keeps only the columns below ``k``: the device
+        rewrites the others"""
+        mirror = getattr(self.owner, "basis_mirror", None)
+        if mirror is not None:
+            mirror.truncate(k)
 
     def dev_combine(self, c, d, s, out, c_out=None, cprev2=None):
         """out = V_k (c + s d) over the whole stored column (krylow.py:41-42); optionally the coordinates c + s d (with
@@ -205,6 +213,7 @@ class GeneralizedKrylowSubspace:
     def retract(self):
         """undo a speculative append whose deferred breakdown flag turned out to be set (the column was not written)"""
         self.k -= 1
+        self._truncate_mirror(self.k)
 
     # ---- the reference's public interface (host ndarrays) -------------------------------------------
     @property
@@ -252,8 +261,12 @@ class GeneralizedKrylowSubspace:
             hx = self.problem.d.halo_exchange if getattr(self.problem, "distributed", False) else None
         else:
             import scipy.sparse as sp
-            op = CsrJacobian(rt, jac_ev, isinstance(jac_ev, (sp.sparray, sp.spmatrix)))
+            from scipy.sparse.linalg import LinearOperator
             res_ev = np.asarray(res_ev, dtype=np.float64).reshape(-1)
+            if isinstance(jac_ev, LinearOperator):  # -J.T @ r on the host (the reference's krylow.py:62)
+                op = _host_operator(rt, jac_ev, (res_ev.shape[0], self.n_glob))
+            else:
+                op = CsrJacobian(rt, jac_ev, isinstance(jac_ev, (sp.sparray, sp.spmatrix)))
             r = rt.zeros(flat_layout_fields(res_ev.shape[0])["ld"])
             rt.upload(res_ev, r[:res_ev.shape[0]])
             hx = None

@@ -721,6 +721,19 @@ int launch_refine(gnk_ctx* ctx, const PanelSource& src, double sign, double* bas
   return 0;
 }
 
+int launch_refine_any(gnk_ctx* ctx, const PanelSource& src, double sign, double* base, int* status, cudaStream_t st) {
+  if (src.k <= 8) return launch_refine<8>(ctx, src, sign, base, status, st);
+  if (src.k <= 16) return launch_refine<16>(ctx, src, sign, base, status, st);
+  if (src.k <= 24) return launch_refine<24>(ctx, src, sign, base, status, st);
+  return launch_refine<32>(ctx, src, sign, base, status, st);
+}
+
+// second pass: 0 the refinement form (chosen on the device, see cholqr_factor1_kernel), 2 always CholeskyQR2
+int second_pass_method(const gnk_ctx* ctx) {
+  static const int refine_on = getenv("GNK_LS_REFINE") ? atoi(getenv("GNK_LS_REFINE")) : 1;
+  return (ctx->ls_method == 2 || !refine_on) ? 2 : 0;
+}
+
 int ensure_scratch(gnk_ctx* ctx, cudaStream_t st) {
   if (!ctx->d_cholqr) {
     GNK_CUDA(cudaMalloc(&ctx->d_cholqr, sizeof(double) * CQ_TOTAL));
@@ -729,10 +742,11 @@ int ensure_scratch(gnk_ctx* ctx, cudaStream_t st) {
   return 0;
 }
 
-// Everything after pass 1: this rank's Gram matrix of [A | y] (fragment order) is at base + CQ_LOCAL.
-template <int NB, int RU>
+// Everything after pass 1: this rank's Gram matrix of [A | y] (fragment order) is at base + CQ_LOCAL.  refine(status)
+// launches the refinement form of pass 2 (d_A may be null if it does not read A; the CholeskyQR2 pass does).
+template <int NB, int RU, class Refine>
 int cholqr_tail(gnk_ctx* ctx, const double* d_A, int64_t lda, int64_t n_rows, int k, const double* d_y, double sign,
-                double* d_out, cudaStream_t st) {
+                double* d_out, cudaStream_t st, Refine&& refine) {
   double* base = ctx->d_cholqr;
   int* status = reinterpret_cast<int*>(base + CQ_STATUS);
   PanelSource src{d_A, lda, d_y, k, n_rows};
@@ -744,8 +758,7 @@ int cholqr_tail(gnk_ctx* ctx, const double* d_A, int64_t lda, int64_t n_rows, in
   const int NE = nblocks(NB) * 64;
   const bool multi = ctx->nranks > 1;
   GNK_REQUIRE(ctx->nranks <= P2P_MAXR, "cholqr: more ranks than the Gram gather buffer holds");
-  static const int refine_on = getenv("GNK_LS_REFINE") ? atoi(getenv("GNK_LS_REFINE")) : 1;
-  const int method = (ctx->ls_method == 2 || !refine_on) ? 2 : 0;
+  const int method = second_pass_method(ctx);
   // with the peer mailboxes attached the factor kernels (single CTAs) run the cross-rank sum themselves
   const gnk_p2p_dev none{nullptr, 0, 1, 0ull};
   const gnk_p2p_dev pd1 = multi ? p2p_next(ctx) : none;
@@ -758,14 +771,8 @@ int cholqr_tail(gnk_ctx* ctx, const double* d_A, int64_t lda, int64_t n_rows, in
   GNK_LAUNCH_CHECK(ctx);
   // pass 2: the refinement form by default (it returns at once unless the status word says 0); the second CholeskyQR2
   // pass only when the caller asked for it (gnk_tsqr_ls_method 2)
-  if (method == 0) {
-    int rc;
-    if (k <= 8) rc = launch_refine<8>(ctx, src, sign, base, status, st);
-    else if (k <= 16) rc = launch_refine<16>(ctx, src, sign, base, status, st);
-    else if (k <= 24) rc = launch_refine<24>(ctx, src, sign, base, status, st);
-    else rc = launch_refine<32>(ctx, src, sign, base, status, st);
-    if (rc) return rc;
-  }
+  if (method == 0)
+    if (int rc = refine(status)) return rc;
   if (method == 2) {
     cholqr_gram2_kernel<NB, RU><<<(unsigned)ctas, GT, 0, st>>>(src, rows_per_cta, base + CQ_T, status, base + CQ_PART,
                                                            ctx->d_tickets + TK_CHOLQR, base + CQ_LOCAL2 + GPAD);
@@ -797,7 +804,9 @@ int run_cholqr(gnk_ctx* ctx, const double* d_A, int64_t lda, int64_t n_rows, int
   GNK_CUDA(gnk_launch(gnk_pdl_for(n_rows), cholqr_gram_kernel<NB, RU>, dim3((unsigned)ctas), dim3(GT), 0, st, src, rows_per_cta,
                       base + CQ_PART, ctx->d_tickets + TK_CHOLQR, base + CQ_LOCAL));
   GNK_LAUNCH_CHECK(ctx);
-  return cholqr_tail<NB, RU>(ctx, d_A, lda, n_rows, k, d_y, sign, d_out, st);
+  return cholqr_tail<NB, RU>(ctx, d_A, lda, n_rows, k, d_y, sign, d_out, st, [&](int* status) {
+    return launch_refine_any(ctx, src, sign, base, status, st);
+  });
 }
 
 // ======================================================================================================================
@@ -880,18 +889,20 @@ __device__ __forceinline__ double lds1(uint32_t a) {
   return v;
 }
 
-template <int NB, int CW>
-__global__ void __launch_bounds__(32 * (CW + 1), 1)
-    stencil_gram_kernel(const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmY,
-                        const __grid_constant__ CUtensorMap tmE, StencilPanel p, int TI, double* __restrict__ JV,
-                        double* __restrict__ partials, unsigned int* ticket, double* __restrict__ Gout) {
-  constexpr int NBLK = nblocks(NB);
+// The sweep shared by the Gram pass and the store-free refinement: ring set-up, producer warp and the 3-row register
+// window.  Every consumer lane calls on_row(tile, e) once per grid row of its segment, e = flat offset of its point pair
+// (grid row * m + j) among the owned unknowns, tile[I] = (sign J V)[e, e + 1] of column 8 I + g -- bit-identical to
+// gnk_stencil_apply -- where the column after the basis holds the residual exactly and the columns beyond it zeros.
+// Returns false at once (nothing issued) if `status` is given and is not 0 (the refinement form was not chosen);
+// otherwise every consumer lane calls on_start() before its first row (after the wait on the predecessor kernel).
+template <int NB, int CW, class OnStart, class OnRow>
+__device__ __forceinline__ bool stencil_sweep(const CUtensorMap& tmV, const CUtensorMap& tmY, const CUtensorMap& tmE,
+                                              const StencilPanel& p, int TI, const int* status, OnStart&& on_start,
+                                              OnRow&& on_row) {
   constexpr int SB = sg_slot_bytes<NB, CW>();
   constexpr int NS = sg_nslot<NB, CW>();
   constexpr int TJ = 8 * CW, PB = sg_plane_bytes<CW>(), YE = sg_ye_bytes<CW>();
-  constexpr int NT = 32 * (CW + 1);
   extern __shared__ __align__(128) unsigned char ring[];
-  __shared__ __align__(16) double red[NBLK * 64];
   __shared__ __align__(8) unsigned long long bars[2 * NS];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int g = lane >> 2, t = lane & 3;
@@ -909,10 +920,7 @@ __global__ void __launch_bounds__(32 * (CW + 1), 1)
   }
   __syncthreads();
   pdl_begin();  // the ring is set up while the predecessor drains; nothing global has been touched yet
-
-  double acc[NBLK][2];
-#pragma unroll
-  for (int b = 0; b < NBLK; ++b) acc[b][0] = acc[b][1] = 0.0;
+  if (status != nullptr && *status != 0) return false;  // uniform across the grid
 
   if (warp == CW) {
     if (lane == 0) {
@@ -935,137 +943,239 @@ __global__ void __launch_bounds__(32 * (CW + 1), 1)
         }
       }
     }
-  } else {
-    // the sign is folded into the weights (exact: every product and every sum is negated symmetrically)
-    const double sg = p.sign;
-    const double d0 = __dadd_rn(4.0 * p.c_lap, -p.c_adv);
-    const double cd = sg * __dadd_rn(-p.c_lap, p.c_adv), cu = sg * -p.c_lap, cl = sg * -p.c_lap;
-    // per column block: byte offset of this lane's pair inside a slot, and what the column is.  Only the LAST block can
-    // hold anything but basis columns (k >= 8 (NB - 1) by the choice of NB).
-    uint32_t poff[NB];
+    return true;
+  }
+  // the sign is folded into the weights (exact: every product and every sum is negated symmetrically)
+  const double sg = p.sign;
+  const double d0 = __dadd_rn(4.0 * p.c_lap, -p.c_adv);
+  const double cd = sg * __dadd_rn(-p.c_lap, p.c_adv), cu = sg * -p.c_lap, cl = sg * -p.c_lap;
+  // per column block: byte offset of this lane's pair inside a slot, and what the column is.  Only the LAST block can
+  // hold anything but basis columns (k >= 8 (NB - 1) by the choice of NB).
+  uint32_t poff[NB];
 #pragma unroll
-    for (int I = 0; I < NB; ++I) poff[I] = (uint32_t)((8 * I + g) * PB + 8 * (4 + 8 * warp + 2 * t));
-    const int lastcol = 8 * (NB - 1) + g;
-    const int lastkind = lastcol < p.k ? 0 : (lastcol == p.k ? 1 : 2);  // 0 basis column, 1 the residual, 2 padding
-    if (lastkind == 1) poff[NB - 1] = (uint32_t)(8 * NB * PB + 8 * (4 + 8 * warp + 2 * t));
-    if (lastkind == 2) poff[NB - 1] = poff[0];                          // any valid (finite) data; multiplied by 0
-    // No selects in the loop: the last block runs the same stencil code with per-lane weights -- a basis column keeps
-    // (cu, cl, dg, cd); the residual column uses (0, 0, 1, 0), which returns `mid` exactly (0 * finite = 0, 0 + x = x);
-    // a padding column uses all zeros.  dg = wsel * (d0 + lam e) + wone is exact for wsel, wone in {0, 1}.
-    const double wsel = lastkind == 0 ? 1.0 : 0.0, wone = lastkind == 1 ? 1.0 : 0.0;
-    const double cuL = wsel * cu, clL = wsel * cl, cdL = wsel * cd;
-    const uint32_t eoff = (uint32_t)(8 * NB * PB + YE + 8 * (4 + 8 * warp + 2 * t));
-    // ring position: slot index and phase advance together (no modulo in the loop)
-    uint32_t slot = 0, phase = 0;
-    auto advance = [&]() {
-      if (++slot == NS) {
-        slot = 0;
-        phase ^= 1u;
-      }
-    };
-    // One grid row: `dn` receives row i + 1 from the ring, then row i (held in `mid`, its slot still resident at
-    // mid_base) is processed with `up` = row i - 1.  Called with the three register rows in rotating roles, so the
-    // window never has to be copied.
-    // a warp whose segment lies beyond the row end (last tile of a row, m not a multiple of TJ) only keeps the ring moving
-    auto row_skip = [&](uint32_t& mid_slot) {
-      mbar_wait(full0 + 8 * slot, phase);
-      __syncwarp();
-      if (lane == 0) mbar_arrive(empty0 + 8 * mid_slot);
-      mid_slot = slot;
-      advance();
-    };
-    auto row_step = [&](double2 (&up)[NB], double2 (&mid)[NB], double2 (&dn)[NB], uint32_t& mid_base,
-                        uint32_t& mid_slot, double* const (&jp)[NB], int64_t ro) {
+  for (int I = 0; I < NB; ++I) poff[I] = (uint32_t)((8 * I + g) * PB + 8 * (4 + 8 * warp + 2 * t));
+  const int lastcol = 8 * (NB - 1) + g;
+  const int lastkind = lastcol < p.k ? 0 : (lastcol == p.k ? 1 : 2);  // 0 basis column, 1 the residual, 2 padding
+  if (lastkind == 1) poff[NB - 1] = (uint32_t)(8 * NB * PB + 8 * (4 + 8 * warp + 2 * t));
+  if (lastkind == 2) poff[NB - 1] = poff[0];                          // any valid (finite) data; multiplied by 0
+  // No selects in the loop: the last block runs the same stencil code with per-lane weights -- a basis column keeps
+  // (cu, cl, dg, cd); the residual column uses (0, 0, 1, 0), which returns `mid` exactly (0 * finite = 0, 0 + x = x);
+  // a padding column uses all zeros.  dg = wsel * (d0 + lam e) + wone is exact for wsel, wone in {0, 1}.
+  const double wsel = lastkind == 0 ? 1.0 : 0.0, wone = lastkind == 1 ? 1.0 : 0.0;
+  const double cuL = wsel * cu, clL = wsel * cl, cdL = wsel * cd;
+  const uint32_t eoff = (uint32_t)(8 * NB * PB + YE + 8 * (4 + 8 * warp + 2 * t));
+  on_start();
+  // ring position: slot index and phase advance together (no modulo in the loop)
+  uint32_t slot = 0, phase = 0;
+  auto advance = [&]() {
+    if (++slot == NS) {
+      slot = 0;
+      phase ^= 1u;
+    }
+  };
+  // One grid row: `dn` receives row i + 1 from the ring, then row i (held in `mid`, its slot still resident at
+  // mid_base) is processed with `up` = row i - 1.  Called with the three register rows in rotating roles, so the
+  // window never has to be copied.
+  // a warp whose segment lies beyond the row end (last tile of a row, m not a multiple of TJ) only keeps the ring moving
+  auto row_skip = [&](uint32_t& mid_slot) {
+    mbar_wait(full0 + 8 * slot, phase);
+    __syncwarp();
+    if (lane == 0) mbar_arrive(empty0 + 8 * mid_slot);
+    mid_slot = slot;
+    advance();
+  };
+  auto row_step = [&](double2 (&up)[NB], double2 (&mid)[NB], double2 (&dn)[NB], uint32_t& mid_base,
+                      uint32_t& mid_slot, int64_t e_off) {
+    mbar_wait(full0 + 8 * slot, phase);
+    const uint32_t base = ring0 + slot * SB;
+#pragma unroll
+    for (int I = 0; I < NB; ++I) dn[I] = lds2(base + poff[I]);
+    double lf[NB], rt[NB];
+#pragma unroll
+    for (int I = 0; I < NB; ++I) {
+      lf[I] = lds1(mid_base + poff[I] - 8);
+      rt[I] = lds1(mid_base + poff[I] + 16);
+    }
+    double2 e = make_double2(0.0, 0.0);
+    if (p.has_e) e = lds2(mid_base + eoff);
+    __syncwarp();
+    if (lane == 0) mbar_arrive(empty0 + 8 * mid_slot);  // the mid row's slot goes back to the producer
+    mid_base = base;
+    mid_slot = slot;
+    advance();
+    const double dga = sg * __dadd_rn(d0, __dmul_rn(p.lam, e.x)), dgb = sg * __dadd_rn(d0, __dmul_rn(p.lam, e.y));
+    const double dgaL = fma(wsel, dga, wone), dgbL = fma(wsel, dgb, wone);
+    double2 tile[NB];
+#pragma unroll
+    for (int I = 0; I < NB; ++I) {
+      const bool last = I == NB - 1;
+      const double oa = apply_refbits(last ? cuL : cu, last ? clL : cl, last ? dgaL : dga, last ? cdL : cd, up[I].x,
+                                      lf[I], mid[I].x, mid[I].y, dn[I].x);
+      const double ob = apply_refbits(last ? cuL : cu, last ? clL : cl, last ? dgbL : dgb, last ? cdL : cd, up[I].y,
+                                      mid[I].x, mid[I].y, rt[I], dn[I].y);
+      tile[I] = make_double2(oa, ob);
+    }
+    on_row(tile, e_off);
+  };
+  for (int64_t task = blockIdx.x; task < ntask; task += gridDim.x) {
+    const int strip = (int)(task / ntj), tj = (int)(task - (int64_t)strip * ntj);
+    const int i0 = strip * TI, i1 = min(i0 + TI, p.rows);
+    const bool active = tj * TJ + 8 * warp < m;  // the last tile of a row may be narrower than TJ (whole segments)
+    double2 ra[NB], rb[NB], rc[NB];
+    {  // row i0 - 1
       mbar_wait(full0 + 8 * slot, phase);
       const uint32_t base = ring0 + slot * SB;
 #pragma unroll
-      for (int I = 0; I < NB; ++I) dn[I] = lds2(base + poff[I]);
-      double lf[NB], rt[NB];
-#pragma unroll
-      for (int I = 0; I < NB; ++I) {
-        lf[I] = lds1(mid_base + poff[I] - 8);
-        rt[I] = lds1(mid_base + poff[I] + 16);
-      }
-      double2 e = make_double2(0.0, 0.0);
-      if (p.has_e) e = lds2(mid_base + eoff);
+      for (int I = 0; I < NB; ++I) ra[I] = lds2(base + poff[I]);
       __syncwarp();
-      if (lane == 0) mbar_arrive(empty0 + 8 * mid_slot);  // the mid row's slot goes back to the producer
-      mid_base = base;
-      mid_slot = slot;
+      if (lane == 0) mbar_arrive(empty0 + 8 * slot);
       advance();
-      const double dga = sg * __dadd_rn(d0, __dmul_rn(p.lam, e.x)), dgb = sg * __dadd_rn(d0, __dmul_rn(p.lam, e.y));
-      const double dgaL = fma(wsel, dga, wone), dgbL = fma(wsel, dgb, wone);
-      double2 tile[NB];
+    }
+    uint32_t mid_base, mid_slot;
+    {  // row i0
+      mbar_wait(full0 + 8 * slot, phase);
+      mid_base = ring0 + slot * SB;
+      mid_slot = slot;
 #pragma unroll
-      for (int I = 0; I < NB; ++I) {
-        const bool last = I == NB - 1;
-        const double oa = apply_refbits(last ? cuL : cu, last ? clL : cl, last ? dgaL : dga, last ? cdL : cd, up[I].x,
-                                        lf[I], mid[I].x, mid[I].y, dn[I].x);
-        const double ob = apply_refbits(last ? cuL : cu, last ? clL : cl, last ? dgbL : dgb, last ? cdL : cd, up[I].y,
-                                        mid[I].x, mid[I].y, rt[I], dn[I].y);
-        tile[I] = make_double2(oa, ob);
-        // J V goes out with plain 128-bit streaming stores (a quad writes 64 contiguous bytes of a column); staging it in
-        // shared memory for cp.async.bulk.tensor stores was built and measured SLOWER in situ (46.2 vs 41.0 ms per solve)
-        if (!last || lastkind == 0) __stcs(reinterpret_cast<double2*>(jp[I] + ro), tile[I]);
+      for (int I = 0; I < NB; ++I) rb[I] = lds2(mid_base + poff[I]);
+      advance();
+    }
+    int64_t e_off = (int64_t)i0 * m + tj * TJ + 8 * warp + 2 * t;
+    int i = i0;
+    if (active) {
+      while (true) {  // three rows per trip, the window rotating through (ra, rb, rc)
+        row_step(ra, rb, rc, mid_base, mid_slot, e_off);
+        e_off += m;
+        if (++i == i1) break;
+        row_step(rb, rc, ra, mid_base, mid_slot, e_off);
+        e_off += m;
+        if (++i == i1) break;
+        row_step(rc, ra, rb, mid_base, mid_slot, e_off);
+        e_off += m;
+        if (++i == i1) break;
       }
+    } else {
+      for (; i < i1; ++i) row_skip(mid_slot);
+    }
+    __syncwarp();
+    if (lane == 0) mbar_arrive(empty0 + 8 * mid_slot);  // row i1 was only ever a dn row
+  }
+  return true;
+}
+
+// Pass 1: the Gram matrix of the panel [sign J V | r], and J V itself when STORE (the CholeskyQR2 pass and the
+// Householder fallback read it back; the refinement form recomputes it in stencil_refine_kernel).
+template <int NB, int CW, bool STORE>
+__global__ void __launch_bounds__(32 * (CW + 1), 1)
+    stencil_gram_kernel(const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmY,
+                        const __grid_constant__ CUtensorMap tmE, StencilPanel p, int TI, double* __restrict__ JV,
+                        double* __restrict__ partials, unsigned int* ticket, double* __restrict__ Gout) {
+  constexpr int NBLK = nblocks(NB);
+  __shared__ __align__(16) double red[NBLK * 64];
+  const int g = (threadIdx.x & 31) >> 2;
+  double acc[NBLK][2];
+#pragma unroll
+  for (int b = 0; b < NBLK; ++b) acc[b][0] = acc[b][1] = 0.0;
+  double* jp[NB];  // this lane's J V columns
+#pragma unroll
+  for (int I = 0; I < NB; ++I) jp[I] = JV + (int64_t)(8 * I + g) * p.ldjv;
+  const bool last_is_basis = 8 * (NB - 1) + g < p.k;
+  stencil_sweep<NB, CW>(tmV, tmY, tmE, p, TI, nullptr, [] {}, [&](const double2 (&tile)[NB], int64_t e) {
+    if constexpr (STORE) {
+      // J V goes out with plain 128-bit streaming stores (a quad writes 64 contiguous bytes of a column); staging it in
+      // shared memory for cp.async.bulk.tensor stores was built and measured SLOWER in situ (46.2 vs 41.0 ms per solve)
 #pragma unroll
       for (int I = 0; I < NB; ++I)
+        if (I < NB - 1 || last_is_basis) __stcs(reinterpret_cast<double2*>(jp[I] + e), tile[I]);
+    }
 #pragma unroll
-        for (int J = I; J < NB; ++J) {
-          const int b = blk_index(NB, I, J);
-          dmma(acc[b][0], acc[b][1], tile[I].x, tile[J].x);
-          dmma(acc[b][0], acc[b][1], tile[I].y, tile[J].y);
-        }
-    };
-    for (int64_t task = blockIdx.x; task < ntask; task += gridDim.x) {
-      const int strip = (int)(task / ntj), tj = (int)(task - (int64_t)strip * ntj);
-      const int i0 = strip * TI, i1 = min(i0 + TI, p.rows);
-      const bool active = tj * TJ + 8 * warp < m;  // the last tile of a row may be narrower than TJ (whole segments)
-      double2 ra[NB], rb[NB], rc[NB];
-      {  // row i0 - 1
-        mbar_wait(full0 + 8 * slot, phase);
-        const uint32_t base = ring0 + slot * SB;
+    for (int I = 0; I < NB; ++I)
 #pragma unroll
-        for (int I = 0; I < NB; ++I) ra[I] = lds2(base + poff[I]);
-        __syncwarp();
-        if (lane == 0) mbar_arrive(empty0 + 8 * slot);
-        advance();
+      for (int J = I; J < NB; ++J) {
+        const int b = blk_index(NB, I, J);
+        dmma(acc[b][0], acc[b][1], tile[I].x, tile[J].x);
+        dmma(acc[b][0], acc[b][1], tile[I].y, tile[J].y);
       }
-      uint32_t mid_base, mid_slot;
-      {  // row i0
-        mbar_wait(full0 + 8 * slot, phase);
-        mid_base = ring0 + slot * SB;
-        mid_slot = slot;
+  });
+  reduce_gram<NBLK, CW, 32 * (CW + 1)>(acc, red, partials, ticket, Gout);
+}
+
+// Pass 2, refinement form, with J V recomputed instead of read back: rho = y - (sign A) d0, g = (sign A)^T rho and
+// sum rho^2 for A = J V_k, the same quantities as cholqr_refine_kernel, without the 8 n k bytes of the J V store in
+// pass 1.  The sweep's lanes hold 8 columns of a point pair each: rho is their weighted sum, completed over the 8 g-lanes
+// by a butterfly (all eight end with the same bits), then every lane accumulates g for its own columns.
+// Output as cholqr_refine_kernel: the last CTA writes (sign A)^T rho, then sum rho^2, to gout.
+template <int NB, int CW>
+__global__ void __launch_bounds__(32 * (CW + 1), 1)
+    stencil_refine_kernel(const __grid_constant__ CUtensorMap tmV, const __grid_constant__ CUtensorMap tmY,
+                          const __grid_constant__ CUtensorMap tmE, StencilPanel p, int TI, double sign,
+                          const double* __restrict__ d0g, const int* __restrict__ status,
+                          double* __restrict__ partials, unsigned int* ticket, double* __restrict__ gout) {
+  constexpr int NC = 8 * NB;  // panel columns held by a warp (basis, residual, padding)
+  __shared__ double wsum[CW][NC + 1];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int g = lane >> 2;
+  double gacc[NB], rr = 0.0;
 #pragma unroll
-        for (int I = 0; I < NB; ++I) rb[I] = lds2(mid_base + poff[I]);
-        advance();
-      }
-      const int j = tj * TJ + 8 * warp + 2 * t;
-      double* jp[NB];  // this lane's J V columns at (row 0, j); ro = i * m advances with the rows
+  for (int I = 0; I < NB; ++I) gacc[I] = 0.0;
+  double w[NB];  // rho = sum over the panel columns of w * column: -sign d0 on the basis, 1 on the residual, 0 beyond
+  auto weights = [&] {
 #pragma unroll
-      for (int I = 0; I < NB; ++I) jp[I] = JV + (int64_t)(8 * I + g) * p.ldjv + j;
-      int64_t ro = (int64_t)i0 * m;
-      int i = i0;
-      if (active) {
-        while (true) {  // three rows per trip, the window rotating through (ra, rb, rc)
-          row_step(ra, rb, rc, mid_base, mid_slot, jp, ro);
-          ro += m;
-          if (++i == i1) break;
-          row_step(rb, rc, ra, mid_base, mid_slot, jp, ro);
-          ro += m;
-          if (++i == i1) break;
-          row_step(rc, ra, rb, mid_base, mid_slot, jp, ro);
-          ro += m;
-          if (++i == i1) break;
-        }
-      } else {
-        for (; i < i1; ++i) row_skip(mid_slot);
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(empty0 + 8 * mid_slot);  // row i1 was only ever a dn row
+    for (int I = 0; I < NB; ++I) {
+      const int col = 8 * I + g;
+      w[I] = col < p.k ? -sign * d0g[col] : (col == p.k ? 1.0 : 0.0);
+    }
+  };
+  const bool run = stencil_sweep<NB, CW>(tmV, tmY, tmE, p, TI, status, weights, [&](const double2 (&tile)[NB], int64_t) {
+    double2 q = make_double2(0.0, 0.0);
+#pragma unroll
+    for (int I = 0; I < NB; ++I) {
+      q.x = fma(w[I], tile[I].x, q.x);
+      q.y = fma(w[I], tile[I].y, q.y);
+    }
+#pragma unroll
+    for (int o = 4; o < 32; o <<= 1) {
+      q.x += __shfl_xor_sync(0xffffffffu, q.x, o);
+      q.y += __shfl_xor_sync(0xffffffffu, q.y, o);
+    }
+#pragma unroll
+    for (int I = 0; I < NB; ++I) gacc[I] = fma(tile[I].x, q.x, fma(tile[I].y, q.y, gacc[I]));
+    rr = fma(q.x, q.x, fma(q.y, q.y, rr));
+  });
+  if (!run) return;
+  // CTA partial: over the 4 t-lanes of a column, then over the consumer warps in warp order
+#pragma unroll
+  for (int I = 0; I < NB; ++I) {
+    gacc[I] += __shfl_xor_sync(0xffffffffu, gacc[I], 1);
+    gacc[I] += __shfl_xor_sync(0xffffffffu, gacc[I], 2);
+  }
+  rr += __shfl_xor_sync(0xffffffffu, rr, 1);
+  rr += __shfl_xor_sync(0xffffffffu, rr, 2);
+  if (warp < CW && (lane & 3) == 0) {
+#pragma unroll
+    for (int I = 0; I < NB; ++I) wsum[warp][8 * I + g] = gacc[I];
+    if (lane == 0) wsum[warp][NC] = rr;  // rho is the same on every g-lane: one lane counts each point
+  }
+  __syncthreads();
+  constexpr int PS = MAXC + 1;  // partial stride: 32 columns, then sum rho^2
+  double* mine = partials + (int64_t)blockIdx.x * PS;
+  if (threadIdx.x <= NC) {
+    double v = wsum[0][threadIdx.x];
+    for (int q = 1; q < CW; ++q) v += wsum[q][threadIdx.x];
+    mine[threadIdx.x == NC ? MAXC : threadIdx.x] = v;
+    __threadfence();
+  }
+  if (!grid_arrive_last(ticket)) return;
+  if (threadIdx.x < PS) {
+    double v = 0.0;
+    const int nb = gridDim.x;
+    const int e = threadIdx.x;
+    if (e < p.k || e == MAXC) {
+      for (int b = 0; b < nb; ++b) v += __ldcg(partials + (int64_t)b * PS + e);
+      if (e < p.k) gout[e] = sign * v;  // (sign A)^T rho
+      else gout[p.k] = v;               // sum rho^2
     }
   }
-  reduce_gram<NBLK, CW, NT>(acc, red, partials, ticket, Gout);
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -1114,36 +1224,60 @@ int make_column_map(CUtensorMap* tm, const double* base, int m, int stored_rows,
   return 0;
 }
 
+// dynamic shared memory of a ring kernel, set once per device (done: one flag per device of that kernel)
+template <class Kern>
+int ring_smem_attr(gnk_ctx* ctx, Kern kern, int dyn, bool (&done)[64]) {
+  if (!done[ctx->device & 63]) {
+    GNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
+    done[ctx->device & 63] = true;
+  }
+  return 0;
+}
+
 template <int NB, int RU, int CW>
 int run_stencil_gram_cw(gnk_ctx* ctx, const gnk_layout* lay, const gnk_bratu* prm, const double* d_expu, const double* d_V,
-                     int64_t ldv, int v_cols, int k, const double* d_r, double sign, double* d_JV, int64_t ldjv,
+                     int64_t ldv, int k, const double* d_r, double sign, double* d_JV, int64_t ldjv,
                      double sign_a, double* d_out, cudaStream_t st) {
   if (int rc = ensure_scratch(ctx, st)) return rc;
   double* base = ctx->d_cholqr;
   constexpr int PW = 8 * CW + 8, TJ = 8 * CW;
   const int stored_rows = lay->rows + 2 * lay->halo;
   CUtensorMap tmV, tmY, tmE;
-  if (int rc = make_column_map(&tmV, d_V, lay->m, stored_rows, ldv, v_cols, 8 * NB, PW)) return rc;
+  // the map ends at column k although a box spans 8 NB columns: no lane consumes a basis column >= k (column k's lanes
+  // read the residual plane, padding lanes column g), so the TMA unit zero-fills them instead of reading them from HBM
+  if (int rc = make_column_map(&tmV, d_V, lay->m, stored_rows, ldv, k, 8 * NB, PW)) return rc;
   if (int rc = make_column_map(&tmY, d_r, lay->m, stored_rows, lay->ld, 1, 1, PW)) return rc;
   const bool has_e = prm->lam != 0.0;
   if (int rc = make_column_map(&tmE, has_e ? d_expu : d_r, lay->m, stored_rows, lay->ld, 1, 1, PW)) return rc;
-  auto kern = stencil_gram_kernel<NB, CW>;
-  constexpr int dyn = sg_dyn_bytes<NB, CW>();
-  static bool attr_set[64] = {false};  // one per template instance
-  if (!attr_set[ctx->device & 63]) {
-    GNK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, dyn));
-    attr_set[ctx->device & 63] = true;
-  }
   const int ntj = (lay->m + TJ - 1) / TJ;
   int TI = 64;
   while (TI > 8 && (int64_t)ntj * ceil_div(lay->rows, TI) < 6LL * ctx->sm_count) TI >>= 1;
   const int64_t ntask = (int64_t)ntj * ceil_div(lay->rows, TI);
   const int ctas = (int)(ntask < ctx->sm_count ? ntask : ctx->sm_count);
   StencilPanel p{lay->m, lay->rows, k, has_e ? 1 : 0, ldjv, prm->c_lap, prm->c_adv, prm->lam, sign};
-  GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), kern, dim3(ctas), dim3(32 * (CW + 1)), (size_t)dyn, st, tmV, tmY, tmE, p, TI, d_JV, base + CQ_PART,
+  constexpr int dyn = sg_dyn_bytes<NB, CW>();
+  static bool attr_store[64] = {false}, attr_free[64] = {false}, attr_refine[64] = {false};  // per template instance
+  const bool store = d_JV != nullptr;
+  auto gram = store ? stencil_gram_kernel<NB, CW, true> : stencil_gram_kernel<NB, CW, false>;
+  if (int rc = ring_smem_attr(ctx, gram, dyn, store ? attr_store : attr_free)) return rc;
+  GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), gram, dim3(ctas), dim3(32 * (CW + 1)), (size_t)dyn, st, tmV, tmY, tmE, p, TI, d_JV, base + CQ_PART,
                       ctx->d_tickets + TK_CHOLQR, base + CQ_LOCAL));
   GNK_LAUNCH_CHECK(ctx);
-  return cholqr_tail<NB, RU>(ctx, d_JV, ldjv, lay->n_own, k, d_r + lay->off, sign_a, d_out, st);
+  const double* d_y = d_r + lay->off;
+  if (store)
+    return cholqr_tail<NB, RU>(ctx, d_JV, ldjv, lay->n_own, k, d_y, sign_a, d_out, st, [&](int* status) {
+      return launch_refine_any(ctx, PanelSource{d_JV, ldjv, d_y, k, lay->n_own}, sign_a, base, status, st);
+    });
+  // J V was not stored: the refinement pass streams V_k through the same ring and applies the stencil again
+  return cholqr_tail<NB, RU>(ctx, nullptr, ldjv, lay->n_own, k, d_y, sign_a, d_out, st, [&](int* status) {
+    auto refine = stencil_refine_kernel<NB, CW>;
+    if (int rc = ring_smem_attr(ctx, refine, dyn, attr_refine)) return rc;
+    GNK_CUDA(gnk_launch(gnk_pdl_for(lay->n_own), refine, dim3(ctas), dim3(32 * (CW + 1)), (size_t)dyn, st, tmV, tmY, tmE, p, TI,
+                        sign_a, (const double*)(base + CQ_D0), (const int*)status, base + CQ_PART,
+                        ctx->d_tickets + TK_CHOLQR, base + CQ_LOCAL2));
+    GNK_LAUNCH_CHECK(ctx);
+    return 0;
+  });
 }
 
 }  // namespace
@@ -1166,19 +1300,20 @@ int gnk_cholqr_try(gnk_ctx* ctx, const double* d_A, int64_t lda, int64_t n_rows,
 // kernel is power-/FP64-bound, more FP64 work in flight lowers the SM clock under the power cap).
 template <int NB, int RU>
 int run_stencil_gram(gnk_ctx* ctx, const gnk_layout* lay, const gnk_bratu* prm, const double* d_expu, const double* d_V,
-                     int64_t ldv, int v_cols, int k, const double* d_r, double sign, double* d_JV, int64_t ldjv,
+                     int64_t ldv, int k, const double* d_r, double sign, double* d_JV, int64_t ldjv,
                      double sign_a, double* d_out, cudaStream_t st) {
-  return run_stencil_gram_cw<NB, RU, 8>(ctx, lay, prm, d_expu, d_V, ldv, v_cols, k, d_r, sign, d_JV, ldjv, sign_a, d_out,
+  return run_stencil_gram_cw<NB, RU, 8>(ctx, lay, prm, d_expu, d_V, ldv, k, d_r, sign, d_JV, ldjv, sign_a, d_out,
                                         st);
 }
 
-// gnk_stencil_gram_ls (gnk_b200.h): J V_k written AND the projected least squares solved with the panel read once.
-// Returns 1 when the panel is not eligible for the fused tensor-pipe path (the caller then runs gnk_stencil_apply +
-// gnk_tsqr_ls): the same conditions as gnk_tsqr_ls's tensor-pipe path, plus whole 8-point segments per grid row.
+// gnk_stencil_gram_ls (gnk_b200.h): J V_k written (unless d_JV is null) AND the projected least squares solved with the
+// panel read once.  Returns 1 when the panel is not eligible for the fused tensor-pipe path (the caller then runs
+// gnk_stencil_apply + gnk_tsqr_ls): the same conditions as gnk_tsqr_ls's tensor-pipe path, plus whole 8-point segments
+// per grid row, plus -- without J V -- the refinement form of the second pass (CholeskyQR2 reads J V back).
 extern "C" int gnk_stencil_gram_ls(gnk_ctx* ctx, const gnk_layout* lay, const gnk_bratu* prm, const double* d_expu,
                                    const double* d_V, int64_t ldv, int v_cols, int k, const double* d_r, double sign,
                                    double* d_JV, int64_t ldjv, double sign_a, double* d_out, void* stream) {
-  GNK_REQUIRE(ctx && lay && prm && d_V && d_r && d_JV && d_out, "gnk_stencil_gram_ls: null argument");
+  GNK_REQUIRE(ctx && lay && prm && d_V && d_r && d_out, "gnk_stencil_gram_ls: null argument");
   GNK_REQUIRE(lay->m > 0 && lay->rows > 0 && lay->halo == 2 && lay->off == 2LL * lay->m &&
                   lay->n_own == (int64_t)lay->rows * lay->m && lay->ld >= (int64_t)(lay->rows + 4) * lay->m,
               "gnk_stencil_gram_ls: inconsistent stencil layout");
@@ -1197,10 +1332,10 @@ extern "C" int gnk_stencil_gram_ls(gnk_ctx* ctx, const gnk_layout* lay, const gn
                        (d_expu == nullptr || (uintptr_t)d_expu % 16 == 0);
   if (!(fused_on && cholqr_on && ctx->ls_method != 1 && (sign == 1.0 || sign == -1.0) &&
         (sign_a == 1.0 || sign_a == -1.0) && aligned && lay->n_own >= 16384 && c <= 32 && c >= cholqr_min &&
-        c >= fused_min && encode_tiled_fn() != nullptr))
+        c >= fused_min && (d_JV != nullptr || second_pass_method(ctx) == 0) && encode_tiled_fn() != nullptr))
     return 1;
-  if (c <= 8) return run_stencil_gram<1, 4>(ctx, lay, prm, d_expu, d_V, ldv, v_cols, k, d_r, sign, d_JV, ldjv, sign_a, d_out, st);
-  if (c <= 16) return run_stencil_gram<2, 2>(ctx, lay, prm, d_expu, d_V, ldv, v_cols, k, d_r, sign, d_JV, ldjv, sign_a, d_out, st);
-  if (c <= 24) return run_stencil_gram<3, 1>(ctx, lay, prm, d_expu, d_V, ldv, v_cols, k, d_r, sign, d_JV, ldjv, sign_a, d_out, st);
-  return run_stencil_gram<4, 1>(ctx, lay, prm, d_expu, d_V, ldv, v_cols, k, d_r, sign, d_JV, ldjv, sign_a, d_out, st);
+  if (c <= 8) return run_stencil_gram<1, 4>(ctx, lay, prm, d_expu, d_V, ldv, k, d_r, sign, d_JV, ldjv, sign_a, d_out, st);
+  if (c <= 16) return run_stencil_gram<2, 2>(ctx, lay, prm, d_expu, d_V, ldv, k, d_r, sign, d_JV, ldjv, sign_a, d_out, st);
+  if (c <= 24) return run_stencil_gram<3, 1>(ctx, lay, prm, d_expu, d_V, ldv, k, d_r, sign, d_JV, ldjv, sign_a, d_out, st);
+  return run_stencil_gram<4, 1>(ctx, lay, prm, d_expu, d_V, ldv, k, d_r, sign, d_JV, ldjv, sign_a, d_out, st);
 }

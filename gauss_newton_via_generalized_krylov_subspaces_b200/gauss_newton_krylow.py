@@ -344,6 +344,12 @@ def gauss_newton_krylow(
     if is_bratu and prob.distributed and not tensor_ls_on_every_rank(prob.sol_fields["m"], rt.world):
         ls_method = 1
     fuse_trial = is_bratu and version == "res_old" and trial_project_fused(prob.sol_fields["m"], rt.world)
+    # One rank: the fused least squares may leave J V_k unstored and apply the stencil to V_k again in its refinement
+    # pass.  That pass costs what the sweep costs -- set by the NB = ceil((k+1)/8) column blocks the kernels carry, not by
+    # k -- while reading J V_k back costs bytes in k; with two or more blocks it is the faster chain once k > 6 NB
+    # (measured at 4096^2 for k = 7..30, DESIGN.md 3.1).  Several ranks keep the stored panel until the store-free pass has run on more than one
+    # GPU.
+    store_free_ok = rt.world == 1
 
     if user_code:
         F_cur[:n_res_own].copy_(r0)
@@ -386,18 +392,22 @@ def gauss_newton_krylow(
                 JV = rt.empty((jv_cap + (jv_cap >= _NB)) * ldjv)
             # projected operator and projected least squares  (:86-89)
             ls_done = False
-            # Bratu + QR: one TMA-staged kernel applies the stencil, stores J V_k and forms the Gram matrix of the
-            # panel in the same sweep (gnk_stencil_gram_ls); it answers 1 when the panel does not qualify
+            jv_valid = True  # J V_k is in JV (the Householder fallback below needs it)
+            # Bratu + QR: one TMA-staged kernel applies the stencil and forms the Gram matrix of the panel in the same
+            # sweep, storing J V_k only when asked (gnk_stencil_gram_ls); it answers 1 when the panel does not qualify
             if (is_bratu and ls_solver == "qr" and ls_method == 0 and k < _NB and not jac_ev.transposed
                     and jac_ev.scale == 1.0):
-                # algorithmic bytes (SURVEY 8d): the SpMM's 16nk + 8n plus the least-squares panel once, 8n(k+1)
-                with rt.mark("spmm+ls", 8.0 * n_res_own * (3 * k + 2)) as mk:
+                store_jv = not (store_free_ok and k >= 8 and k > 6 * ((k + 8) // 8))
+                # algorithmic bytes (SURVEY 8d): without the store, sweep and refinement each read V_k, e^u and one
+                # residual vector (16nk + 32n); with it, the SpMM's 16nk + 8n plus the panel once, 8n(k+1)
+                with rt.mark("spmm+ls", 8.0 * n_res_own * (3 * k + 2 if store_jv else 2 * k + 4)) as mk:
                     rc = lib.gnk_stencil_gram_ls(rt.ctx, C.byref(sol_lay), C.byref(prob.d.prm), ptr(jac_ev.expu),
-                                                 ptr(krylow.V), ld, krylow.cap, k, ptr(F_cur), -1.0, ptr(JV), ldjv,
-                                                 -1.0, ptr(blk), rt.stream)
+                                                 ptr(krylow.V), ld, krylow.cap, k, ptr(F_cur), -1.0,
+                                                 ptr(JV) if store_jv else None, ldjv, -1.0, ptr(blk), rt.stream)
                     mk.cancel = rc != 0
                 if rc == 0:
                     ls_done = True
+                    jv_valid = store_jv
                 elif rc != 1:
                     _lib.check(rc, "gnk_stencil_gram_ls")
             if not ls_done:
@@ -497,6 +507,9 @@ def gauss_newton_krylow(
             except _LeastSquaresRefused:
                 # CholeskyQR2 met a numerically rank deficient panel (d = 0 was written, the trial above evaluated the
                 # unchanged iterate and is not counted): same panel again through the Householder TSQR
+                if not jv_valid:
+                    with rt.mark("spmm", 8.0 * n_res_own * (2 * k + 1)):
+                        jac_ev.matmat(krylow.V, ld, k, JV, ldjv)
                 with rt.mark("tsqr", 8.0 * n_res_own * (k + 1)):
                     tsqr_solve(rt, JV, ldjv, n_res_own, k, F_cur[res_off:], -1.0, blk, householder=True)
                 state["rank_reported"] = False

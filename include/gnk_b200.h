@@ -213,13 +213,17 @@ int gnk_basis_ls_wide(gnk_ctx* ctx, double* d_P, int64_t ldp, int64_t n_rows, in
  * (gauss_newton_krylow.py:86 `JV = jac_ev @ krylow.basis` followed by :89 `linear_least_squares(-1 * JV, res_ev)`):
  *   JV[:, j] = sign * (M V[:, j]), j < k   -- written (owned rows, column stride ldjv), bit-identical to gnk_stencil_apply
  *   d_out    = the result block of gnk_tsqr_ls(JV, ldjv, n_own, k, r, sign_a)
- * with the least-squares panel READ ONCE: a TMA-staged, warp-specialised kernel streams V_k through shared memory
- * (cp.async.bulk.tensor row slots, mbarrier ring), applies the stencil, stores J V and accumulates the Gram matrix of
- * [J V | r] with FP64 tensor-core MMAs in the same sweep; the refinement (or second CholeskyQR2) pass then reads J V
- * once more.  d_V: v_cols >= k stored columns (stride ldv, halo rows valid), d_r: the residual as a stored column,
- * d_expu as in gnk_stencil_apply.  Returns 1 -- nothing launched -- when the panel does not qualify (fewer than 16384
- * owned unknowns, more than 32 panel columns, m not a multiple of 8, Householder path pinned, GNK_LS_FUSED=0, ...): the
- * caller then issues gnk_stencil_apply + gnk_tsqr_ls.  Refusal (d_out[k+2] = -1) as for gnk_tsqr_ls; J V is valid then. */
+ * with the least-squares panel never read back from HBM: a TMA-staged, warp-specialised kernel streams V_k through
+ * shared memory (cp.async.bulk.tensor row slots, mbarrier ring), applies the stencil, stores J V and accumulates the
+ * Gram matrix of [J V | r] with FP64 tensor-core MMAs in the same sweep; the refinement (or second CholeskyQR2) pass
+ * then reads J V once more.  d_JV may be NULL: J V is then not stored, and the refinement pass streams V_k through the
+ * same ring and applies the stencil again (8 n k bytes fewer); the Gram matrix, the first factor and the refinement
+ * decision are bit-identical to the storing call, d may differ in the last bits (g is summed in another order).
+ * d_V: v_cols >= k stored columns (stride ldv, halo rows valid), d_r: the residual as a stored column, d_expu as in
+ * gnk_stencil_apply.  Returns 1 -- nothing launched -- when the panel does not qualify (fewer than 16384 owned unknowns,
+ * more than 32 panel columns, m not a multiple of 8, Householder path pinned, GNK_LS_FUSED=0, d_JV NULL with the
+ * CholeskyQR2 pass pinned (method 2), ...): the caller then issues gnk_stencil_apply + gnk_tsqr_ls.  Refusal
+ * (d_out[k+2] = -1) as for gnk_tsqr_ls; J V is valid then if it was stored, else the caller forms it for the fallback. */
 int gnk_stencil_gram_ls(gnk_ctx* ctx, const gnk_layout* lay, const gnk_bratu* prm, const double* d_expu,
                         const double* d_V, int64_t ldv, int v_cols, int k, const double* d_r, double sign,
                         double* d_JV, int64_t ldjv, double sign_a, double* d_out, void* stream);
